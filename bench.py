@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - Kalman logp+grad filter-steps/s (draws x T) on N B200s, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--draws B] [--n T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--draws B] [--n T] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE batched logp+grad evaluation (theta[B,n_theta] -> logp[B], dlogp/dtheta[B,n_theta]).
@@ -16,6 +16,11 @@ A "step" is ONE batched logp+grad evaluation (theta[B,n_theta] -> logp[B], dlogp
 k+1).  `e2e` legs are host to host: every rank replays its own HostStepGraph (pinned theta -> H2D -> kernels -> D2H of
 its shard into its pinned buffer, chunked so that copies overlap kernels, stream-synchronised every step) - a
 host-resident sampler needs no device collective at all.  Rank 0 prints ONE JSON line.
+
+Both blocks time --steps steps per leg (c5: --c5-steps if given).  The inputs are seeded, so runs with the same
+arguments see identical inputs; `--dump-outputs DIR` makes rank 0 write what the resident leg returned in its last timed
+step, every draw's logp and gradient in draw order, as float64 `DIR/logp.npy`, `DIR/grad.npy` (and `DIR/c5_*.npy`), so
+that two builds can be compared output for output (see dump_rows for the sampling of large legs).
 """
 from __future__ import annotations
 
@@ -54,13 +59,37 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of the captured CUDA graphs")
     ap.add_argument("--c5-draws", type=int, default=0, help="c5 block: draws per GPU (0 = 2^20, 2^21 at 8 GPUs)")
-    ap.add_argument("--c5-steps", type=int, default=0, help="c5 block: timed steps (0 = min(--steps, 8))")
+    ap.add_argument("--c5-steps", type=int, default=0, help="c5 block: timed steps (0 = --steps)")
     ap.add_argument("--no-c5", action="store_true", help="skip the c5 block")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (logp, grad) arrays of the last timed step of each GPU leg to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1 or a.c5_steps < 0:
+        ap.error("--steps must be >= 1 and --c5-steps >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl b200")
+    return a
 
 
 def workload_name(a):
     return f"BayesianARMA(1,1) stationary init, {a.draws} draws/GPU x T={a.n}, standard filter, logp+dlogp/dtheta"
+
+
+DUMP_MAX_ROWS = 1 << 18   # per leg: 2 legs x 2^18 draws x (logp + <= 6 grads + index) x 8 B stays under 64 MB in all
+
+
+def dump_rows(out_dir, prefix, rows):
+    """Writes packed per-draw rows [N, 1 + n_theta] = (logp, dlogp/dtheta) as float64 ``<prefix>logp.npy`` [N] and
+    ``<prefix>grad.npy`` [N, n_theta].  Above DUMP_MAX_ROWS draws only a fixed, seeded sample of draws is written (the
+    same draws on every run with the same arguments), and ``<prefix>draw_index.npy`` lists them in ascending order."""
+    rows = rows.detach().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    if rows.shape[0] > DUMP_MAX_ROWS:
+        idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], DUMP_MAX_ROWS, replace=False))
+        rows = rows[idx]
+        np.save(os.path.join(out_dir, prefix + "draw_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, prefix + "logp.npy"), np.ascontiguousarray(rows[:, 0], dtype=np.float64))
+    np.save(os.path.join(out_dir, prefix + "grad.npy"), np.ascontiguousarray(rows[:, 1:], dtype=np.float64))
 
 
 # ---------------------------------------------------------------------------------------------- CPU side
@@ -284,12 +313,13 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
-        """K calls bracketed by barrier + synchronize on both sides, CUDA events on the launching stream, max over ranks."""
+        """K calls bracketed by barrier + synchronize on both sides, CUDA events on the launching stream, max over ranks.
+        Returns (ms per call, what the last call returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -297,7 +327,7 @@ def main():
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms / steps
+        return ms / steps, out
 
     def gather_graph(model, theta_d, waves):
         """Resident leg for N > 1 (and the wave pipeline of c5): one kernel graph per wave + NCCL all-gathers; eager fallback."""
@@ -347,7 +377,9 @@ def main():
         step_resident()
     launches0 = lib.kfb_launch_count()
     with ClockSampler(local) as clk:
-        ms_step = timed(step_resident, a.steps)
+        ms_step, last = timed(step_resident, a.steps)
+    if a.dump_outputs and rank == 0:   # every draw of every rank, in draw order
+        dump_rows(a.dump_outputs, "", last if world == 1 else step_resident.rows())
     launches = lib.kfb_launch_count() - launches0
     if launches == 0:  # graph replays do not pass through the launch counter: count one eager evaluation instead
         l0 = lib.kfb_launch_count()
@@ -358,7 +390,7 @@ def main():
 
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, a.steps)
+    ms_e2e, _ = timed(step_e2e, a.steps)
 
     # per-kernel durations of the two recursion kernels, CUDA events on the launching stream
     mats = model._scatter(theta_d)
@@ -498,7 +530,7 @@ def bench_c5(a, world, rank, dev, timed, gather_graph, use_graph):
     # 8-GPU step to it.
     waves = B5 >> 19 if (B5 >= (1 << 19) and B5 % (1 << 19) == 0) else (2 if B5 % 2 == 0 else 1)
     h = B5 // waves
-    steps = a.c5_steps or max(2, min(a.steps, 8))
+    steps = a.c5_steps or a.steps
     spec, y, theta = arma21_workload(B5, a.n, seed=1 + rank)      # every rank draws its own shard
     nt = spec.n_theta
     theta_h = torch.from_numpy(np.ascontiguousarray(theta)).pin_memory()
@@ -508,7 +540,9 @@ def bench_c5(a, world, rank, dev, timed, gather_graph, use_graph):
     gsg, how = gather_graph(model, theta_d, waves)
     for _ in range(2):
         gsg()
-    ms_res = timed(gsg, steps)
+    ms_res, _ = timed(gsg, steps)
+    if a.dump_outputs and rank == 0:
+        dump_rows(a.dump_outputs, "c5_", gsg.rows())
     bad = int((gsg.info != 0).sum())
     out0 = gsg.out[0, rank, :4].cpu().numpy().tolist() if rank == 0 else None
     host = model.capture_host_step(theta_h, out_h, chunks=waves, sequential=True) if use_graph else None
@@ -524,7 +558,7 @@ def bench_c5(a, world, rank, dev, timed, gather_graph, use_graph):
 
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, steps)
+    ms_e2e, _ = timed(step_e2e, steps)
     total = B5 * world * a.n
     return {
         "workload": f"BayesianARMA(2,1) stationary init, {B5} draws/GPU x T={a.n} ({B5 * world} draws in total), standard "

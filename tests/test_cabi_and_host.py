@@ -276,3 +276,27 @@ def test_reference_arm_uses_every_core_under_torchrun_env_and_only_rank0_prints(
     assert line["c5"]["cores"] == line["cpu_baseline"]["cores"]
     out = subprocess.run(cmd, env=dict(env, RANK="1"), capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0 and not [ln for ln in out.stdout.splitlines() if ln.startswith("{")]
+
+
+def test_bench_dump_rows_writes_all_or_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: small legs are written whole, large ones as the same seeded sample of draws every time."""
+    import bench
+
+    small = torch.arange(10 * 6, dtype=torch.float64).reshape(10, 6)
+    bench.dump_rows(str(tmp_path / "s"), "", small)
+    assert sorted(os.listdir(tmp_path / "s")) == ["grad.npy", "logp.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "s" / "logp.npy"), small[:, 0].numpy())
+    np.testing.assert_array_equal(np.load(tmp_path / "s" / "grad.npy"), small[:, 1:].numpy())
+
+    n = bench.DUMP_MAX_ROWS + 1000
+    big = torch.arange(n, dtype=torch.float64)[:, None] * torch.tensor([1.0, 2.0, 3.0])
+    for d in ("a", "b"):
+        bench.dump_rows(str(tmp_path / d), "c5_", big)
+    idx = np.load(tmp_path / "a" / "c5_draw_index.npy")
+    assert idx.dtype == np.float64 and idx.shape == (bench.DUMP_MAX_ROWS,) and (np.diff(idx) > 0).all()
+    assert idx[0] >= 0 and idx[-1] < n
+    for name in ("c5_draw_index", "c5_logp", "c5_grad"):
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float64 and np.array_equal(a, b), name
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "c5_logp.npy"), idx)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "c5_grad.npy"), idx[:, None] * [2.0, 3.0])

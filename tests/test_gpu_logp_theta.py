@@ -558,3 +558,33 @@ def test_theta_level_smoother_matches_oracle():
 
 def rel_err_np(a, b):
     return float(np.abs(np.asarray(a) - np.asarray(b)).max() / max(np.abs(np.asarray(b)).max(), 1e-300))
+
+
+def test_bench_dump_outputs_are_the_timed_paths_results(tmp_path):
+    """`bench.py --dump-outputs`: --steps sets the timed steps of both legs, and the dumped (logp, grad) of the headline
+    ARMA(1,1) and c5 ARMA(2,1) legs equal a direct evaluation of the same seeded workloads."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    from pymc_statespace_b200.synthetic import arma11_workload, arma21_workload
+    from tests.helpers import ROOT
+
+    B, B5, n, steps = 512, 4096, 64, 10
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+           "--draws", str(B), "--n", str(n), "--c5-draws", str(B5), "--no-cpu-baseline", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-3000:]
+    lines = [ln for ln in out.stdout.splitlines() if ln.startswith("{")]
+    assert len(lines) == 1
+    line = json.loads(lines[0])
+    assert line["steps"] == steps and line["c5"]["steps"] == steps
+    assert sorted(os.listdir(tmp_path)) == ["c5_grad.npy", "c5_logp.npy", "grad.npy", "logp.npy"]
+    for prefix, (spec, y, theta) in (("", arma11_workload(B, n)), ("c5_", arma21_workload(B5, n))):
+        logp, grad, _ = _run(spec, y, theta)
+        got_l, got_g = np.load(tmp_path / f"{prefix}logp.npy"), np.load(tmp_path / f"{prefix}grad.npy")
+        assert got_l.dtype == np.float64 and got_g.dtype == np.float64
+        assert got_l.shape == logp.shape and got_g.shape == grad.shape
+        np.testing.assert_allclose(got_l, logp, rtol=1e-12, atol=0)
+        np.testing.assert_allclose(got_g, grad, rtol=1e-12, atol=1e-12 * np.abs(grad).max())
