@@ -85,6 +85,17 @@ enum {
                                     (BayesianARMA / SARIMAX, reference models/SARIMAX.py:59-98).  Only honoured together
                                     with the two flags above; the columns >= 1 of the T gradient are then returned as 0 */
 
+/* Time-parallel evaluation (k_endog = 1, k_states <= 4, standard / single / cholesky): one CTA per unit runs the filter
+ * and its adjoint as blocked scans over time (Saerkkae & Garcia-Fernandez filtering elements forward, affine and
+ * congruence scans backward), instead of one thread walking all n steps.  For few units and long series (one NUTS draw
+ * per call); with many units the sequential kernels are faster.  Same outputs, gradients and info codes as without the
+ * flag, to rounding (the sums run in another fixed order; two runs give identical bits).  Any other geometry with the
+ * flag set returns KFB_ERR_UNSUPPORTED (k_endog > 1, k_states > 4, univariate, steady_state).  The structure promises
+ * above are not used on this path (nothing is skipped or verified).  A unit whose parallel element is undefined at some
+ * step (Z C Z^T + H = 0 there: an observation without noise given the previous state) is run by one thread of its CTA
+ * with the sequential recursion; no info code marks it.  The forward pass always uses the tape part of the workspace. */
+#define KFB_FLAG_TIME_PARALLEL 128u
+
 typedef struct kfb_desc {
   int32_t filter_kind;
   uint32_t flags;

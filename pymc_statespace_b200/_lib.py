@@ -25,6 +25,7 @@ KFB_FLAG_Z_UNIT0 = 8
 KFB_FLAG_H_ZERO = 16
 KFB_FLAG_T_COMPANION = 32
 KFB_FLAG_NO_MISSING = 64
+KFB_FLAG_TIME_PARALLEL = 128
 KFB_INFO_DARE_FAILED = 0x40000001
 KFB_INFO_NOT_STATIONARY = 0x40000002
 KFB_INFO_BAD_STRUCTURE = 0x40000003

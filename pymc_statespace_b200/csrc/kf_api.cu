@@ -21,6 +21,9 @@ bool p1_adjoint_supported(int m, int p, int mk);
 cudaError_t launch_p1_adjoint(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 cudaError_t launch_p1_forward(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 
+bool tpar_supported(int m, int p, int mk);
+cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
+
 coopT_launch_fn coopT_launcher_m5(int p, int mk);
 coopT_launch_fn coopT_launcher_m6(int p, int mk);
 coopT_launch_fn coopT_launcher_m7(int p, int mk);
@@ -121,6 +124,7 @@ struct Plan {
   double ll_const, d_sign;
   bool tv_any, use_thread;
   bool compressed;   // k_endog = 1 kernels with all four structure promises: tape entries hold a_t and the leading block of P_t
+  bool tpar;         // KFB_FLAG_TIME_PARALLEL: one CTA per unit, scans over time (kf_tpar.cu); tape [u][t][a_t, P_t]
   long long U, nD;
   int nTC;           // time entries of C = R Q R^T (1 or n)
   long long C_bs;    // 0 if R and Q are shared by all draws
@@ -149,6 +153,9 @@ static kfb_status make_plan(const kfb_desc* d, bool save, Plan* pl) {
   }
   pl->tv_any = d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts;
   if (pl->tv_any && (pl->mk == MK_UNIV || pl->mk == MK_STEADY)) return KFB_ERR_UNSUPPORTED;
+  // time-parallel form: k_endog = 1, k_states <= 4, standard-family filters only
+  pl->tpar = (d->flags & KFB_FLAG_TIME_PARALLEL) != 0;
+  if (pl->tpar && !tpar_supported(d->m, d->p, pl->mk)) return KFB_ERR_UNSUPPORTED;
   pl->U = d->n_draws * d->n_series;
   pl->nD = d->n_draws;
   pl->nTC = (d->R_ts || d->Q_ts) ? d->n : 1;
@@ -171,7 +178,11 @@ static kfb_status make_plan(const kfb_desc* d, bool save, Plan* pl) {
   pl->compressed = pl->use_thread && !pl->tv_any && d->y_bs == 0 && d->n_series == 1 && (d->flags & kPromises) == kPromises &&
                    !(d->flags & KFB_FLAG_GENERIC_ADJOINT) && p1_adjoint_supported(d->m, d->p, pl->mk);
   pl->off_tape = pl->off_gC = 0;
-  if (save) {
+  if (pl->tpar) {
+    // the forward pass always writes the tape (its parallel map reads the predicted moments back from it)
+    pl->off_tape = take((size_t)pl->U * d->n * (d->m + d->m * d->m));
+    if (save) pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
+  } else if (save) {
     const size_t entry = pl->compressed ? (size_t)(1 + ((d->m - 1) * d->m) / 2) : (size_t)tape_width(d->m);
     pl->off_tape = take((size_t)tape_units_padded(pl->U) * (d->n > 1 ? d->n - 1 : 0) * entry);
     pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
@@ -297,7 +308,7 @@ kfb_status kfb_forward(const kfb_desc* desc, const kfb_inputs* in, const kfb_out
   fill_args(desc, in, pl, ws, &A);
   A.loglik = out->loglik; A.ll_obs = out->ll_obs; A.fs = out->filtered_states; A.ps = out->predicted_states;
   A.fc = out->filtered_covs; A.pc = out->predicted_covs; A.info = out->info;
-  A.tape = save_for_backward ? (double*)(ws + pl.off_tape) : nullptr;
+  A.tape = (save_for_backward || pl.tpar) ? (double*)(ws + pl.off_tape) : nullptr;
   const long long nDC = pl.C_bs ? desc->n_draws : 1;
   cudaError_t e = launch_rqr_forward(nDC, pl.nTC, desc->m, desc->r, MatArg{in->R, desc->R_bs, desc->R_ts},
                                      MatArg{in->Q, desc->Q_bs, desc->Q_ts}, (double*)(ws + pl.off_C), s);
@@ -314,6 +325,10 @@ kfb_status kfb_forward(const kfb_desc* desc, const kfb_inputs* in, const kfb_out
     e = fast ? fast(D, s) : launch_dare(D, false, s);  // even k_states 18..32, k_endog 1: tensor-core mapping (kf_rowsD.cuh)
     if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
     if (e != cudaSuccess) return cuda_fail(e);
+  }
+  if (pl.tpar) {
+    e = launch_tpar(A, false, s);
+    return e == cudaSuccess ? KFB_OK : cuda_fail(e);
   }
   return launch_main(desc, pl, A, false, s);
 }
@@ -340,8 +355,13 @@ kfb_status kfb_backward(const kfb_desc* desc, const kfb_inputs* in, const kfb_co
     A.gPss = (double*)(ws + pl.off_gPss);
     A.gGss = (double*)(ws + pl.off_gGss);
   }
-  st = launch_main(desc, pl, A, true, s);
-  if (st != KFB_OK) return st;
+  if (pl.tpar) {
+    cudaError_t e = launch_tpar(A, true, s);
+    if (e != cudaSuccess) return cuda_fail(e);
+  } else {
+    st = launch_main(desc, pl, A, true, s);
+    if (st != KFB_OK) return st;
+  }
   if (pl.mk == MK_STEADY) {
     // chain (P_steady-bar, F_inv-bar) through the DARE (utils/pytensor_scipy.py:39-60) into T, Z, H, C
     DareArgs D;

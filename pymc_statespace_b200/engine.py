@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from ._lib import (FILTER_KIND, KFB_FLAG_CORRECTED, KFB_FLAG_FORCE_COOP, KFB_FLAG_GENERIC_ADJOINT, KFB_FLAG_H_ZERO,
-                   KFB_FLAG_NO_MISSING, KFB_FLAG_T_COMPANION, KFB_FLAG_Z_UNIT0, KfbCotangents, KfbDesc, KfbGrads, KfbInputs,
+                   KFB_FLAG_NO_MISSING, KFB_FLAG_T_COMPANION, KFB_FLAG_TIME_PARALLEL, KFB_FLAG_Z_UNIT0, KfbCotangents, KfbDesc, KfbGrads, KfbInputs,
                    KfbOutputs, check, load)
 
 MATRIX_NAMES = ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")
@@ -44,12 +44,17 @@ class BatchedKalman:
     base = shared by all draws; base+1 = one per draw ``[B,...]``; names listed in ``time_varying`` carry
     an extra time axis right before the matrix axes (``[n,...]`` or ``[B,n,...]``), i.e. time-first as in
     reference ``filters/utilities.py:9-14``.  ``y`` is ``[n,p]`` (shared) or ``[S,n,p]`` (one per series).
+
+    ``time_parallel=True`` asks for the time-parallel kernels (one CTA per unit, scans over time: faster with few units
+    and long series, see DESIGN.md section 8).  They exist for k_endog = 1, k_states <= 4 and the standard / single /
+    cholesky filters; any other geometry runs the sequential kernels exactly as without the option.
+    ``time_parallel_active`` says which path runs.
     """
 
     def __init__(self, kind: str, n: int, m: int, p: int, r: int, n_draws: int, n_series: int = 1,
                  strict_reference: bool = True, time_varying: Iterable[str] = (), device="cuda",
                  force_coop: bool = False, generic_adjoint: bool = False, z_unit0: bool = False, h_zero: bool = False,
-                 pad_odd: bool = True, t_companion: bool = False, no_missing: bool = False):
+                 pad_odd: bool = True, t_companion: bool = False, no_missing: bool = False, time_parallel: bool = False):
         kind = kind.lower()
         if kind not in FILTER_KIND:
             raise NotImplementedError("The following are valid filter types: " + ", ".join(FILTER_KIND))
@@ -70,6 +75,9 @@ class BatchedKalman:
                       | (KFB_FLAG_T_COMPANION if (t_companion and h_zero and z_unit0) else 0)
                       # + no NaN in y: with all four the tape holds only what varies from step to step
                       | (KFB_FLAG_NO_MISSING if (no_missing and t_companion and h_zero and z_unit0) else 0))
+        self.time_parallel = bool(time_parallel)
+        if self.time_parallel and kind in ("standard", "single", "cholesky") and self.p == 1 and self.m <= 4:
+            self.flags |= KFB_FLAG_TIME_PARALLEL
         self._base = {"a0": (m,), "P0": (m, m), "T": (m, m), "Z": (p, m), "R": (m, r), "H": (p, p), "Q": (r, r),
                       "c": (m,), "d": (p,)}
         self._desc = None
@@ -86,6 +94,11 @@ class BatchedKalman:
                 and self.n_series == 1 and kind in ("standard", "single", "cholesky", "steady_state")):
             self._inner = BatchedKalman(kind, n, m + 1, p, r, n_draws, n_series, strict_reference, (), device,
                                         generic_adjoint=generic_adjoint, pad_odd=False)
+
+    @property
+    def time_parallel_active(self) -> bool:
+        """True if forward / backward run the time-parallel kernels (``time_parallel=True`` on a geometry that has them)."""
+        return bool(self.flags & KFB_FLAG_TIME_PARALLEL)
 
     # ------------------------------------------------------------------ helpers
     def _canon(self, name, t):

@@ -61,6 +61,8 @@ class BaseFilter:
         self.non_seq_names: List[str] = []
         self.eye_states = self.eye_posdef = self.eye_endog = None  # attrs of the reference object; unused here
         self.strict_reference = strict_reference
+        # opt-in time-parallel kernels (k_endog = 1, k_states <= 4): faster for one draw per call over long series
+        self.time_parallel = False
         self.device = device
 
     @staticmethod

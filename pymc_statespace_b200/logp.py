@@ -166,7 +166,8 @@ def logp_and_grad_in_waves(spec: StateSpaceSpec, data, theta: torch.Tensor, filt
 
 class KalmanLogp:
     def __init__(self, spec: StateSpaceSpec, data, n_draws: int, filter_type: str = "standard",
-                 strict_reference: bool = True, device="cuda", force_coop: bool = False, pad_to_fused: bool = True):
+                 strict_reference: bool = True, device="cuda", force_coop: bool = False, pad_to_fused: bool = True,
+                 time_parallel: bool = False):
         # sizes between the fused instantiations (odd k_states in 9..31; e.g. seasonal models of period 12 or 24): embed
         # the model in the next instantiated (even) size - exact (models.pad_spec) and far cheaper than the generic
         # run-time-dims kernels, because the tensor-core kernels work on zero-padded 16 x 16 / 32 x 32 tiles anyway
@@ -178,6 +179,7 @@ class KalmanLogp:
         self.device = torch.device(device)
         self.lib = load()
         self.filter_type, self.strict_reference, self._force_coop = filter_type, strict_reference, force_coop
+        self.time_parallel = bool(time_parallel)  # BatchedKalman(time_parallel=...): scans over time for few draws
         y = data.detach().to(dtype=torch.float64) if isinstance(data, torch.Tensor) else np.asarray(data, dtype=np.float64)
         if y.ndim == 1:
             y = y[:, None]
@@ -203,7 +205,7 @@ class KalmanLogp:
         self.kalman = BatchedKalman(filter_type, self.n, spec.k_states, spec.k_endog, spec.k_posdef, n_draws=self.B,
                                     strict_reference=strict_reference, device=device, force_coop=force_coop,
                                     z_unit0=z_unit0, h_zero=h_zero, pad_odd=pad_to_fused, t_companion=t_companion,
-                                    no_missing=not bool(torch.isnan(self.y).any()))
+                                    no_missing=not bool(torch.isnan(self.y).any()), time_parallel=time_parallel)
         m, pp, r = spec.k_states, spec.k_endog, spec.k_posdef
         self._shape = {"a0": (m,), "P0": (m, m), "T": (m, m), "Z": (pp, m), "R": (m, r), "H": (pp, pp), "Q": (r, r),
                        "c": (m,), "d": (pp,)}
@@ -321,7 +323,8 @@ class KalmanLogp:
     def clone_for(self, n_draws: int) -> "KalmanLogp":
         """A second evaluator of the same model / data / filter for ``n_draws`` draws (own workspace and tape)."""
         return KalmanLogp(self.spec, self.y, n_draws=n_draws, filter_type=self.filter_type,
-                          strict_reference=self.strict_reference, device=self.device, force_coop=self._force_coop)
+                          strict_reference=self.strict_reference, device=self.device, force_coop=self._force_coop,
+                          time_parallel=self.time_parallel)
 
     def logp_and_grad(self, theta, g_loglik: Optional[torch.Tensor] = None):
         """Returns (logp[B], dlogp/dtheta[B, n_theta]); ``self.info[B]`` holds per-draw status."""

@@ -44,16 +44,18 @@ def _require():
 class KalmanFilterOp(Op):
     """(data, a0, P0, T, Z, R, H, Q[, c][, d]) -> the 6 outputs of BaseFilter.build_graph (kalman_filter.py:184-191)."""
 
-    __props__ = ("kind", "strict_reference", "has_c", "has_d")
+    __props__ = ("kind", "strict_reference", "has_c", "has_d", "time_parallel")
 
-    def __init__(self, kind, strict_reference=True, has_c=False, has_d=False):
+    def __init__(self, kind, strict_reference=True, has_c=False, has_d=False, time_parallel=False):
         self.kind, self.strict_reference, self.has_c, self.has_d = kind, bool(strict_reference), bool(has_c), bool(has_d)
+        self.time_parallel = bool(time_parallel)
 
     def _filter(self):
         from .filters import FILTER_FACTORY
 
         f = FILTER_FACTORY[self.kind]()
         f.strict_reference = self.strict_reference
+        f.time_parallel = self.time_parallel
         return f
 
     def _split(self, inputs):
@@ -101,7 +103,8 @@ class KalmanFilterOp(Op):
             g_ll = pt.zeros((), dtype="float64")
         if isinstance(g_llobs.type, DisconnectedType):
             g_llobs = pt.zeros_like(outputs[5])
-        grads = KalmanFilterGradOp(self.kind, self.strict_reference, self.has_c, self.has_d)(*inputs, g_ll, g_llobs)
+        grads = KalmanFilterGradOp(self.kind, self.strict_reference, self.has_c, self.has_d,
+                                   self.time_parallel)(*inputs, g_ll, g_llobs)
         if not isinstance(grads, (list, tuple)):
             grads = [grads]
         data_grad = pytensor.gradient.DisconnectedType()()
@@ -111,10 +114,11 @@ class KalmanFilterOp(Op):
 class KalmanFilterGradOp(Op):
     """(inputs..., g_loglik, g_ll_obs) -> cotangents of (a0, P0, T, Z, R, H, Q[, c][, d]) via kfb_backward."""
 
-    __props__ = ("kind", "strict_reference", "has_c", "has_d")
+    __props__ = ("kind", "strict_reference", "has_c", "has_d", "time_parallel")
 
-    def __init__(self, kind, strict_reference=True, has_c=False, has_d=False):
+    def __init__(self, kind, strict_reference=True, has_c=False, has_d=False, time_parallel=False):
         self.kind, self.strict_reference, self.has_c, self.has_d = kind, bool(strict_reference), bool(has_c), bool(has_d)
+        self.time_parallel = bool(time_parallel)
 
     def make_node(self, *inputs):
         _require()
@@ -136,6 +140,7 @@ class KalmanFilterGradOp(Op):
         arrs = arrs[:-2]
         flt = FILTER_FACTORY[self.kind]()
         flt.strict_reference = self.strict_reference
+        flt.time_parallel = self.time_parallel
         names = _input_names(self.has_c, self.has_d)
         # one loglik-only forward (hot-path kernels + tape) and the adjoint kernel, replayed as ONE CUDA graph with a single
         # pinned upload / download (seam.SeamGraph); no full-output pass, no autograd tape
@@ -156,5 +161,6 @@ def build_symbolic_graph(flt, data, a0, P0, T, Z, R, H, Q, c=None, d=None):
     ndims = {n: pt.as_tensor_variable(x).ndim for n, x in zip(_input_names(c is not None, d is not None), inputs)}
     if flt.kind in ("steady_state", "univariate") and any(ndims.get(k) == 3 for k in ("T", "Z", "R", "H", "Q", "c", "d")):
         raise ValueError("All system matrices must be time-invariant to use this filter")
-    op = KalmanFilterOp(flt.kind, flt.strict_reference, c is not None, d is not None)
+    op = KalmanFilterOp(flt.kind, flt.strict_reference, c is not None, d is not None,
+                        bool(getattr(flt, "time_parallel", False)))
     return list(op(*inputs))

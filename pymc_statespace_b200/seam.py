@@ -36,7 +36,7 @@ class SeamGraph:
         n, m, p, r, tv = flt._validate(meta["data"], *[meta.get(k) for k in MATRIX_NAMES])
         self.n, self.m, self.p = n, m, p
         self.bk = BatchedKalman(flt.kind, n, m, p, r, n_draws=1, strict_reference=flt.strict_reference, time_varying=tv,
-                                device=self.device)
+                                device=self.device, time_parallel=bool(getattr(flt, "time_parallel", False)))
         # ---- staging layout (float64 elements): inputs [data | matrices | g_loglik | g_ll_obs], outputs per mode
         self._in_names = ("data",) + self.present + (("g_loglik",) if mode == "grad" else ()) \
             + (("g_ll_obs",) if self.with_llobs else ())
@@ -129,7 +129,8 @@ def seam_graph(flt, arrays: Dict[str, np.ndarray], mode: str, with_llobs: bool =
     """The cached graph of this geometry (PyMC calls the Op once per leapfrog step with the same shapes)."""
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     shapes = {k: tuple(np.shape(a)) for k, a in arrays.items() if k == "data" or k in MATRIX_NAMES}
-    key = (flt.kind, bool(flt.strict_reference), mode, bool(with_llobs), str(dev), tuple(sorted(shapes.items())))
+    key = (flt.kind, bool(flt.strict_reference), bool(getattr(flt, "time_parallel", False)), mode, bool(with_llobs),
+           str(dev), tuple(sorted(shapes.items())))
     g = _CACHE.get(key)
     if g is None:
         if len(_CACHE) > 32:

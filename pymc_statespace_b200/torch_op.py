@@ -66,13 +66,14 @@ _BK_CACHE = {}
 def _evaluator(flt, n, m, p, r, tv, device):
     """One BatchedKalman (and its workspace) per problem geometry: PyMC calls the Op once per leapfrog step with the
     same shapes, so the evaluator and its device buffers are built once (ADVICE r1)."""
-    key = (flt.kind, n, m, p, r, bool(flt.strict_reference), tuple(tv), str(device))
+    tpar = bool(getattr(flt, "time_parallel", False))
+    key = (flt.kind, n, m, p, r, bool(flt.strict_reference), tpar, tuple(tv), str(device))
     bk = _BK_CACHE.get(key)
     if bk is None:
         if len(_BK_CACHE) > 64:
             _BK_CACHE.clear()
         bk = _BK_CACHE[key] = BatchedKalman(flt.kind, n, m, p, r, n_draws=1, strict_reference=flt.strict_reference,
-                                            time_varying=tv, device=device)
+                                            time_varying=tv, device=device, time_parallel=tpar)
     return bk
 
 
