@@ -165,6 +165,16 @@ kfb_status kfb_smoother(int64_t n_draws, int64_t n_series, int32_t n, int32_t m,
                         const double *filtered_states, const double *filtered_covs, double *smoothed_states,
                         double *smoothed_covs, void *workspace, size_t workspace_bytes, void *stream);
 
+/* kfb_smoother with flags (0: exactly kfb_smoother).  KFB_FLAG_TIME_PARALLEL: one CTA per unit and a blocked scan over
+ * time of the smoothing elements (Saerkkae & Garcia-Fernandez 2021), then a walk of every chunk with the literal RTS
+ * step; a unit whose scan disagrees with that walk (or meets a NaN) is re-run by the sequential recursion.  Faster for
+ * few units over long series; results agree with the sequential smoother to rounding.  k_states 1..4, else
+ * KFB_ERR_UNSUPPORTED; any other flag bit: KFB_ERR_INVALID_ARG.  Same workspace rule as kfb_smoother (no tape). */
+kfb_status kfb_smoother_ex(int64_t n_draws, int64_t n_series, int32_t n, int32_t m, int32_t r, const double *T,
+                           int64_t T_bs, const double *R, int64_t R_bs, const double *Q, int64_t Q_bs,
+                           const double *filtered_states, const double *filtered_covs, double *smoothed_states,
+                           double *smoothed_covs, void *workspace, size_t workspace_bytes, uint32_t flags, void *stream);
+
 /* Stationary initial covariance: X = A X A^T + C with C = R Q R^T
  * (reference models/SARIMAX.py:100-107, models/VARMAX.py:143-150:
  *  solve_discrete_lyapunov(T, R Q R^T, method="bilinear")).  X[B,m,m]; info[B] (0 ok, 1 = no

@@ -80,6 +80,8 @@ EXPORTS = {
                               ctypes.POINTER(KfbGrads), _vp, ctypes.c_size_t, _vp]),
     "kfb_smoother": (_c_i32, [_c_i64, _c_i64, _c_i32, _c_i32, _c_i32, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp, _vp,
                               _vp, ctypes.c_size_t, _vp]),
+    "kfb_smoother_ex": (_c_i32, [_c_i64, _c_i64, _c_i32, _c_i32, _c_i32, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp,
+                                 _vp, _vp, ctypes.c_size_t, ctypes.c_uint32, _vp]),
     "kfb_lyapunov_forward": (_c_i32, [_c_i64, _c_i32, _c_i32, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp]),
     "kfb_lyapunov_backward": (_c_i32, [_c_i64, _c_i32, _c_i32, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp,
                                        _vp, _vp, _vp]),

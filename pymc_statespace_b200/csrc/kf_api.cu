@@ -23,6 +23,8 @@ cudaError_t launch_p1_forward(const KfArgs& A, int y_smem_doubles, int bulk_ok, 
 
 bool tpar_supported(int m, int p, int mk);
 cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
+bool tpar_smoother_supported(int m);
+cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
 
 coopT_launch_fn coopT_launcher_m5(int p, int mk);
 coopT_launch_fn coopT_launcher_m6(int p, int mk);
@@ -388,9 +390,20 @@ kfb_status kfb_smoother(int64_t n_draws, int64_t n_series, int32_t n, int32_t m,
                         const double* R, int64_t R_bs, const double* Q, int64_t Q_bs, const double* filtered_states,
                         const double* filtered_covs, double* smoothed_states, double* smoothed_covs, void* workspace,
                         size_t workspace_bytes, void* stream) {
+  return kfb_smoother_ex(n_draws, n_series, n, m, r, T, T_bs, R, R_bs, Q, Q_bs, filtered_states, filtered_covs,
+                         smoothed_states, smoothed_covs, workspace, workspace_bytes, 0u, stream);
+}
+
+kfb_status kfb_smoother_ex(int64_t n_draws, int64_t n_series, int32_t n, int32_t m, int32_t r, const double* T,
+                           int64_t T_bs, const double* R, int64_t R_bs, const double* Q, int64_t Q_bs,
+                           const double* filtered_states, const double* filtered_covs, double* smoothed_states,
+                           double* smoothed_covs, void* workspace, size_t workspace_bytes, uint32_t flags, void* stream) {
   if (n_draws <= 0 || n_series <= 0 || n <= 0 || m <= 0 || r <= 0 || !T || !R || !Q || !filtered_states || !filtered_covs ||
       !smoothed_states || !smoothed_covs)
     return KFB_ERR_INVALID_ARG;
+  if (flags & ~KFB_FLAG_TIME_PARALLEL) return KFB_ERR_INVALID_ARG;
+  const bool tpar = (flags & KFB_FLAG_TIME_PARALLEL) != 0;
+  if (tpar && !tpar_smoother_supported(m)) return KFB_ERR_UNSUPPORTED;
   const bool C_batched = R_bs || Q_bs;
   const long long nDC = C_batched ? n_draws : 1;
   const size_t need = (size_t)nDC * m * m * sizeof(double);
@@ -403,8 +416,12 @@ kfb_status kfb_smoother(int64_t n_draws, int64_t n_series, int32_t n, int32_t m,
   S.T = MatArg{T, T_bs, 0};
   S.C = MatArg{(const double*)workspace, C_batched ? (long long)m * m : 0, 0};
   S.fs = filtered_states; S.fc = filtered_covs; S.ss = smoothed_states; S.sc = smoothed_covs;
-  const smoother_launch_fn per_thread = find_smoother_thread_launcher(m);
-  e = per_thread ? per_thread(S, s) : launch_smoother(S, s);
+  if (tpar) {
+    e = launch_tpar_smoother(S, s);
+  } else {
+    const smoother_launch_fn per_thread = find_smoother_thread_launcher(m);
+    e = per_thread ? per_thread(S, s) : launch_smoother(S, s);
+  }
   if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
 }

@@ -116,6 +116,70 @@ KFB_HD void chol_solve(X& x, const TM& Lw, TM& G, const TM& S, int m) {
   x.sync();
 }
 
+// The gain of one RTS step from the filtered (a, P) of step t: ah = T a, Ph = T P T^T + C and G = pinv(Ph) T P (the gain
+// is G^T).  W, V, Pinv are scratch; S1 is left holding T P.  T and C may be buffers or pointers to memory.
+template <class X, class TT, class TM, class TV>
+KFB_HD void smoother_gain(X& x, const TT& T, const TT& C, const TV& a, const TM& P, TV& ah, TM& Ph, TM& G, TM& W, TM& V,
+                          TM& Pinv, TM& S1) {
+  const int m = x.m();
+  KFB_FOR(i, m) {
+    double s = 0.0;
+    for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], a[k], s);
+    ah[i] = s;
+  }
+  gemm<false, false, 0>(x, S1, T, P, m, m, m);           // T P
+  KFB_FOR(i, m * m) Ph[i] = C[i];
+  x.sync();
+  gemm<false, true, 1>(x, Ph, S1, T, m, m, m);           // P_hat = T P T^T + C
+  KFB_FOR(idx, m * m) {
+    const int i = x.div_m(idx), j = idx - i * m;
+    W[idx] = 0.5 * (Ph[idx] + Ph[j * m + i]);
+  }
+  KFB_FOR(i, m * m) V[i] = W[i];
+  x.sync();
+  if (chol_factor(x, V, m)) {                            // sym(P_hat) positive definite: pinv = inverse
+    chol_solve(x, V, G, S1, m);                          // G = P_hat^-1 T P ; gain = G^T
+  } else {
+    x.sync();
+    jacobi_eigen(x, W, V, m);
+    double lmax = 0.0;
+    KFB_FOR(i, m) lmax = fmax(lmax, fabs(W[i * m + i]));
+    lmax = x.reduce_max(lmax);
+    const double cutoff = 1.0e-15 * lmax;
+    KFB_FOR(idx, m * m) {                                // Pinv = V diag(1/lambda) V^T
+      const int i = x.div_m(idx), j = idx - i * m;
+      double s = 0.0;
+      for (int k = 0; k < m; ++k) {
+        const double lam = W[k * m + k];
+        if (fabs(lam) > cutoff) s = kf_fma(V[i * m + k] / lam, V[j * m + k], s);
+      }
+      Pinv[idx] = s;
+    }
+    x.sync();
+    gemm<false, false, 0>(x, G, Pinv, S1, m, m, m);      // G = pinv(P_hat) T P ; gain = G^T
+  }
+}
+
+// The RTS update in place on (as, Ps), the smoothed moments of step t+1 on entry and of step t on return:
+// a_s = a + G^T (a_s' - a_hat), P_s = P + G^T (P_s' - P_hat) G.  da, W, S1 are scratch.
+template <class X, class TM, class TV>
+KFB_HD void smoother_update(X& x, const TM& G, const TV& a, const TM& P, const TV& ah, const TM& Ph, TV& as, TM& Ps,
+                            TV& da, TM& W, TM& S1) {
+  const int m = x.m();
+  KFB_FOR(i, m) da[i] = as[i] - ah[i];
+  KFB_FOR(i, m * m) W[i] = Ps[i] - Ph[i];
+  x.sync();
+  KFB_FOR(i, m) {                                        // a_s = a + G^T (a_s' - a_hat)
+    double s = a[i];
+    for (int k = 0; k < m; ++k) s = kf_fma(G[k * m + i], da[k], s);
+    as[i] = s;
+  }
+  gemm<true, false, 0>(x, S1, G, W, m, m, m);            // G^T (P_s' - P_hat)
+  KFB_FOR(i, m * m) Ps[i] = P[i];
+  x.sync();
+  gemm<false, false, 1>(x, Ps, S1, G, m, m, m);          // P_s = P + G^T (.) G
+}
+
 template <class X>
 KFB_HD void smoother_unit(X& x, const SmoothArgs& A, long long u) {
   const int m = x.m(), n = A.n;
@@ -135,54 +199,8 @@ KFB_HD void smoother_unit(X& x, const SmoothArgs& A, long long u) {
     KFB_FOR(i, m) a[i] = fs[(long long)t * m + i];
     KFB_FOR(i, m * m) P[i] = fc[(long long)t * m * m + i];
     x.sync();
-    KFB_FOR(i, m) {
-      double s = 0.0;
-      for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], a[k], s);
-      ah[i] = s;
-    }
-    gemm<false, false, 0>(x, S1, T, P, m, m, m);           // T P
-    KFB_FOR(i, m * m) Ph[i] = C[i];
-    x.sync();
-    gemm<false, true, 1>(x, Ph, S1, T, m, m, m);           // P_hat = T P T^T + C
-    KFB_FOR(idx, m * m) {
-      const int i = x.div_m(idx), j = idx - i * m;
-      W[idx] = 0.5 * (Ph[idx] + Ph[j * m + i]);
-    }
-    KFB_FOR(i, m * m) V[i] = W[i];
-    x.sync();
-    if (chol_factor(x, V, m)) {                            // sym(P_hat) positive definite: pinv = inverse
-      chol_solve(x, V, G, S1, m);                          // G = P_hat^-1 T P ; gain = G^T
-    } else {
-      x.sync();
-      jacobi_eigen(x, W, V, m);
-      double lmax = 0.0;
-      KFB_FOR(i, m) lmax = fmax(lmax, fabs(W[i * m + i]));
-      lmax = x.reduce_max(lmax);
-      const double cutoff = 1.0e-15 * lmax;
-      KFB_FOR(idx, m * m) {                                // Pinv = V diag(1/lambda) V^T
-        const int i = x.div_m(idx), j = idx - i * m;
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) {
-          const double lam = W[k * m + k];
-          if (fabs(lam) > cutoff) s = kf_fma(V[i * m + k] / lam, V[j * m + k], s);
-        }
-        Pinv[idx] = s;
-      }
-      x.sync();
-      gemm<false, false, 0>(x, G, Pinv, S1, m, m, m);      // G = pinv(P_hat) T P ; gain = G^T
-    }
-    KFB_FOR(i, m) da[i] = as[i] - ah[i];
-    KFB_FOR(i, m * m) W[i] = Ps[i] - Ph[i];
-    x.sync();
-    KFB_FOR(i, m) {                                        // a_s = a + G^T (a_s' - a_hat)
-      double s = a[i];
-      for (int k = 0; k < m; ++k) s = kf_fma(G[k * m + i], da[k], s);
-      as[i] = s;
-    }
-    gemm<true, false, 0>(x, S1, G, W, m, m, m);            // G^T (P_s' - P_hat)
-    KFB_FOR(i, m * m) Ps[i] = P[i];
-    x.sync();
-    gemm<false, false, 1>(x, Ps, S1, G, m, m, m);          // P_s = P + G^T (.) G
+    smoother_gain(x, T, C, a, P, ah, Ph, G, W, V, Pinv, S1);
+    smoother_update(x, G, a, P, ah, Ph, as, Ps, da, W, S1);
     KFB_FOR(i, m) ss[(long long)t * m + i] = as[i];
     KFB_FOR(i, m * m) sc[(long long)t * m * m + i] = Ps[i];
     x.sync();

@@ -276,10 +276,24 @@ class BatchedKalman:
         return grads
 
 
-def rts_smoother(T, R, Q, filtered_states, filtered_covs, n_series: int = 1):
+TIME_PARALLEL_SMOOTHER_MAX_STATES = 4  # kfb_smoother_ex with KFB_FLAG_TIME_PARALLEL covers k_states 1..4
+
+
+def smoother_workspace_numel(n_draws: int, m: int) -> int:
+    """float64 elements of the workspace rts_smoother needs (R Q R^T per draw; enough whether or not R, Q are shared)."""
+    return max(n_draws, 1) * m * m
+
+
+def rts_smoother(T, R, Q, filtered_states, filtered_covs, n_series: int = 1, time_parallel: bool = False, out=None,
+                 workspace=None):
     """Batched RTS smoother (reference filters/kalman_smoother.py:56-104; SURVEY section 8(f) row f2).
     T:[B,m,m]|[m,m], R:[B,m,r]|[m,r], Q:[B,r,r]|[r,r] static; filtered_states [U,n,m], filtered_covs [U,n,m,m]
-    (outputs of BatchedKalman.forward).  Returns (smoothed_states [U,n,m], smoothed_covs [U,n,m,m])."""
+    (outputs of BatchedKalman.forward).  Returns (smoothed_states [U,n,m], smoothed_covs [U,n,m,m]).
+
+    ``time_parallel=True`` runs the time-parallel kernel (one CTA per unit, a scan over time; faster for few units over
+    long series) for k_states <= 4; at larger k_states the sequential kernel runs, as BatchedKalman falls back.
+    ``out=(ss, sc)`` and ``workspace`` (float64, ``smoother_workspace_numel(n_draws, m)`` elements) may be preallocated, so
+    that a CUDA graph can capture the call without allocating."""
     lib = load()
     fs, fc = filtered_states.contiguous(), filtered_covs.contiguous()
     U, n, m = fs.shape
@@ -289,12 +303,21 @@ def rts_smoother(T, R, Q, filtered_states, filtered_covs, n_series: int = 1):
     for name, t, nd in (("T", T, 2), ("R", R, 2), ("Q", Q, 2)):
         if t.ndim == nd + 1 and t.shape[0] != n_draws:
             raise ValueError(f"{name}: leading dimension {t.shape[0]} != n_draws {n_draws}")
-    ss, sc = torch.empty_like(fs), torch.empty_like(fc)
-    ws = torch.empty(max(n_draws, 1) * m * m, dtype=torch.float64, device=fs.device)
+    if out is None:
+        ss, sc = torch.empty_like(fs), torch.empty_like(fc)
+    else:
+        ss, sc = out
+        if ss.shape != fs.shape or sc.shape != fc.shape or not (ss.is_contiguous() and sc.is_contiguous()):
+            raise ValueError("out: contiguous tensors of the shapes of filtered_states and filtered_covs")
+    ws = workspace
+    if ws is None:
+        ws = torch.empty(smoother_workspace_numel(n_draws, m), dtype=torch.float64, device=fs.device)
+    flags = KFB_FLAG_TIME_PARALLEL if time_parallel and m <= TIME_PARALLEL_SMOOTHER_MAX_STATES else 0
     with torch.cuda.device(fs.device):
-        check(lib.kfb_smoother(n_draws, n_series, n, m, r, _ptr(T), m * m if T.ndim == 3 else 0, _ptr(R),
-                               m * r if R.ndim == 3 else 0, _ptr(Q), r * r if Q.ndim == 3 else 0, _ptr(fs), _ptr(fc),
-                               _ptr(ss), _ptr(sc), _ptr(ws), ws.numel() * 8, _stream_ptr(fs.device)), "kfb_smoother")
+        check(lib.kfb_smoother_ex(n_draws, n_series, n, m, r, _ptr(T), m * m if T.ndim == 3 else 0, _ptr(R),
+                                  m * r if R.ndim == 3 else 0, _ptr(Q), r * r if Q.ndim == 3 else 0, _ptr(fs), _ptr(fc),
+                                  _ptr(ss), _ptr(sc), _ptr(ws), ws.numel() * 8, flags, _stream_ptr(fs.device)),
+              "kfb_smoother_ex")
     return ss, sc
 
 

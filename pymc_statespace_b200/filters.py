@@ -178,29 +178,41 @@ class UnivariateFilter(BaseFilter):
 
 
 class KalmanSmoother:
-    """reference pymc_statespace/filters/kalman_smoother.py:11-104 (static T, R, Q; numpy or torch inputs, eager).
+    """reference pymc_statespace/filters/kalman_smoother.py:11-104 (static T, R, Q).
     ``build_graph(T, R, Q, filtered_states[n,m,1], filtered_covariances[n,m,m])`` ->
-    ``[smoothed_states[n,m,1], smoothed_covariances[n,m,m]]``.  Not on the logp/grad path (SURVEY section 8(f) f2)."""
+    ``[smoothed_states[n,m,1], smoothed_covariances[n,m,m]]``.  Not on the logp/grad path (SURVEY section 8(f) f2).
+
+    PyTensor inputs give the two symbolic outputs of ``KalmanSmootherOp`` (no gradient through them); numpy inputs run
+    one replayed CUDA graph (``seam.smooth_numpy``); torch inputs run eagerly."""
 
     def __init__(self, mode=None):
         self.mode = mode
         self.seq_names: List[str] = []
         self.non_seq_names: List[str] = []
+        # opt-in time-parallel kernel (k_states <= 4): faster for one draw per call over long series
+        self.time_parallel = False
 
     def build_graph(self, T, R, Q, filtered_states, filtered_covariances, mode=None):
+        self.mode = mode
+        args = [T, R, Q, filtered_states, filtered_covariances]
+        if any(_is_pytensor_variable(x) for x in args):
+            from .pytensor_op import build_smoother_graph
+
+            return build_smoother_graph(self, *args)
         import torch
 
         from .engine import rts_smoother
 
-        self.mode = mode
-        args = [T, R, Q, filtered_states, filtered_covariances]
-        if any(_is_pytensor_variable(x) for x in args):
-            raise NotImplementedError("the B200 smoother is eager (numpy / torch inputs); keep the reference's "
-                                      "KalmanSmoother for symbolic graphs")
         _, _, self.seq_names, self.non_seq_names = split_vars_into_seq_and_nonseq([T, R, Q], ["T", "R", "Q"])
         if self.seq_names:
             raise NotImplementedError("time-varying T, R, Q are not supported by the B200 smoother")
         as_numpy = not any(isinstance(x, torch.Tensor) for x in args)
+        if as_numpy:
+            if not torch.cuda.is_available():
+                raise RuntimeError("pymc_statespace_b200 needs a CUDA device (no CPU fallback)")
+            from .seam import smooth_numpy
+
+            return smooth_numpy(*[np.asarray(x, dtype=np.float64) for x in args], time_parallel=self.time_parallel)
         dev = next((x.device for x in args if isinstance(x, torch.Tensor) and x.is_cuda), None)
         if dev is None:
             if not torch.cuda.is_available():
@@ -209,9 +221,9 @@ class KalmanSmoother:
         prep = lambda x: (x if isinstance(x, torch.Tensor) else torch.as_tensor(np.ascontiguousarray(  # noqa: E731
             np.asarray(x, dtype=np.float64)))).to(device=dev, dtype=torch.float64)
         T, R, Q, fs, fc = (prep(x) for x in args)
-        ss, sc = rts_smoother(T, R, Q, fs[None, :, :, 0].contiguous(), fc[None].contiguous())
-        out = [ss[0][..., None], sc[0]]
-        return [o.cpu().numpy() for o in out] if as_numpy else out
+        ss, sc = rts_smoother(T, R, Q, fs[None, :, :, 0].contiguous(), fc[None].contiguous(),
+                              time_parallel=self.time_parallel)
+        return [ss[0][..., None], sc[0]]
 
 
 # reference pymc_statespace/core/statespace.py:25-31

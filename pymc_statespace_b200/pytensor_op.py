@@ -164,3 +164,50 @@ def build_symbolic_graph(flt, data, a0, P0, T, Z, R, H, Q, c=None, d=None):
     op = KalmanFilterOp(flt.kind, flt.strict_reference, c is not None, d is not None,
                         bool(getattr(flt, "time_parallel", False)))
     return list(op(*inputs))
+
+
+class KalmanSmootherOp(Op):
+    """(T, R, Q, filtered_states[n,m,1], filtered_covariances[n,m,m]) -> [smoothed_states[n,m,1],
+    smoothed_covariances[n,m,m]]: the RTS smoother of KalmanSmoother.build_graph (reference kalman_smoother.py:56-104),
+    one replayed CUDA graph per call (seam.smooth_numpy).  Not differentiable."""
+
+    __props__ = ("time_parallel",)
+
+    def __init__(self, time_parallel=False):
+        self.time_parallel = bool(time_parallel)
+
+    def make_node(self, T, R, Q, filtered_states, filtered_covariances):
+        _require()
+        inputs = [pt.as_tensor_variable(x) for x in (T, R, Q, filtered_states, filtered_covariances)]
+        from pytensor.tensor.type import TensorType
+
+        outs = [TensorType("float64", shape=(None, None, None))() for _ in range(2)]
+        return Apply(self, inputs, outs)
+
+    def infer_shape(self, fgraph, node, shapes):
+        n, m = shapes[4][0], shapes[4][1]  # filtered_covariances [n, m, m]; perform returns [n, m, 1] and [n, m, m]
+        return [(n, m, 1), (n, m, m)]
+
+    def perform(self, node, inputs, output_storage):
+        from .seam import smooth_numpy  # CUDA is initialised here, in the process that evaluates the graph
+
+        outs = smooth_numpy(*[np.asarray(x, dtype=np.float64) for x in inputs], time_parallel=self.time_parallel)
+        for storage, o in zip(output_storage, outs):
+            storage[0] = np.asarray(o, dtype=np.float64)
+
+    def L_op(self, inputs, outputs, output_grads):
+        for g, name in zip(output_grads, ("smoothed_states", "smoothed_covariances")):
+            if not isinstance(g.type, DisconnectedType):
+                raise NotImplementedError(
+                    f"gradient through {name} is not implemented: the smoothed moments are Deterministics of the "
+                    "reference model, evaluated per saved draw, and are not differentiable here")
+        return [pytensor.gradient.DisconnectedType()() for _ in inputs]
+
+
+def build_smoother_graph(smoother, T, R, Q, filtered_states, filtered_covariances):
+    """What KalmanSmoother.build_graph returns for PyTensor inputs: the 2 symbolic outputs of one KalmanSmootherOp."""
+    _require()
+    if any(pt.as_tensor_variable(x).ndim == 3 for x in (T, R, Q)):
+        raise NotImplementedError("time-varying T, R, Q are not supported by the B200 smoother")
+    op = KalmanSmootherOp(bool(getattr(smoother, "time_parallel", False)))
+    return list(op(T, R, Q, filtered_states, filtered_covariances))

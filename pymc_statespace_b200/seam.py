@@ -20,6 +20,21 @@ from .engine import MATRIX_NAMES, BatchedKalman
 _SIX = ("filtered_states", "predicted_states", "filtered_covs", "predicted_covs", "loglik", "ll_obs")
 
 
+def _stage(device, names: Sequence[str], shapes):
+    """One pinned host buffer and one device buffer holding the named arrays back to back, with numpy / torch views."""
+    sizes = [int(np.prod(shapes[k])) for k in names]
+    total = max(sum(sizes), 1)
+    host = torch.empty(total, dtype=torch.float64).pin_memory()
+    dev = torch.empty(total, dtype=torch.float64, device=device)
+    host_np, dev_v, off = {}, {}, 0
+    hn = host.numpy()
+    for k, sz in zip(names, sizes):
+        host_np[k] = hn[off:off + sz].reshape(shapes[k])
+        dev_v[k] = dev[off:off + sz].view(shapes[k])
+        off += sz
+    return host, dev, host_np, dev_v
+
+
 class SeamGraph:
     """One problem geometry, one replayable graph.  ``mode="six"``: the reference's six outputs;
     ``mode="grad"``: loglik + cotangents of every matrix passed, for ``g_loglik * loglik + g_ll_obs . ll_obs``."""
@@ -52,8 +67,8 @@ class SeamGraph:
                 out_shapes["g_" + k] = (1,) + ((n,) if k in tv else ()) + self.bk._base[k]
             self._out_names = ("loglik",) + tuple("g_" + k for k in self.present)
         self._out_shapes = out_shapes
-        self.hin, self.din, self._hin_np, self._din_v = self._stage(self._in_names, self._in_shapes)
-        self.hout, self.dout, self._hout_np, self._dout_v = self._stage(self._out_names, out_shapes)
+        self.hin, self.din, self._hin_np, self._din_v = _stage(self.device, self._in_names, self._in_shapes)
+        self.hout, self.dout, self._hout_np, self._dout_v = _stage(self.device, self._out_names, out_shapes)
         self.hinfo = torch.zeros(1, dtype=torch.int32).pin_memory()
         self.dinfo = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._user_shapes = {k: tuple(shapes[k]) for k in self.present}
@@ -72,19 +87,6 @@ class SeamGraph:
         with torch.cuda.graph(self.graph, stream=side):
             self._enqueue()
         torch.cuda.current_stream(self.device).wait_stream(side)
-
-    def _stage(self, names: Sequence[str], shapes):
-        sizes = [int(np.prod(shapes[k])) for k in names]
-        total = max(sum(sizes), 1)
-        host = torch.empty(total, dtype=torch.float64).pin_memory()
-        dev = torch.empty(total, dtype=torch.float64, device=self.device)
-        host_np, dev_v, off = {}, {}, 0
-        hn = host.numpy()
-        for k, sz in zip(names, sizes):
-            host_np[k] = hn[off:off + sz].reshape(shapes[k])
-            dev_v[k] = dev[off:off + sz].view(shapes[k])
-            off += sz
-        return host, dev, host_np, dev_v
 
     def _enqueue(self):
         v = self._din_v
@@ -160,3 +162,80 @@ def logp_grads_numpy(flt, arrays: Dict[str, np.ndarray], g_loglik=1.0, g_ll_obs:
     g = seam_graph(flt, arrays, "grad", with_llobs=use_llobs, device=device)
     o = g(call)
     return float(o["loglik"]), {k: o["g_" + k] for k in g.present}
+
+
+class SmoothSeamGraph:
+    """The RTS smoother of one geometry at one unit per call (what PyMC's per-draw evaluation of the smoothed
+    ``pm.Deterministic``s sends): one pinned upload of [T | R | Q | filtered_states | filtered_covs], the R Q R^T hoist and
+    the smoother kernel, one pinned download, replayed as one CUDA graph."""
+
+    def __init__(self, shapes: Dict[str, Tuple[int, ...]], time_parallel: bool = False, device=None):
+        from .engine import rts_smoother, smoother_workspace_numel
+
+        self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        if self.device.type != "cuda":
+            raise RuntimeError("pymc_statespace_b200 needs a CUDA device (no CPU fallback)")
+        self.time_parallel = bool(time_parallel)
+        n, m = shapes["fc"][0], shapes["fc"][-1]
+        self.n, self.m = n, m
+        self._in_names = ("T", "R", "Q", "fs", "fc")
+        self._in_shapes = {"T": tuple(shapes["T"]), "R": tuple(shapes["R"]), "Q": tuple(shapes["Q"]), "fs": (1, n, m),
+                           "fc": (1, n, m, m)}
+        self._out_names = ("ss", "sc")
+        self._out_shapes = {"ss": (1, n, m), "sc": (1, n, m, m)}
+        self.hin, self.din, self._hin_np, self._din_v = _stage(self.device, self._in_names, self._in_shapes)
+        self.hout, self.dout, self._hout_np, self._dout_v = _stage(self.device, self._out_names, self._out_shapes)
+        self._ws = torch.empty(smoother_workspace_numel(1, m), dtype=torch.float64, device=self.device)
+        self._smooth = rts_smoother
+        side = torch.cuda.Stream(self.device)
+        side.wait_stream(torch.cuda.current_stream(self.device))
+        self.hin.zero_()
+        self._hin_np["Q"][...] = np.eye(self._in_shapes["Q"][-1])  # a well-posed dummy problem for the warm-up runs
+        self._hin_np["fc"][...] = np.eye(m)
+        with torch.cuda.stream(side):
+            self._enqueue()
+            self._enqueue()
+        side.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph, stream=side):
+            self._enqueue()
+        torch.cuda.current_stream(self.device).wait_stream(side)
+
+    def _enqueue(self):
+        v = self._din_v
+        self.din.copy_(self.hin, non_blocking=True)
+        self._smooth(v["T"], v["R"], v["Q"], v["fs"], v["fc"], time_parallel=self.time_parallel,
+                     out=(self._dout_v["ss"], self._dout_v["sc"]), workspace=self._ws)
+        self.hout.copy_(self.dout, non_blocking=True)
+
+    def __call__(self, arrays: Dict[str, np.ndarray]) -> Dict[str, np.ndarray]:
+        """``arrays``: T, R, Q, fs [n,m(,1)], fc [n,m,m].  Returns fresh numpy arrays ss [n,m], sc [n,m,m]."""
+        for k in self._in_names:
+            np.copyto(self._hin_np[k], np.asarray(arrays[k], dtype=np.float64).reshape(self._in_shapes[k]))
+        with torch.cuda.device(self.device):
+            self.graph.replay()
+            torch.cuda.current_stream(self.device).synchronize()
+        return {k: np.array(self._hout_np[k][0]) for k in self._out_names}
+
+
+_SMOOTH_CACHE: Dict[tuple, SmoothSeamGraph] = {}
+
+
+def smooth_graph(arrays: Dict[str, np.ndarray], time_parallel: bool = False, device=None) -> SmoothSeamGraph:
+    """The cached smoother graph of this geometry, keyed by (time_parallel, shapes, device)."""
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    shapes = {k: tuple(np.shape(arrays[k])) for k in ("T", "R", "Q", "fs", "fc")}
+    key = (bool(time_parallel), tuple(sorted(shapes.items())), str(dev))
+    g = _SMOOTH_CACHE.get(key)
+    if g is None:
+        if len(_SMOOTH_CACHE) > 32:
+            _SMOOTH_CACHE.clear()
+        g = _SMOOTH_CACHE[key] = SmoothSeamGraph(shapes, time_parallel, dev)
+    return g
+
+
+def smooth_numpy(T, R, Q, filtered_states, filtered_covariances, time_parallel: bool = False, device=None):
+    """numpy in -> the reference's [smoothed_states[n,m,1], smoothed_covariances[n,m,m]] (kalman_smoother.py:56-104)."""
+    arrays = {"T": T, "R": R, "Q": Q, "fs": filtered_states, "fc": filtered_covariances}
+    o = smooth_graph(arrays, time_parallel, device)(arrays)
+    return [o["ss"][..., None], o["sc"]]
