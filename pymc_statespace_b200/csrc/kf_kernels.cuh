@@ -1,4 +1,4 @@
-// kf_kernels.cuh - __global__ wrappers around forward_unit / backward_unit (kf_core.cuh).
+// kf_kernels.cuh - __global__ wrappers around forward_unit / backward_unit (kf_core.cuh), and CTA-wide helpers.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -50,6 +50,38 @@ __device__ __forceinline__ void stage_y(double* ysm, const double* ysrc, int cou
   }
   for (int i = bulk_doubles + threadIdx.x; i < count; i += blockDim.x) ysm[i] = ysrc[i];
   __syncthreads();
+}
+
+// Inclusive scan of one element per thread across an NT-thread CTA (Hillis-Steele, fixed order, so reruns give identical
+// bits): a prefix scan, sh[tid] <- sh[0] (x) .. (x) sh[tid], or with SUFFIX a suffix scan, sh[tid] <- sh[tid] (x) .. (x)
+// sh[NT-1].  On entry sh[tid] holds this thread's element (the scan synchronises before reading it); on exit, its
+// inclusive scan.  combine(lower, higher, out) gets the lower index first; out does not alias either operand.
+template <class Elem, int NT, bool SUFFIX, class Combine>
+__device__ __forceinline__ void cta_scan(Elem* sh, Combine combine) {
+  const int tid = threadIdx.x;
+  Elem agg, tmp;
+  __syncthreads();
+  agg = sh[tid];
+  for (int off = 1; off < NT; off <<= 1) {
+    const bool active = SUFFIX ? tid + off < NT : tid >= off;
+    if (active) {
+      if constexpr (SUFFIX) combine(agg, sh[tid + off], tmp);
+      else combine(sh[tid - off], agg, tmp);
+    }
+    __syncthreads();
+    if (active) { agg = tmp; sh[tid] = agg; }
+    __syncthreads();
+  }
+}
+
+// Fixed-order CTA tree sum of `w` doubles per thread (red[tid * w + k]); the result is left in red[0 .. w-1].
+template <int NT>
+__device__ __forceinline__ void cta_sum(double* red, int w) {
+  for (int s = NT / 2; s > 0; s >>= 1) {
+    if ((int)threadIdx.x < s)
+      for (int k = 0; k < w; ++k) red[threadIdx.x * w + k] += red[(threadIdx.x + s) * w + k];
+    __syncthreads();
+  }
 }
 
 // MODE: 0 = forward, loglik (+tape) only; 1 = forward with per-step outputs; 2 = adjoint.

@@ -29,8 +29,12 @@
 // of the literal one-step adjoint (adjoint_step, the p = 1 instance of kf_pred.cuh's step) reduced in a fixed order.
 // Step 0 runs that literal adjoint, so abar_0 and the full-matrix Pbar_0 (non-symmetric P0) are the sequential ones.
 //
-// Everything here is KFB_HD so that tests/tpar_host compiles it for the host and checks it against the oracle.
+// Each phase of a pass is a function over one chunk [lo, hi) of one unit (filt_fold_chunk .. adjoint_chunk); the kernels
+// of kf_tpar.cu add only the CTA scans, the fallback decisions and the reductions.  Everything here is KFB_HD so that
+// tests/tpar_host runs the same chunk functions on the host, with its own scans, and checks them against the oracle.
 #pragma once
+#include <climits>
+
 #include "kf_ctx.cuh"
 #include "kf_pred.cuh"
 
@@ -39,6 +43,22 @@ namespace tpar {
 
 template <int M>
 using TX = ThreadCtx<M, 1, false>;
+
+// Threads per CTA of the time-parallel kernels (filter and smoother): 256 while one thread's operands fit the register
+// file; the filtering element of k_states 3 / 4 is 33 / 56 doubles, and the smoother's gain buffers and aggregates no
+// longer fit either, so those run 128 threads (a few more steps per thread, one scan level less).
+template <int M>
+KFB_HD constexpr int tpar_threads() { return M <= 2 ? 256 : 128; }
+
+// Steps [lo, hi) of chunk k of K over n steps: contiguous chunks of ceil(n / K) steps; the last ones may be short or empty.
+struct Chunk {
+  int lo, hi;
+};
+KFB_HD Chunk chunk_of(int k, int K, int n) {
+  const int len = (n + K - 1) / K;
+  const int lo = k * len < n ? k * len : n;
+  return {lo, lo + len < n ? lo + len : n};
+}
 
 // one unit's inputs (k_endog = 1); time strides 0 = static
 struct UnitView {
@@ -410,6 +430,41 @@ KFB_HD void forward_sequential_tape(const UnitView& v, double* tape) {
   }
 }
 
+// The aggregate e_lo (x) .. (x) e_{hi-1} of a chunk's filtering elements (the identity if the chunk is empty).  Returns
+// false if one of them is undefined.
+template <int M>
+KFB_HD bool filt_fold_chunk(const UnitView& v, int lo, int hi, FiltElem<M>& agg) {
+  FiltElem<M> e, tmp;
+  filt_identity<M>(agg);
+  bool undefined = false;
+  for (int t = lo; t < hi; ++t) {
+    if (t == 0) filt_element0<M>(v, e);
+    else undefined |= !filt_element<M>(v, t, e);
+    if (t == lo) agg = e;
+    else { filt_combine<M>(agg, e, tmp); agg = tmp; }
+  }
+  return !undefined;
+}
+
+// Re-runs a chunk from `prefix`, the scanned aggregate of all steps before lo (unused if lo == 0): the filtered moments
+// of every step, written to the tape as the predicted moments of the step after it.  Tape entry 0 is (a0, P0).
+template <int M>
+KFB_HD void filt_rerun_chunk(const UnitView& v, int lo, int hi, const FiltElem<M>* prefix, double* tape) {
+  FiltElem<M> f, e, tmp;
+  for (int t = lo; t < hi; ++t) {
+    if (t == 0) {
+      filt_element0<M>(v, f);
+      for (int i = 0; i < M; ++i) tape[i] = v.a0[i];
+      for (int i = 0; i < M * M; ++i) tape[M + i] = v.P0[i];
+    } else {
+      filt_element<M>(v, t, e);
+      filt_combine<M>(t == lo ? *prefix : f, e, tmp);
+      f = tmp;
+    }
+    if (t + 1 < v.n) predict_to_tape<M>(v, t, f.b, f.C, tape + (long long)(t + 1) * tape_entry<M>());
+  }
+}
+
 // Per-step forward outputs from the tape entry of step t (the literal update of kf_core.cuh).  Returns ll_t; *bad is set
 // if F_t is not a positive finite number.
 struct FwdOut {
@@ -421,6 +476,24 @@ struct FwdOut {
 // expanding (an MA coefficient |theta| > 1 makes A = (I - K Z) T grow like theta^k over a chunk while the filter itself
 // stays stable), and the scan's moments then drift by 1e-8 .. 1e+10.
 constexpr double TPAR_DRIFT_TOL = 1e-10;
+
+// True if (a, P) differs from (a_ref, P_ref) by more than tol relative to the scale of (a, P): max|P| for P, and
+// max(max|a|, sqrt max|P|) for a.  A NaN on either side counts as drift.
+template <int M>
+KFB_HD bool drifted(const double* a, const double* P, const double* a_ref, const double* P_ref, double tol) {
+  double sP = 0.0, sa = 0.0;
+#pragma unroll
+  for (int i = 0; i < M * M; ++i) sP = fmax(sP, fabs(P[i]));
+#pragma unroll
+  for (int i = 0; i < M; ++i) sa = fmax(sa, fabs(a[i]));
+  sa = fmax(sa, sqrt(sP));
+  bool ok = true;  // a NaN on either side fails its comparison
+#pragma unroll
+  for (int i = 0; i < M * M; ++i) ok = ok && (fabs(P[i] - P_ref[i]) <= tol * sP);
+#pragma unroll
+  for (int i = 0; i < M; ++i) ok = ok && (fabs(a[i] - a_ref[i]) <= tol * sa);
+  return !ok;
+}
 
 // *drift is set if `next` (tape entry t + 1; null: no check) is not one literal step from `entry` to within
 // TPAR_DRIFT_TOL (relative to the predicted moments; a NaN counts as drift).
@@ -457,25 +530,33 @@ KFB_HD double forward_map_step(const UnitView& v, int t, const double* entry, co
   if (o.pc) for (int i = 0; i < M * M; ++i) o.pc[(long long)t * M * M + i] = P[i];
   if (!next && !(t == v.n - 1 && (o.ps || o.pc))) return ll;
   predict(x, prm.T, C, c, af, Pf, a, P, tmp.S1, tmp.S2);
-  if (next) {
-    double sP = 0.0, sa = 0.0;
-#pragma unroll
-    for (int i = 0; i < M * M; ++i) sP = fmax(sP, fabs(P[i]));
-#pragma unroll
-    for (int i = 0; i < M; ++i) sa = fmax(sa, fabs(a[i]));
-    sa = fmax(sa, sqrt(sP));
-    bool ok = true;  // a NaN on either side fails its comparison
-#pragma unroll
-    for (int i = 0; i < M * M; ++i) ok = ok && (fabs(P[i] - next[M + i]) <= TPAR_DRIFT_TOL * sP);
-#pragma unroll
-    for (int i = 0; i < M; ++i) ok = ok && (fabs(a[i] - next[i]) <= TPAR_DRIFT_TOL * sa);
-    *drift = !ok;
-  }
+  if (next) *drift = drifted<M>(&a[0], &P[0], next, next + M, TPAR_DRIFT_TOL);
   if (t == v.n - 1) {
     if (o.ps) for (int i = 0; i < M; ++i) o.ps[(long long)(t + 1) * M + i] = a[i];
     if (o.pc) for (int i = 0; i < M * M; ++i) o.pc[(long long)(t + 1) * M * M + i] = P[i];
   }
   return ll;
+}
+
+// forward_map_step over a chunk in step order, with the check if `check`.  Returns true if a step drifted; *ll receives
+// the chunk's sum of ll_t and *first_bad its first step with a bad F_t (INT_MAX: none).
+template <int M>
+KFB_HD bool forward_map_chunk(const UnitView& v, int lo, int hi, const double* tape, bool check, const FwdOut& o,
+                              double* ll, int* first_bad) {
+  constexpr int E = tape_entry<M>();
+  double s = 0.0;
+  int fb = INT_MAX;
+  bool drift_any = false;
+  for (int t = lo; t < hi; ++t) {
+    bool bad, drift;
+    const double* next = (check && t + 1 < v.n) ? tape + (long long)(t + 1) * E : nullptr;
+    s += forward_map_step<M>(v, t, tape + (long long)t * E, next, o, &bad, &drift);
+    if (bad && fb == INT_MAX) fb = t;
+    drift_any |= drift;
+  }
+  *ll = s;
+  *first_bad = fb;
+  return drift_any;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -799,6 +880,103 @@ KFB_HD void adjoint_step(const BwdStep<M>& B, double ds, const double* ab, const
         Pb_prev[i * M + j] = s;
       }
   }
+}
+
+// The aggregate f_lo o .. o f_{hi-1} of a chunk's abar elements, folded from hi-1 down (the identity if it is empty).
+template <int M>
+KFB_HD void aff_fold_chunk(const UnitView& v, int lo, int hi, const double* tape, double gl, const double* gllo,
+                           AffElem<M>& agg) {
+  TX<M> x{nullptr, nullptr, 0, 1};
+  BwdStep<M> B(x);
+  AffElem<M> e, tmp;
+  aff_identity<M>(agg);
+  for (int t = hi - 1; t >= lo; --t) {
+    bwd_load<M>(x, v, t, tape + (long long)t * tape_entry<M>(), gl, gllo, B);
+    aff_element<M>(B, e);
+    if (t == hi - 1) agg = e;
+    else { aff_combine<M>(e, agg, tmp); agg = tmp; }
+  }
+}
+
+// The aggregate of a chunk's congruence elements for sym(Pbar).  Their forcing needs abar_{t+1}, which is walked down
+// from ab_hi (abar at hi).
+template <int M>
+KFB_HD void cong_fold_chunk(const UnitView& v, int lo, int hi, const double* tape, double gl, const double* gllo,
+                            const double* ab_hi, CongElem<M>& agg) {
+  TX<M> x{nullptr, nullptr, 0, 1};
+  BwdStep<M> B(x);
+  CongElem<M> e, tmp;
+  double ab[M], abn[M];
+  cong_identity<M>(agg);
+  for (int i = 0; i < M; ++i) ab[i] = ab_hi[i];
+  for (int t = hi - 1; t >= lo; --t) {
+    bwd_load<M>(x, v, t, tape + (long long)t * tape_entry<M>(), gl, gllo, B);
+    cong_element<M>(B, ab, e);
+    aff_apply<M>(B, ab, abn);
+    for (int i = 0; i < M; ++i) ab[i] = abn[i];
+    if (t == hi - 1) agg = e;
+    else { cong_combine<M>(e, agg, tmp); agg = tmp; }
+  }
+}
+
+// One unit's parameter cotangents, any may be null: a0 [M], P0 [M, M], and T, C, c, Z, H, d with one row per step where
+// that input is time-varying (its UnitView stride is not 0), one row where it is static.
+struct GradOut {
+  double *a0, *P0, *T, *C, *c, *Z, *H, *d;
+};
+
+// sums of the static inputs' cotangents, laid out T, C (M x M each), c, Z (M each), H, d
+template <int M>
+KFB_HD constexpr int static_grad_width() { return 2 * M * M + 2 * M + 2; }
+
+// The literal one-step adjoint of every step of a chunk, from hi-1 down to lo, starting from abar = ab_hi and
+// sym(Pbar) = X at hi (X is overwritten).  Time-varying inputs' cotangents are written per step; those of static inputs
+// are summed in that step order into acc[static_grad_width<M>()].  Step 0 also writes the a0 / P0 cotangents.
+template <int M>
+KFB_HD void adjoint_chunk(const UnitView& v, int lo, int hi, const double* tape, double gl, const double* gllo,
+                          const double* ab_hi, double* X, const GradOut& out, double* acc) {
+  TX<M> x{nullptr, nullptr, 0, 1};
+  BwdStep<M> B(x);
+  StepGrad<M> g;
+  CongElem<M> e;
+  double ab[M], abn[M];
+  for (int k = 0; k < static_grad_width<M>(); ++k) acc[k] = 0.0;
+  for (int i = 0; i < M; ++i) ab[i] = ab_hi[i];
+  for (int t = hi - 1; t >= lo; --t) {
+    bwd_load<M>(x, v, t, tape + (long long)t * tape_entry<M>(), gl, gllo, B);
+    if (t == 0) {
+      adjoint_step<M>(B, v.d_sign, ab, X, g, out.a0, out.P0);  // abar_0, Pbar_0 are the a0 / P0 cotangents
+    } else {
+      adjoint_step<M>(B, v.d_sign, ab, X, g, nullptr, nullptr);
+      cong_element<M>(B, ab, e);
+      cong_apply<M>(e, X);
+      aff_apply<M>(B, ab, abn);
+      for (int i = 0; i < M; ++i) ab[i] = abn[i];
+    }
+    if (v.T_ts) { if (out.T) for (int i = 0; i < M * M; ++i) out.T[(long long)t * M * M + i] = g.T[i]; }
+    else for (int i = 0; i < M * M; ++i) acc[i] += g.T[i];
+    if (v.C_ts) { if (out.C) for (int i = 0; i < M * M; ++i) out.C[(long long)t * M * M + i] = g.C[i]; }
+    else for (int i = 0; i < M * M; ++i) acc[M * M + i] += g.C[i];
+    if (v.c_ts) { if (out.c) for (int i = 0; i < M; ++i) out.c[(long long)t * M + i] = g.c[i]; }
+    else for (int i = 0; i < M; ++i) acc[2 * M * M + i] += g.c[i];
+    if (v.Z_ts) { if (out.Z) for (int i = 0; i < M; ++i) out.Z[(long long)t * M + i] = g.Z[i]; }
+    else for (int i = 0; i < M; ++i) acc[2 * M * M + M + i] += g.Z[i];
+    if (v.H_ts) { if (out.H) out.H[t] = g.H; }
+    else acc[2 * M * M + 2 * M] += g.H;
+    if (v.d_ts) { if (out.d) out.d[t] = g.d; }
+    else acc[2 * M * M + 2 * M + 1] += g.d;
+  }
+}
+
+// Entry k of the unit's static cotangent sums (adjoint_chunk's acc layout) to its output, if that input is static.
+template <int M>
+KFB_HD void store_static_grad(const UnitView& v, const GradOut& out, int k, double s) {
+  if (k < M * M) { if (out.T && !v.T_ts) out.T[k] = s; }
+  else if (k < 2 * M * M) { if (out.C && !v.C_ts) out.C[k - M * M] = s; }
+  else if (k < 2 * M * M + M) { if (out.c && !v.c_ts) out.c[k - 2 * M * M] = s; }
+  else if (k < 2 * M * M + 2 * M) { if (out.Z && !v.Z_ts) out.Z[k - 2 * M * M - M] = s; }
+  else if (k == 2 * M * M + 2 * M) { if (out.H && !v.H_ts) out.H[0] = s; }
+  else { if (out.d && !v.d_ts) out.d[0] = s; }
 }
 
 }  // namespace tpar

@@ -21,7 +21,8 @@
 //     A scan over products of gains has no accuracy guarantee, so on any drift the whole unit is re-run by the
 //     sequential recursion (smoother_unit's steps) - this smoother never returns what the sequential one would not.
 //
-// Everything here is KFB_HD so that tests/tpar_smooth_host compiles it for the host and checks it against the oracle.
+// Everything here is KFB_HD so that tests/tpar_host runs the same fold and walk on the host and checks them against the
+// oracle.
 #pragma once
 #include "kf_smooth.cuh"
 #include "kf_tpar.cuh"
@@ -185,18 +186,8 @@ KFB_HD bool smooth_walk_check(const SmoothView& v, int lo, int hi, const SmoothE
     for (int i = 0; i < M * M; ++i) L[i] = next->L[i];
   }
   smooth_run<M>(v, lo, hi, nullptr, g, L, true);
-  double sP = 0.0, sa = 0.0;
-#pragma unroll
-  for (int i = 0; i < M * M; ++i) sP = fmax(sP, fabs(L[i]));
-#pragma unroll
-  for (int i = 0; i < M; ++i) sa = fmax(sa, fabs(g[i]));
-  sa = fmax(sa, sqrt(sP));
-  bool ok = true;  // a NaN on either side fails its comparison
-#pragma unroll
-  for (int i = 0; i < M * M; ++i) ok = ok && (fabs(L[i] - own.L[i]) <= tol * sP);
-#pragma unroll
-  for (int i = 0; i < M; ++i) ok = ok && (fabs(g[i] - own.g[i]) <= tol * sa);
-  return lo > 0 && !ok;
+  const bool drift = drifted<M>(g, L, own.g, own.L, tol);  // outside the `lo > 0` branch: k_states 4 spills inside it
+  return lo > 0 && drift;
 }
 
 // The sequential recursion for one unit on one thread (the drift fallback): the walk of the whole series from the

@@ -1,7 +1,9 @@
-"""TEST-ONLY: the time-parallel filter and adjoint (csrc/kf_tpar.cuh) compiled for the host.
+"""TEST-ONLY: the time-parallel filter and adjoint (csrc/kf_tpar.cuh) and RTS smoother (csrc/kf_tpar_smooth.cuh)
+compiled for the host.
 
-``run`` emulates the CTA's blocked scans with ``nchunks`` chunks and a chosen scan tree (see tpar_host.cpp), so the
-combination operators can be checked against the oracle without a GPU.  Not part of the product.
+``run`` (filter and adjoint) and ``smooth_run`` (smoother) emulate the CTA's blocked scans with ``nchunks`` chunks and a
+chosen scan tree (see tpar_host.cpp), so the elements and their combination can be checked against the oracle without a
+GPU.  ``smooth_sequential`` runs the sequential smoother of kf_smooth.cuh the same way.  Not part of the product.
 """
 from __future__ import annotations
 
@@ -85,3 +87,34 @@ def run(kind, data, a0, P0, T, Z, R, H, Q, c=None, d=None, strict=True, nchunks=
         g["Pss"], g["Gss"] = None, None
         grads = hostsim.chain_to_inputs(kind, g, T, Z, R, H, Q, C, None, None)
     return outs, grads, int(info[0]), int(seq[0])
+
+
+def _smooth_prep(T, R, Q, fs, fc):
+    f8 = lambda x: np.ascontiguousarray(np.asarray(x, dtype=np.float64))  # noqa: E731
+    T, R, Q, fs, fc = map(f8, (T, R, Q, fs, fc))
+    C = f8(R @ Q @ R.T)
+    n, m = fc.shape[0], fc.shape[-1]
+    return T, C, f8(fs.reshape(n, m)), fc, n, m
+
+
+def smooth_run(T, R, Q, fs, fc, nchunks=8, tree=1, seed=1, tol=1e-10):
+    """Returns (smoothed_states [n,m,1], smoothed_covs [n,m,m], fallback): fallback = 1 if the walk disagreed with the
+    scan and the unit was re-run by the sequential recursion."""
+    lib = build()
+    T, C, fs, fc, n, m = _smooth_prep(T, R, Q, fs, fc)
+    ss, sc = np.zeros((n, m)), np.zeros((n, m, m))
+    fb = np.zeros(1, dtype=np.int32)
+    rc = lib.tpar_host_smooth_run(m, n, _p(T), _p(C), _p(fs), _p(fc), _p(ss), _p(sc), int(nchunks), int(tree),
+                                  ctypes.c_uint(seed), ctypes.c_double(tol), _p(fb))
+    if rc != 0:
+        raise RuntimeError(f"tpar_host_smooth_run rc={rc}")
+    return ss[..., None], sc, int(fb[0])
+
+
+def smooth_sequential(T, R, Q, fs, fc):
+    lib = build()
+    T, C, fs, fc, n, m = _smooth_prep(T, R, Q, fs, fc)
+    ss, sc = np.zeros((n, m)), np.zeros((n, m, m))
+    if lib.tpar_host_smooth_sequential(m, n, _p(T), _p(C), _p(fs), _p(fc), _p(ss), _p(sc)) != 0:
+        raise RuntimeError("tpar_host_smooth_sequential")
+    return ss[..., None], sc
