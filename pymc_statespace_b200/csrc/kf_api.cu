@@ -217,8 +217,9 @@ static void fill_args(const kfb_desc* d, const kfb_inputs* in, const Plan& pl, c
   A->ll_const = pl.ll_const;
   A->d_sign = pl.d_sign;
   if (d->p == 1 && !d->Z_ts && !d->H_ts)
-    A->struct_flags = ((d->flags & KFB_FLAG_Z_UNIT0) ? 1 : 0) | ((d->flags & KFB_FLAG_H_ZERO) ? 2 : 0) |
-                      ((d->flags & KFB_FLAG_T_COMPANION) ? 4 : 0);
+    A->struct_flags = ((d->flags & KFB_FLAG_Z_UNIT0) ? KF_STRUCT_Z_UNIT0 : 0) |
+                      ((d->flags & KFB_FLAG_H_ZERO) ? KF_STRUCT_H_ZERO : 0) |
+                      ((d->flags & KFB_FLAG_T_COMPANION) ? KF_STRUCT_T_COMPANION : 0);
 }
 
 static kfb_status cuda_fail(cudaError_t e) {
@@ -240,11 +241,11 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
     const bool p1_ok = !pl.tv_any && d->y_bs == 0 && d->n_series == 1 && !(d->flags & KFB_FLAG_GENERIC_ADJOINT) &&
                        p1_adjoint_supported(d->m, d->p, pl.mk);
     const bool full = A.ll_obs || A.fs || A.ps || A.fc || A.pc;
-    // all four structure promises on the k_endog = 1 kernels: compressed tape entries (kf_p1.cuh, ZU == 3) - decided from
-    // the descriptor alone, so that the forward pass and the adjoint always agree on the format
+    // all four structure promises on the k_endog = 1 kernels: compressed tape entries (kf_p1.cuh, ZU_REDUCED) - decided
+    // from the descriptor alone (make_plan), so that the forward pass and the adjoint always agree on the format
     KfArgs B = A;
-    if (pl.compressed && p1_ok && (A.struct_flags & 7) == 7) B.struct_flags |= 8;
-    if ((B.struct_flags & 8) && bwd && (A.gZ || A.gH)) return KFB_ERR_UNSUPPORTED;  // Z, H were promised constant
+    if (pl.compressed) B.struct_flags |= KF_STRUCT_COMPRESSED;
+    if (pl.compressed && bwd && (A.gZ || A.gH)) return KFB_ERR_UNSUPPORTED;  // Z, H were promised constant
     if (p1_ok && bwd)
       e = launch_p1_adjoint(B, ysm, bulk_ok, s);
     else if (p1_ok && !full)

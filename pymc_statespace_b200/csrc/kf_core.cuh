@@ -36,6 +36,15 @@ struct MatArg {
   long long ts;  // stride between time steps; 0 = static
 };
 
+// KfArgs::struct_flags bits.  The first three are caller promises (kfb200.h flags), set only for k_endog = 1 with static
+// Z and H; the k_endog = 1 kernels skip the products with the known zeros and ones and check the promises per unit.
+constexpr int KF_STRUCT_Z_UNIT0 = 1;      // Z = [1, 0, .., 0]           (KFB_FLAG_Z_UNIT0)
+constexpr int KF_STRUCT_H_ZERO = 2;       // H = 0                       (KFB_FLAG_H_ZERO)
+constexpr int KF_STRUCT_T_COMPANION = 4;  // T = [t | e_0 .. e_{m-2}]    (KFB_FLAG_T_COMPANION)
+// the tape entries are the reduced recursion's (a_t[0], leading block of P_t): set by the C-ABI layer when the three
+// promises above and KFB_FLAG_NO_MISSING hold, so that the forward pass and the adjoint agree on the format
+constexpr int KF_STRUCT_COMPRESSED = 8;
+
 struct KfArgs {
   long long U, n_series;
   int n, m, p, math_kind;
@@ -46,7 +55,7 @@ struct KfArgs {
   double *loglik, *ll_obs, *fs, *ps, *fc, *pc;
   int* info;
   const int* dare_info;  // steady state: per-draw status of the DARE solve (0 = ok) or null
-  int struct_flags;      // bit 0: Z = [1, 0, .., 0] (k_endog = 1); bit 1: H = 0   (caller's promises, kfb200.h flags)
+  int struct_flags;      // KF_STRUCT_* bits (above)
   double* tape;  // predicted (a_t, tri(P_t)) for t = 1..n-1
   // backward
   const double *g_loglik, *g_ll_obs;

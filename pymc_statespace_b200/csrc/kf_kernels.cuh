@@ -104,7 +104,7 @@ __device__ __forceinline__ void run_unit(X& x, const KfArgs& A, long long u) {
 template <int M, int P, int MK, bool TV, class X>
 __device__ __forceinline__ void run_unit_full(X& x, const KfArgs& A, long long u) {
   if constexpr (P == 1 && MK == MK_STD && !TV) {
-    if (A.struct_flags & 8) p1::forward_full_p1<M, true>(x, A, u);  // compressed tape entries (see kf_api.cu: launch_main)
+    if (A.struct_flags & KF_STRUCT_COMPRESSED) p1::forward_full_p1<M, true>(x, A, u);
     else p1::forward_full_p1<M, false>(x, A, u);
   } else {
     run_unit<MK, 1>(x, A, u);

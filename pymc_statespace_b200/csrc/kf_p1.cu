@@ -103,11 +103,11 @@ struct RingTape {
 constexpr int P1_WPC = KFB_P1_WPC;      // warps per CTA (the observation stream is staged once per CTA)
 constexpr int P1_SLOTS = KFB_P1_SLOTS;  // ring slots per warp (SLOTS - 1 entries in flight)
 
-template <int M, bool NEED_Z, bool NEED_H, bool HAS_GOBS, int ZU = 0, bool H0 = false>
+template <int M, bool NEED_Z, bool NEED_H, bool HAS_GOBS, int ZU, bool H0>
 __global__ void __launch_bounds__(32 * P1_WPC, (M <= 2) ? KFB_P1_MINB : 4)
     kf_p1_adjoint_kernel(const __grid_constant__ KfArgs A, int y_smem_doubles, int bulk_ok) {
   extern __shared__ __align__(128) double kf_dyn_smem[];
-  constexpr int KT = (ZU == 4) ? Dim<M>::KTA : Dim<M>::KT;
+  constexpr int KT = tape_doubles<M, ZU>;
   const double* yp = A.y.p;
   if (y_smem_doubles > 0) {
     stage_y(kf_dyn_smem, A.y.p, y_smem_doubles, bulk_ok != 0);
@@ -129,9 +129,9 @@ __global__ void __launch_bounds__(32 * P1_WPC, (M <= 2) ? KFB_P1_MINB : 4)
   backward_unit_p1<M, NEED_Z, NEED_H, HAS_GOBS, RingTape<M, P1_SLOTS, KT>, ZU, H0>(A, store ? u : A.U - 1, store, yp, tape);
 }
 
-template <int M, bool NEED_Z, bool NEED_H, bool HAS_GOBS, int ZU = 0, bool H0 = false>
+template <int M, bool NEED_Z, bool NEED_H, bool HAS_GOBS, int ZU, bool H0>
 static cudaError_t launch_one(const KfArgs& A, int ysm, int bulk_ok, cudaStream_t s) {
-  constexpr int KT = (ZU == 4) ? Dim<M>::KTA : Dim<M>::KT;
+  constexpr int KT = tape_doubles<M, ZU>;
   const int block = 32 * P1_WPC;
   const unsigned grid = (unsigned)((A.U + block - 1) / block);
   const size_t smem = (size_t)((ysm + 15) & ~15) * 8 + (size_t)P1_WPC * P1_SLOTS * (KT * 32 * 8 + 8);
@@ -147,115 +147,35 @@ static cudaError_t launch_one(const KfArgs& A, int ysm, int bulk_ok, cudaStream_
 
 template <int M>
 static cudaError_t launch_m(const KfArgs& A, int ysm, int bulk_ok, cudaStream_t s) {
-  const bool z = A.gZ != nullptr, h = A.gH != nullptr, g = A.g_ll_obs != nullptr;
-  if (!z && !h && (A.struct_flags & 15) == 15) {  // + no missing observation: reduced recursion, tape = (a_t[0], leading block of P_t)
-    return g ? launch_one<M, false, false, true, 4, true>(A, ysm, bulk_ok, s)
-             : launch_one<M, false, false, false, 4, true>(A, ysm, bulk_ok, s);
-  }
-  if (!z && !h && (A.struct_flags & 7) == 7) {  // + companion T (ARMA / SARIMAX): only column 0 of T-bar exists
-    return g ? launch_one<M, false, false, true, 2, true>(A, ysm, bulk_ok, s)
-             : launch_one<M, false, false, false, 2, true>(A, ysm, bulk_ok, s);
-  }
-  if (!z && !h && (A.struct_flags & 1)) {  // structured design row (and observation variance): fewer products per step
-    const bool h0 = (A.struct_flags & 2) != 0;
-    if (g) return h0 ? launch_one<M, false, false, true, true, true>(A, ysm, bulk_ok, s)
-                     : launch_one<M, false, false, true, true, false>(A, ysm, bulk_ok, s);
-    return h0 ? launch_one<M, false, false, false, true, true>(A, ysm, bulk_ok, s)
-              : launch_one<M, false, false, false, true, false>(A, ysm, bulk_ok, s);
-  }
-  if (g) {
-    if (z) return launch_one<M, true, true, true>(A, ysm, bulk_ok, s);
-    if (h) return launch_one<M, false, true, true>(A, ysm, bulk_ok, s);
-    return launch_one<M, false, false, true>(A, ysm, bulk_ok, s);
-  }
-  if (z) return launch_one<M, true, true, false>(A, ysm, bulk_ok, s);
-  if (h) return launch_one<M, false, true, false>(A, ysm, bulk_ok, s);
-  return launch_one<M, false, false, false>(A, ysm, bulk_ok, s);
+  return with_adjoint_variant(A, [&](auto v) {
+    using V = decltype(v);
+    return launch_one<M, V::NEED_Z, V::NEED_H, V::HAS_GOBS, V::ZU, V::H0>(A, ysm, bulk_ok, s);
+  });
 }
 
 // ---- forward (loglik + tape) -------------------------------------------------------------------------------
-// Tape entry of a warp and step -> shared memory -> ONE TMA bulk store (cp.async.bulk.global.shared::cta, SASS UBLKCP).
-// Measured at 65,536 draws: the forward pass computes in 0.34 ms but took 0.53 ms with per-lane STG.64 stores - the
-// per-SM store path, not HBM, was the limit at 14 resident warps per SM.  Two slots per warp; a slot is reused only after
-// the bulk store issued from it two steps earlier has finished READING it (cp.async.bulk.wait_group.read 1).
-#ifndef KFB_P1_BULK_STORE
-#define KFB_P1_BULK_STORE 0
-#endif
-template <int M>
-struct BulkSink {
-  static constexpr int KT = Dim<M>::KT;
-  static constexpr unsigned BYTES = KT * 32 * 8;
-  unsigned slot0_s;  // shared-window address of this warp's two staging slots
-  unsigned lane, par;
-  __device__ __forceinline__ void put(double* tq, const double (&a)[M], const double (&P)[Dim<M>::NS]) {
-    asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");  // (only lane 0 owns bulk groups)
-    __syncwarp();
-    const unsigned dst = slot0_s + par * BYTES + lane * 8u;
-#pragma unroll
-    for (int k = 0; k < M; ++k) asm volatile("st.shared.f64 [%0], %1;" ::"r"(dst + k * 256u), "d"(a[k]) : "memory");
-#pragma unroll
-    for (int k = 0; k < Dim<M>::NS; ++k)
-      asm volatile("st.shared.f64 [%0], %1;" ::"r"(dst + (M + k) * 256u), "d"(P[k]) : "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the async proxy
-    __syncwarp();
-    if (lane == 0) {
-      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(tq), "r"(slot0_s + par * BYTES),
-                   "r"(BYTES)
-                   : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    par ^= 1u;
-  }
-  __device__ __forceinline__ void finish() {
-    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-    __syncwarp();
-  }
-};
-
-template <int M, bool SAVE, int ZU = 0, bool H0 = false>
+template <int M, bool SAVE, int ZU, bool H0>
 __global__ void __launch_bounds__(64, (M <= 2) ? 8 : 4)
     kf_p1_forward_kernel(const __grid_constant__ KfArgs A, int y_smem_doubles, int bulk_ok) {
   extern __shared__ __align__(128) double kf_dyn_smem[];
-  constexpr int KT = (ZU == 4) ? Dim<M>::KTA : Dim<M>::KT;  // doubles per tape entry
+  constexpr int KT = tape_doubles<M, ZU>;
   const double* yp = A.y.p;
   if (y_smem_doubles > 0) {
     stage_y(kf_dyn_smem, A.y.p, y_smem_doubles, bulk_ok != 0);
     yp = kf_dyn_smem;
   }
   const long long u = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-#if defined(KFB_P1_DEBUG_TSTEP0)  // experiment only: every step overwrites the same (L2-resident) entry
-  const long long tstep = 0;
-#else
   const long long tstep = (long long)KT * tape_units_padded(A.U);
-#endif
-  if (SAVE && KFB_P1_BULK_STORE) {
-    // warp-collective stores: the padding lanes of the last warp run along on the last unit's inputs (their columns of
-    // the padded tape are never read)
-    const int lane = threadIdx.x & 31;
-    const long long u0 = u - lane;
-    if (u0 >= A.U) return;
-    BulkSink<M> sink;
-    sink.slot0_s = (unsigned)__cvta_generic_to_shared(kf_dyn_smem + ((y_smem_doubles + 15) & ~15)) +
-                   (unsigned)((threadIdx.x >> 5) * 2 * Dim<M>::KT * 32 * 8);
-    sink.lane = (unsigned)lane;
-    sink.par = 0;
-    double* tp = A.tape + (u >> 5) * (KT * 32) + lane;
-    const bool store = u < A.U;
-    forward_unit_p1<M, SAVE, ZU, H0, BulkSink<M>>(A, store ? u : A.U - 1, store, yp, tp - lane, tstep, sink);
-    return;
-  }
   if (u >= A.U) return;
   double* tp = SAVE ? A.tape + (u >> 5) * (KT * 32) + (u & 31) : nullptr;
   forward_unit_p1<M, SAVE, ZU, H0>(A, u, true, yp, tp, tstep);
 }
 
-template <int M, bool SAVE, int ZU = 0, bool H0 = false>
+template <int M, bool SAVE, int ZU, bool H0>
 static cudaError_t launch_fwd_one(const KfArgs& A, int ysm, int bulk_ok, cudaStream_t s) {
   const int block = 64;
   const unsigned grid = (unsigned)((A.U + block - 1) / block);
-  const size_t smem = (SAVE && KFB_P1_BULK_STORE)
-                          ? (size_t)((ysm + 15) & ~15) * 8 + (size_t)(block / 32) * 2 * Dim<M>::KT * 32 * 8
-                          : (size_t)((ysm + 1) & ~1) * 8;
+  const size_t smem = (size_t)((ysm + 1) & ~1) * 8;
   auto kern = kf_p1_forward_kernel<M, SAVE, ZU, H0>;
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -268,16 +188,11 @@ static cudaError_t launch_fwd_one(const KfArgs& A, int ysm, int bulk_ok, cudaStr
 
 template <int M>
 static cudaError_t launch_fwd_m(const KfArgs& A, int ysm, int bulk_ok, cudaStream_t s) {
-  if ((A.struct_flags & 15) == 15)
-    return A.tape ? launch_fwd_one<M, true, 4, true>(A, ysm, bulk_ok, s) : launch_fwd_one<M, false, 4, true>(A, ysm, bulk_ok, s);
-  if ((A.struct_flags & 7) == 7)
-    return A.tape ? launch_fwd_one<M, true, 2, true>(A, ysm, bulk_ok, s) : launch_fwd_one<M, false, 2, true>(A, ysm, bulk_ok, s);
-  if (A.struct_flags & 1) {
-    if (A.struct_flags & 2)
-      return A.tape ? launch_fwd_one<M, true, true, true>(A, ysm, bulk_ok, s) : launch_fwd_one<M, false, true, true>(A, ysm, bulk_ok, s);
-    return A.tape ? launch_fwd_one<M, true, true, false>(A, ysm, bulk_ok, s) : launch_fwd_one<M, false, true, false>(A, ysm, bulk_ok, s);
-  }
-  return A.tape ? launch_fwd_one<M, true>(A, ysm, bulk_ok, s) : launch_fwd_one<M, false>(A, ysm, bulk_ok, s);
+  return with_forward_variant(A, [&](auto v) {
+    using V = decltype(v);
+    return A.tape ? launch_fwd_one<M, true, V::ZU, V::H0>(A, ysm, bulk_ok, s)
+                  : launch_fwd_one<M, false, V::ZU, V::H0>(A, ysm, bulk_ok, s);
+  });
 }
 
 }  // namespace p1

@@ -3,7 +3,7 @@
 // m x m x m products on the FP64 TENSOR CORES (mma.sync.m8n8k4.f64, "DMMA"), everything else row-per-lane as in kf_rows.cuh.
 //
 // Why: with DFMA every multiply-add needs at least one operand from shared memory and a broadcast load delivers one
-// double per wavefront, so the warp-per-unit DFMA kernel of round 1 (tools/attic/kf_rowsL.cuh) sat at 94 % of the
+// double per wavefront, so the warp-per-unit DFMA kernel of round 1 sat at 94 % of the
 // shared-memory wavefront peak with the fp64 pipe 35 % active (profiles/r1_ncu_rowsL.md).  A DMMA consumes one A and one
 // B element per lane for eight multiply-adds per lane, and a fragment is reused for NT tiles: ~0.06 shared-memory operands
 // per multiply-add.  tools/dmma_probe.cu measured 37.1 TFLOP/s for register-operand DMMA on this B200 - the same as the

@@ -14,7 +14,7 @@
 
 using namespace kfb;
 
-static int g_p1 = 0;    // 1: adjoint through kf_p1.cuh (k_endog = 1, standard family) after the predictor-form forward
+static int g_p1 = 0;    // k_endog = 1: 1: forward + adjoint of kf_p1.cuh, 2: generic forward + kf_p1.cuh adjoint
 static int g_pred = 0;  // 1: run the one-step-predictor programs (kf_pred.cuh) where they exist
 
 template <int MK, class X>
@@ -29,55 +29,28 @@ static void run_both(X& x, KfArgs& A, int do_bwd) {
   }
 }
 
+// The k_endog = 1 kernels' instantiation choice (kf_p1.cuh: with_forward_variant / with_adjoint_variant), with the tape
+// in the kernels' layout for one unit and read back directly instead of through the TMA ring.
 template <int M>
-static void run_p1(ThreadCtx<M, 1>& x, KfArgs& A, int do_bwd) {
-  const bool zu = (A.struct_flags & 1) != 0, h0 = (A.struct_flags & 2) != 0;
-  if (g_p1 == 1 && (A.struct_flags & 7) == 7 && !A.gZ && !A.gH) {  // + companion T (+ complete data: compressed tape)
-    const bool ct = (A.struct_flags & 8) != 0;
-    constexpr int KTA_ = p1::Dim<M>::KTA;  // reduced recursion: (a_t[0], leading block of P_t)
-    if (ct) p1::forward_unit_p1<M, true, 4, true>(A, 0, true, A.y.p, A.tape, (long long)KTA_ * 32);
-    else p1::forward_unit_p1<M, true, 2, true>(A, 0, true, A.y.p, x.tape_base(A, 0), x.tape_step(A));
-    if (!do_bwd) return;
-    if (ct) {
-      p1::DirectTape<M, KTA_> tc{A.tape + (long long)(A.n - 2) * KTA_ * 32, (long long)KTA_ * 32, 32};
-      if (A.g_ll_obs) p1::backward_unit_p1<M, false, false, true, p1::DirectTape<M, KTA_>, 4, true>(A, 0, true, A.y.p, tc);
-      else p1::backward_unit_p1<M, false, false, false, p1::DirectTape<M, KTA_>, 4, true>(A, 0, true, A.y.p, tc);
-    } else {
-      p1::DirectTape<M> tc{x.tape_base(A, 0) + (long long)(A.n - 2) * x.tape_step(A), x.tape_step(A), x.tape_elem(A)};
-      if (A.g_ll_obs) p1::backward_unit_p1<M, false, false, true, p1::DirectTape<M>, 2, true>(A, 0, true, A.y.p, tc);
-      else p1::backward_unit_p1<M, false, false, false, p1::DirectTape<M>, 2, true>(A, 0, true, A.y.p, tc);
-    }
-    return;
-  }
-  if (g_p1 == 2) forward_unit_pred<MK_STD>(x, A, 0);  // generic forward + specialised adjoint
-  else if (zu && h0) p1::forward_unit_p1<M, true, true, true>(A, 0, true, A.y.p, x.tape_base(A, 0), x.tape_step(A));
-  else if (zu) p1::forward_unit_p1<M, true, true, false>(A, 0, true, A.y.p, x.tape_base(A, 0), x.tape_step(A));
-  else p1::forward_unit_p1<M, true>(A, 0, true, A.y.p, x.tape_base(A, 0), x.tape_step(A));
-  if (!do_bwd) return;
-  if (zu && !A.gZ && !A.gH) {
-    p1::DirectTape<M> tp2{x.tape_base(A, 0) + (long long)(A.n - 2) * x.tape_step(A), x.tape_step(A), x.tape_elem(A)};
-    if (A.g_ll_obs) {
-      if (h0) p1::backward_unit_p1<M, false, false, true, p1::DirectTape<M>, true, true>(A, 0, true, A.y.p, tp2);
-      else p1::backward_unit_p1<M, false, false, true, p1::DirectTape<M>, true, false>(A, 0, true, A.y.p, tp2);
-    } else {
-      if (h0) p1::backward_unit_p1<M, false, false, false, p1::DirectTape<M>, true, true>(A, 0, true, A.y.p, tp2);
-      else p1::backward_unit_p1<M, false, false, false, p1::DirectTape<M>, true, false>(A, 0, true, A.y.p, tp2);
-    }
-    return;
-  }
-  p1::DirectTape<M> tape{x.tape_base(A, 0) + (long long)(A.n - 2) * x.tape_step(A), x.tape_step(A), x.tape_elem(A)};
-  const bool z = A.gZ != nullptr, hh = A.gH != nullptr;
-#define KFB_P1RUN(ZZ, HH, GG) p1::backward_unit_p1<M, ZZ, HH, GG>(A, 0, true, A.y.p, tape)
-  if (A.g_ll_obs) {
-    if (z) KFB_P1RUN(true, true, true);
-    else if (hh) KFB_P1RUN(false, true, true);
-    else KFB_P1RUN(false, false, true);
+static void run_p1(KfArgs& A, int do_bwd) {
+  if (g_p1 == 2) {  // generic forward (full tape entries) + specialised adjoint
+    ThreadCtx<M, 1> x{nullptr, nullptr, 0, 1};
+    forward_unit_pred<MK_STD>(x, A, 0);
+    A.struct_flags &= ~KF_STRUCT_COMPRESSED;
   } else {
-    if (z) KFB_P1RUN(true, true, false);
-    else if (hh) KFB_P1RUN(false, true, false);
-    else KFB_P1RUN(false, false, false);
+    p1::with_forward_variant(A, [&](auto v) {
+      using V = decltype(v);
+      p1::forward_unit_p1<M, true, V::ZU, V::H0>(A, 0, true, A.y.p, A.tape, (long long)p1::tape_doubles<M, V::ZU> * 32);
+    });
   }
-#undef KFB_P1RUN
+  if (!do_bwd) return;
+  p1::with_adjoint_variant(A, [&](auto v) {
+    using V = decltype(v);
+    constexpr int KT = p1::tape_doubles<M, V::ZU>;
+    using Tape = p1::DirectTape<M, KT>;
+    Tape tape{A.tape + (long long)(A.n - 2) * KT * 32, (long long)KT * 32, 32};
+    p1::backward_unit_p1<M, V::NEED_Z, V::NEED_H, V::HAS_GOBS, Tape, V::ZU, V::H0>(A, 0, true, A.y.p, tape);
+  });
 }
 
 template <class X>
@@ -111,16 +84,16 @@ extern "C" int hostsim_run(int mk, int m, int p, int n, const double* y, const d
   A.gPss = gPss; A.gGss = gGss;
 
   g_pred = (static_dims >> 1) & 1;
-  A.struct_flags = (static_dims >> 4) & 15;  // bit 4: Z = [1, 0, ..], bit 5: H = 0, bit 6: companion T, bit 7: no missing y
+  A.struct_flags = (static_dims >> 4) & 15;  // bits 4..7: KF_STRUCT_Z_UNIT0, _H_ZERO, _T_COMPANION, _COMPRESSED
   g_p1 = (static_dims >> 2) & 3;  // 1: specialised forward + adjoint, 2: generic forward + specialised adjoint
   static_dims &= 1;
   if (g_p1) {
     if (p != 1 || mk != MK_STD || ts[0] || ts[1] || ts[2] || ts[3] || ts[4] || ts[5]) return 7;
-#define KFB_P1CASE(MM)                \
-  if (m == MM) {                      \
-    ThreadCtx<MM, 1> x{nullptr, nullptr, 0, 1}; \
-    run_p1<MM>(x, A, do_bwd);         \
-    return 0;                         \
+    if ((A.struct_flags & p1::REDUCED_FLAGS) == p1::REDUCED_FLAGS && (gZ || gH)) return 7;  // the C ABI refuses it too
+#define KFB_P1CASE(MM)   \
+  if (m == MM) {         \
+    run_p1<MM>(A, do_bwd); \
+    return 0;            \
   }
     KFB_P1CASE(1) KFB_P1CASE(2) KFB_P1CASE(3) KFB_P1CASE(4)
 #undef KFB_P1CASE

@@ -299,7 +299,7 @@ def test_subwarp_kernels_many_units_not_multiple_of_group():
                          ids=lambda d: "m%dp%dr%d" % d)
 def test_fused_row_kernels_hot_path(dims, wrt):
     """The theta-level hot path of mid-size / large systems: loglik-only forward + adjoint WITHOUT Z-bar go through the
-    fused row kernels (kf_rows.cuh: 4 lanes x 2 rows, k_states 5..8; kf_rowsL.cuh: warp per unit, k_states 30), with and
+    fused row kernels (kf_rows.cuh: 4 lanes x 2 rows, k_states 5..8; kf_rowsD.cuh: warp per unit, k_states 10..32), with and
     without T-bar (separate instantiations / code paths).  13 units: partial last warp; shared y with missing rows."""
     from pymc_statespace_b200 import BatchedKalman
 

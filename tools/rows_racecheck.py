@@ -13,7 +13,7 @@ lp, g = m.logp_and_grad(th)
 torch.cuda.synchronize()
 print("logp sum", float(lp.sum()), "grad abs sum", float(g.abs().sum()))
 
-# large systems (kf_rowsL.cuh): trend + seasonal, k_states = 30 (no T-bar), and a random k_states = 30 system with T-bar
+# large systems (kf_rowsD.cuh): trend + seasonal, k_states = 30 (no T-bar), and a random k_states = 30 system with T-bar
 from pymc_statespace_b200.synthetic import trend_seasonal_workload
 spec, y, theta = trend_seasonal_workload(n_draws=6, n=12)
 m = KalmanLogp(spec, y, n_draws=6, filter_type="standard")
