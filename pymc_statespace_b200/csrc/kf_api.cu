@@ -125,7 +125,7 @@ struct Plan {
   int mk;
   double ll_const, d_sign;
   bool tv_any, use_thread;
-  bool compressed;   // k_endog = 1 kernels with all four structure promises: tape entries hold a_t and the leading block of P_t
+  bool compressed;   // k_endog = 1 kernels with all four structure promises: the compressed tape (CTape, kf_core.cuh)
   bool tpar;         // KFB_FLAG_TIME_PARALLEL: one CTA per unit, scans over time (kf_tpar.cu); tape [u][t][a_t, P_t]
   long long U, nD;
   int nTC;           // time entries of C = R Q R^T (1 or n)
@@ -185,8 +185,9 @@ static kfb_status make_plan(const kfb_desc* d, bool save, Plan* pl) {
     pl->off_tape = take((size_t)pl->U * d->n * (d->m + d->m * d->m));
     if (save) pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
   } else if (save) {
-    const size_t entry = pl->compressed ? (size_t)(1 + ((d->m - 1) * d->m) / 2) : (size_t)tape_width(d->m);
-    pl->off_tape = take((size_t)tape_units_padded(pl->U) * (d->n > 1 ? d->n - 1 : 0) * entry);
+    const size_t entries = pl->compressed ? (size_t)ctape_steps_padded(d->n) * ctape_entry_doubles(d->m)
+                                          : (size_t)(d->n > 1 ? d->n - 1 : 0) * tape_width(d->m);
+    pl->off_tape = take((size_t)tape_units_padded(pl->U) * entries);
     pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
     if (pl->mk == MK_STEADY) {
       pl->off_gPss = take((size_t)pl->U * d->m * d->m);

@@ -41,8 +41,8 @@ struct MatArg {
 constexpr int KF_STRUCT_Z_UNIT0 = 1;      // Z = [1, 0, .., 0]           (KFB_FLAG_Z_UNIT0)
 constexpr int KF_STRUCT_H_ZERO = 2;       // H = 0                       (KFB_FLAG_H_ZERO)
 constexpr int KF_STRUCT_T_COMPANION = 4;  // T = [t | e_0 .. e_{m-2}]    (KFB_FLAG_T_COMPANION)
-// the tape entries are the reduced recursion's (a_t[0], leading block of P_t): set by the C-ABI layer when the three
-// promises above and KFB_FLAG_NO_MISSING hold, so that the forward pass and the adjoint agree on the format
+// the tape is the reduced recursion's compressed tape (CTape below): set by the C-ABI layer when the three promises above
+// and KFB_FLAG_NO_MISSING hold, so that the forward pass and the adjoint agree on the format
 constexpr int KF_STRUCT_COMPRESSED = 8;
 
 struct KfArgs {
@@ -56,7 +56,7 @@ struct KfArgs {
   int* info;
   const int* dare_info;  // steady state: per-draw status of the DARE solve (0 = ok) or null
   int struct_flags;      // KF_STRUCT_* bits (above)
-  double* tape;  // predicted (a_t, tri(P_t)) for t = 1..n-1
+  double* tape;  // predicted (a_t, tri(P_t)) for t = 1..n-1 (KF_STRUCT_COMPRESSED: the CTape entries below)
   // backward
   const double *g_loglik, *g_ll_obs;
   double *ga0, *gP0, *gT, *gZ, *gH, *gC, *gc, *gd, *gPss, *gGss;
@@ -65,6 +65,42 @@ struct KfArgs {
 KFB_HD int tape_width(int m) { return m + (m * (m + 1)) / 2; }
 // the tape holds whole warps of units (thread-per-unit layout [t-1][warp][k][32])
 KFB_HD long long tape_units_padded(long long U) { return (U + 31) & ~31LL; }
+
+// Compressed tape of the k_endog = 1 kernels (KF_STRUCT_COMPRESSED; kf_p1.cuh, ZU_REDUCED).  The entry of step t holds
+// what the reduced adjoint reads: (v_t, 1 / F_t, P_t[0][1 .. m-2]), KT = m doubles (1 at m = 1: v_t alone, F is a
+// constant of the draw there).  S = KF_CTAPE_STEPS consecutive steps of one warp are one contiguous block, so the
+// adjoint fetches S steps with one bulk copy:  [t / S][warp][t % S][row of the step].  In a row, each lane's doubles go
+// in pairs (element k < KT & ~1 at (k / 2) * 64 + 2 lane + k % 2: one 16-byte store / LDS.128 per pair) and an odd last
+// element at (KT & ~1) * 32 + lane.  Step 0 is never taped: its slot in block 0 is not read.  The forward kernels, the
+// adjoint's ring and the host build all locate entries through this struct; kfb_workspace_bytes sizes the tape with
+// ctape_steps_padded.
+#ifndef KFB_P1_TAPE_STEPS
+#define KFB_P1_TAPE_STEPS 4
+#endif
+constexpr int KF_CTAPE_STEPS = KFB_P1_TAPE_STEPS;
+static_assert((KF_CTAPE_STEPS & (KF_CTAPE_STEPS - 1)) == 0 && KF_CTAPE_STEPS <= 16, "a power of two <= 16");
+KFB_HD constexpr int ctape_entry_doubles(int m) { return m >= 2 ? m : 1; }
+// time entries per unit: steps 0 .. n-1 rounded up to whole blocks (none when nothing is taped)
+KFB_HD long long ctape_steps_padded(int n) {
+  return n > 1 ? (long long)((n + KF_CTAPE_STEPS - 1) / KF_CTAPE_STEPS) * KF_CTAPE_STEPS : 0;
+}
+template <int KT>
+struct CTape {
+  static constexpr int S = KF_CTAPE_STEPS;
+  static constexpr int ROW = KT * 32;   // doubles of one step of one warp
+  static constexpr int BLOCK = S * ROW;  // doubles of one block of one warp
+  // doubles between the blocks t / S and t / S + 1 of a warp
+  KFB_HD static long long block_stride(long long U) { return (long long)BLOCK * (tape_units_padded(U) >> 5); }
+  // doubles from the start of the tape to the row of unit u's warp at step t
+  KFB_HD static long long row(long long U, long long u, int t) {
+    const unsigned tu = (unsigned)t;
+    return (long long)(tu / S) * block_stride(U) + (u >> 5) * BLOCK + (long long)((tu % S) * ROW);
+  }
+  // element k of a lane within a row
+  KFB_HD static constexpr int lane_offset(int lane, int k) {
+    return k < (KT & ~1) ? (k >> 1) * 64 + 2 * lane + (k & 1) : (KT & ~1) * 32 + lane;
+  }
+};
 
 KFB_HD double kf_fma(double a, double b, double c) {
 #if defined(__CUDA_ARCH__)
