@@ -12,11 +12,6 @@ static std::atomic<long long> g_launches{0};
 static thread_local const char* g_cuda_err = "";
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
-thread_launch_fn thread_launcher_m1(int p, int mk, bool tv);
-thread_launch_fn thread_launcher_m2(int p, int mk, bool tv);
-thread_launch_fn thread_launcher_m3(int p, int mk, bool tv);
-thread_launch_fn thread_launcher_m4(int p, int mk, bool tv);
-
 bool p1_adjoint_supported(int m, int p, int mk);
 cudaError_t launch_p1_adjoint(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 cudaError_t launch_p1_forward(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
@@ -26,97 +21,55 @@ cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
 bool tpar_smoother_supported(int m);
 cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
 
-coopT_launch_fn coopT_launcher_m5(int p, int mk);
-coopT_launch_fn coopT_launcher_m6(int p, int mk);
-coopT_launch_fn coopT_launcher_m7(int p, int mk);
-coopT_launch_fn coopT_launcher_m8(int p, int mk);
-coopT_launch_fn coopT_launcher_m10(int p, int mk);
-coopT_launch_fn coopT_launcher_m12(int p, int mk);
-coopT_launch_fn coopT_launcher_m14(int p, int mk);
-coopT_launch_fn coopT_launcher_m16(int p, int mk);
-coopT_launch_fn coopT_launcher_m18(int p, int mk);
-coopT_launch_fn coopT_launcher_m20(int p, int mk);
-coopT_launch_fn coopT_launcher_m22(int p, int mk);
-coopT_launch_fn coopT_launcher_m24(int p, int mk);
-coopT_launch_fn coopT_launcher_m26(int p, int mk);
-coopT_launch_fn coopT_launcher_m28(int p, int mk);
-coopT_launch_fn coopT_launcher_m30(int p, int mk);
-coopT_launch_fn coopT_launcher_m32(int p, int mk);
+// k_states with launchers of their own, one object per size (kf_thread.cu: thread-per-unit filters and smoother;
+// kf_coopT.cu: compile-time-dims kernels; the tensor-core DARE in kf_coopT.cu from k_states 10).  The Makefile repeats
+// the first two lists (THREAD_MS, COOPT_MS): a size missing there leaves an undefined symbol in libkfb200.so.
+#define KFB_THREAD_SIZES(X) X(1) X(2) X(3) X(4)
+#define KFB_COOPT_SIZES(X) X(5) X(6) X(7) X(8) X(10) X(12) X(14) X(16) X(18) X(20) X(22) X(24) X(26) X(28) X(30) X(32)
+#define KFB_DARED_SIZES(X) X(10) X(12) X(14) X(16) X(18) X(20) X(22) X(24) X(26) X(28) X(30) X(32)
 
-dare_launch_fn dareD_launcher_m10(int p);
-dare_launch_fn dareD_launcher_m12(int p);
-dare_launch_fn dareD_launcher_m14(int p);
-dare_launch_fn dareD_launcher_m16(int p);
-dare_launch_fn dareD_launcher_m18(int p);
-dare_launch_fn dareD_launcher_m20(int p);
-dare_launch_fn dareD_launcher_m22(int p);
-dare_launch_fn dareD_launcher_m24(int p);
-dare_launch_fn dareD_launcher_m26(int p);
-dare_launch_fn dareD_launcher_m28(int p);
-dare_launch_fn dareD_launcher_m30(int p);
-dare_launch_fn dareD_launcher_m32(int p);
+#define KFB_DECL(M) thread_launch_fn thread_launcher_m##M(int p, int mk, bool tv); smoother_launch_fn smoother_thread_m##M();
+KFB_THREAD_SIZES(KFB_DECL)
+#undef KFB_DECL
+#define KFB_DECL(M) coopT_launch_fn coopT_launcher_m##M(int p, int mk);
+KFB_COOPT_SIZES(KFB_DECL)
+#undef KFB_DECL
+#define KFB_DECL(M) dare_launch_fn dareD_launcher_m##M(int p);
+KFB_DARED_SIZES(KFB_DECL)
+#undef KFB_DECL
 
-dare_launch_fn find_dareD_launcher(int m, int p) {
+thread_launch_fn find_thread_launcher(int m, int p, int mk, bool tv) {
   switch (m) {
-    case 10: return dareD_launcher_m10(p);
-    case 12: return dareD_launcher_m12(p);
-    case 14: return dareD_launcher_m14(p);
-    case 16: return dareD_launcher_m16(p);
-    case 18: return dareD_launcher_m18(p);
-    case 20: return dareD_launcher_m20(p);
-    case 22: return dareD_launcher_m22(p);
-    case 24: return dareD_launcher_m24(p);
-    case 26: return dareD_launcher_m26(p);
-    case 28: return dareD_launcher_m28(p);
-    case 30: return dareD_launcher_m30(p);
-    case 32: return dareD_launcher_m32(p);
+#define KFB_CASE(M) case M: return thread_launcher_m##M(p, mk, tv);
+    KFB_THREAD_SIZES(KFB_CASE)
+#undef KFB_CASE
+    default: return nullptr;
+  }
+}
+
+smoother_launch_fn find_smoother_thread_launcher(int m) {
+  switch (m) {
+#define KFB_CASE(M) case M: return smoother_thread_m##M();
+    KFB_THREAD_SIZES(KFB_CASE)
+#undef KFB_CASE
     default: return nullptr;
   }
 }
 
 coopT_launch_fn find_coopT_launcher(int m, int p, int mk) {
   switch (m) {
-    case 5: return coopT_launcher_m5(p, mk);
-    case 6: return coopT_launcher_m6(p, mk);
-    case 7: return coopT_launcher_m7(p, mk);
-    case 8: return coopT_launcher_m8(p, mk);
-    case 10: return coopT_launcher_m10(p, mk);
-    case 12: return coopT_launcher_m12(p, mk);
-    case 14: return coopT_launcher_m14(p, mk);
-    case 16: return coopT_launcher_m16(p, mk);
-    case 18: return coopT_launcher_m18(p, mk);
-    case 20: return coopT_launcher_m20(p, mk);
-    case 22: return coopT_launcher_m22(p, mk);
-    case 24: return coopT_launcher_m24(p, mk);
-    case 26: return coopT_launcher_m26(p, mk);
-    case 28: return coopT_launcher_m28(p, mk);
-    case 30: return coopT_launcher_m30(p, mk);
-    case 32: return coopT_launcher_m32(p, mk);
+#define KFB_CASE(M) case M: return coopT_launcher_m##M(p, mk);
+    KFB_COOPT_SIZES(KFB_CASE)
+#undef KFB_CASE
     default: return nullptr;
   }
 }
 
-smoother_launch_fn smoother_thread_m1();
-smoother_launch_fn smoother_thread_m2();
-smoother_launch_fn smoother_thread_m3();
-smoother_launch_fn smoother_thread_m4();
-
-smoother_launch_fn find_smoother_thread_launcher(int m) {
+dare_launch_fn find_dareD_launcher(int m, int p) {
   switch (m) {
-    case 1: return smoother_thread_m1();
-    case 2: return smoother_thread_m2();
-    case 3: return smoother_thread_m3();
-    case 4: return smoother_thread_m4();
-    default: return nullptr;
-  }
-}
-
-thread_launch_fn find_thread_launcher(int m, int p, int mk, bool tv) {
-  switch (m) {
-    case 1: return thread_launcher_m1(p, mk, tv);
-    case 2: return thread_launcher_m2(p, mk, tv);
-    case 3: return thread_launcher_m3(p, mk, tv);
-    case 4: return thread_launcher_m4(p, mk, tv);
+#define KFB_CASE(M) case M: return dareD_launcher_m##M(p);
+    KFB_DARED_SIZES(KFB_CASE)
+#undef KFB_CASE
     default: return nullptr;
   }
 }
@@ -241,7 +194,6 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
     // k_endog = 1, shared observations: the specialised adjoint with the TMA tape ring (kf_p1.cu)
     const bool p1_ok = !pl.tv_any && d->y_bs == 0 && d->n_series == 1 && !(d->flags & KFB_FLAG_GENERIC_ADJOINT) &&
                        p1_adjoint_supported(d->m, d->p, pl.mk);
-    const bool full = A.ll_obs || A.fs || A.ps || A.fc || A.pc;
     // all four structure promises on the k_endog = 1 kernels: compressed tape entries (kf_p1.cuh, ZU_REDUCED) - decided
     // from the descriptor alone (make_plan), so that the forward pass and the adjoint always agree on the format
     KfArgs B = A;
@@ -249,7 +201,7 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
     if (pl.compressed && bwd && (A.gZ || A.gH)) return KFB_ERR_UNSUPPORTED;  // Z, H were promised constant
     if (p1_ok && bwd)
       e = launch_p1_adjoint(B, ysm, bulk_ok, s);
-    else if (p1_ok && !full)
+    else if (p1_ok && !wants_step_outputs(A))
       e = launch_p1_forward(B, ysm, bulk_ok, s);
     else
       e = find_thread_launcher(d->m, d->p, pl.mk, pl.tv_any)(B, bwd, ysm, bulk_ok, s);

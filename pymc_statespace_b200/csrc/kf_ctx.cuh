@@ -23,7 +23,6 @@ struct RegBuf {
 template <int M, int P, bool TV_ = false>
 struct ThreadCtx {
   static constexpr bool TV = TV_;
-  static constexpr bool PIPELINE = false;  // adjoint: overlap gain(t-1) with adjoint(t)
   static constexpr bool SKIP_LB = false;   // adjoint without T-bar / Z-bar: keep the single code path (a run-time branch cost the m = 2 kernel 14 %)
   template <int SZ>
   using Buf = RegBuf<(SZ == SZ_M ? M : SZ == SZ_P ? P : SZ == SZ_MM ? M * M : SZ == SZ_MP ? M * P : SZ == SZ_PP ? P * P : M + (M * (M + 1)) / 2)>;
@@ -200,6 +199,48 @@ struct ThreadCtx {
   KFB_HD long long tape_elem(const KfArgs&) const { return 32; }
 };
 
+// Compile-time parameters of one thread-per-unit instantiation, handed to the caller's launcher as a tag.
+template <int M_, int P_, int MK_, bool TV_>
+struct ThreadInst {
+  static constexpr int M = M_, P = P_, MK = MK_;
+  static constexpr bool TV = TV_;
+};
+
+template <int M, int P, class Run>
+bool with_thread_kind(int mk, bool tv, Run& run) {
+  if (tv) {  // univariate / steady state: static matrices only
+    if (mk != MK_STD) return false;
+    run(ThreadInst<M, P, MK_STD, true>{});
+    return true;
+  }
+  switch (mk) {
+    case MK_STD: run(ThreadInst<M, P, MK_STD, false>{}); return true;
+    case MK_UNIV: run(ThreadInst<M, P, MK_UNIV, false>{}); return true;
+    case MK_STEADY: run(ThreadInst<M, P, MK_STEADY, false>{}); return true;
+    default: return false;  // MK_CHOLS: cooperative kernels only
+  }
+}
+
+template <int M, int P = 1, class Run>
+bool with_thread_p(int p, int mk, bool tv, Run& run) {
+  if constexpr (P > M || P > 3) return false;
+  else return p == P ? with_thread_kind<M, P>(mk, tv, run) : with_thread_p<M, P + 1>(p, mk, tv, run);
+}
+
+// Which thread-per-unit kernels exist, for the device launchers (kf_thread.cu) and the host build of the kernels alike:
+// k_states 1..4, k_endog 1..min(k_states, 3).  Calls run(ThreadInst<M, P, MK, TV>{}) and returns true, or returns false
+// when (m, p, mk, tv) has no instantiation.
+template <class Run>
+bool with_thread_instance(int m, int p, int mk, bool tv, Run&& run) {
+  switch (m) {
+    case 1: return with_thread_p<1>(p, mk, tv, run);
+    case 2: return with_thread_p<2>(p, mk, tv, run);
+    case 3: return with_thread_p<3>(p, mk, tv, run);
+    case 4: return with_thread_p<4>(p, mk, tv, run);
+    default: return false;
+  }
+}
+
 // ---------------------------------------------------------------------------
 // CoopCtx: G lanes cooperate on one unit; run-time dims; buffers are bump-allocated from a per-unit
 // shared-memory arena.  G == 32: one warp per unit (sync = __syncwarp); G == blockDim.x: one CTA per
@@ -207,7 +248,6 @@ struct ThreadCtx {
 // ---------------------------------------------------------------------------
 struct CoopCtx {
   static constexpr bool TV = true;
-  static constexpr bool PIPELINE = false;
   static constexpr bool SKIP_LB = true;    // adjoint without T-bar / Z-bar: skip the dense Lb product (kf_pred.cuh)
   int m_, p_, lane_, G_;
   double* arena;
@@ -218,6 +258,16 @@ struct CoopCtx {
   KFB_HD void set_dims(int m, int p) {
     m_ = m;
     p_ = p;
+  }
+  // G lanes (this one is `lane`) on an empty arena of `cap` doubles; `red` is the caller's
+  KFB_HD void init(int m, int p, double* arena_, int cap_, int lane, int G) {
+    set_dims(m, p);
+    arena = arena_;
+    off = 0;
+    cap = cap_;
+    overflow = false;
+    lane_ = lane;
+    G_ = G;
   }
   // NOTE: a multiply-high ("magic number") division was tried here; nvcc 12.9 then mis-compiled the unrolled
   // P - K K^T F loop of univariate_inner for k_states = 30 (compute-sanitizer racecheck: cross-thread RAW hazard,
@@ -353,7 +403,6 @@ KFB_HD void gemm(CoopCtx& x, TC& C, const TAa& A, const TBb& B, int r, int kk, i
 template <int M, int P, int G_>
 struct CoopCtxT {
   static constexpr bool TV = false;
-  static constexpr bool PIPELINE = false;
   static constexpr bool SKIP_LB = true;    // adjoint without T-bar / Z-bar: skip the dense Lb product (kf_pred.cuh)
   static constexpr int KT = M + (M * (M + 1)) / 2;
   int lane_;

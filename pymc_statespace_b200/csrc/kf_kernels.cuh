@@ -4,8 +4,7 @@
 
 #include "kf_ctx.cuh"
 #include "kf_dare.cuh"
-#include "kf_pred.cuh"
-#include "kf_p1.cuh"
+#include "kf_run.cuh"
 #include "kf_rows.cuh"
 #include "kf_rowsD.cuh"
 #include "kf_rowsU.cuh"
@@ -84,33 +83,6 @@ __device__ __forceinline__ void cta_sum(double* red, int w) {
   }
 }
 
-// MODE: 0 = forward, loglik (+tape) only; 1 = forward with per-step outputs; 2 = adjoint.
-// The hot path (MODE 0 / 2 of the standard-family and steady-state filters) runs in one-step-predictor form.
-template <int MK, int MODE, class X>
-__device__ __forceinline__ void run_unit(X& x, const KfArgs& A, long long u) {
-  constexpr bool PRED = (MK == MK_STD || MK == MK_STEADY);
-  if (MODE == 2) {
-    if (PRED) backward_unit_pred<MK>(x, A, u);
-    else backward_unit<MK>(x, A, u);
-  } else if (MODE == 0 && PRED) {
-    forward_unit_pred<MK>(x, A, u);
-  } else {
-    forward_unit<MK, MODE == 1>(x, A, u);
-  }
-}
-
-// full-output forward of the thread-per-unit kernels: one observed series + standard-family filter + static matrices run
-// the step written for that case (kf_p1.cuh: forward_full_p1), everything else the generic two-stage program
-template <int M, int P, int MK, bool TV, class X>
-__device__ __forceinline__ void run_unit_full(X& x, const KfArgs& A, long long u) {
-  if constexpr (P == 1 && MK == MK_STD && !TV) {
-    if (A.struct_flags & KF_STRUCT_COMPRESSED) p1::forward_full_p1<M, true>(x, A, u);
-    else p1::forward_full_p1<M, false>(x, A, u);
-  } else {
-    run_unit<MK, 1>(x, A, u);
-  }
-}
-
 // 65,536 units (the headline batch) need 443 resident threads per SM for a single wave: the pipelined adjoint of the
 // k_states <= 2 kernels is capped at 7 CTAs x 64 threads per SM (<= 144 registers) instead of spilling into a 2nd wave.
 template <int M, int P, int MK, int MODE, bool TV = false>
@@ -146,29 +118,22 @@ __global__ void __launch_bounds__(KFB_THREAD_BLOCK)
   run_unit<MK, MODE>(x, A, u);
 }
 
+// Run-time-dims kernels (CoopCtx): one warp (WARP, warp w on arena w of the CTA's shared memory) or the whole CTA per
+// unit.  This thread's unit; in warp mode the caller returns when it is >= the unit count.
+template <bool WARP>
+__device__ __forceinline__ long long coop_unit() {
+  return WARP ? (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5) : (long long)blockIdx.x;
+}
+
 template <int MK, int MODE, bool WARP>
 __global__ void __launch_bounds__(WARP ? 128 : 256, WARP ? 4 : 2) kf_coop_kernel(const __grid_constant__ KfArgs A, int arena_doubles) {
   extern __shared__ __align__(16) double kf_dyn_smem[];
   CoopCtx x;
-  x.set_dims(A.m, A.p);
-  x.off = 0;
-  x.cap = arena_doubles;
-  x.overflow = false;
+  x.init(A.m, A.p, WARP ? kf_dyn_smem + (size_t)(threadIdx.x >> 5) * arena_doubles : kf_dyn_smem, arena_doubles,
+         WARP ? threadIdx.x & 31 : threadIdx.x, WARP ? 32 : blockDim.x);
+  const long long u = coop_unit<WARP>();
+  if (WARP && u >= A.U) return;
   x.red = nullptr;
-  long long u;
-  if (WARP) {
-    const int warp = threadIdx.x >> 5;
-    x.lane_ = threadIdx.x & 31;
-    x.G_ = 32;
-    x.arena = kf_dyn_smem + (size_t)warp * arena_doubles;
-    u = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
-    if (u >= A.U) return;
-  } else {
-    x.lane_ = threadIdx.x;
-    x.G_ = blockDim.x;
-    x.arena = kf_dyn_smem;
-    u = blockIdx.x;
-  }
   run_unit<MK, MODE>(x, A, u);
   if (x.overflow) __trap();
 }
@@ -256,13 +221,12 @@ __global__ void __launch_bounds__(128, BWD ? 2 : 3) kf_rowsU_kernel(const __grid
 
 // Fused row-per-lane, warp-per-unit programs for large systems with the m^3 products on the FP64 tensor cores
 // (kf_rowsD.cuh); MK = MK_STD or MK_STEADY.  BWD = adjoint, NEED_T = with T-bar.
-#ifndef KFB_ROWSH_MINB
-// 16 x 16 tiles (k_states 10..16): 12 warps per SM, <= 168 registers.  Seasonal period 12, 65,536 x 1000, swizzled tiles:
-// 2 -> 241 ms, 3 -> 231 ms, 4 -> 250 ms (128 registers: the adjoint spills 150-390 bytes per thread).
-#define KFB_ROWSH_MINB 3
-#endif
+// Resident CTAs per SM with 16 x 16 tiles (k_states 10..16): 12 warps per SM, <= 168 registers.  Seasonal period 12,
+// 65,536 x 1000, swizzled tiles: 2 -> 241 ms, 3 -> 231 ms, 4 -> 250 ms (128 registers: the adjoint spills 150-390 bytes
+// per thread).
+constexpr int ROWSH_MIN_BLOCKS = 3;
 template <int M, int P, int MK, bool BWD, bool NEED_T>
-__global__ void __launch_bounds__(128, M <= 16 ? KFB_ROWSH_MINB : 1) kf_rowsD_kernel(const __grid_constant__ KfArgs A) {
+__global__ void __launch_bounds__(128, M <= 16 ? ROWSH_MIN_BLOCKS : 1) kf_rowsD_kernel(const __grid_constant__ KfArgs A) {
   extern __shared__ __align__(16) double kf_dyn_smem[];
   constexpr int per_unit = BWD ? RowsDLayout<M, P, NEED_T>::bwd_doubles : RowsDLayout<M, P, false>::fwd_doubles;
   const int warp = threadIdx.x >> 5;
@@ -275,7 +239,7 @@ __global__ void __launch_bounds__(128, M <= 16 ? KFB_ROWSH_MINB : 1) kf_rowsD_ke
 
 // same mapping, all six outputs of the reference (rowsD_forward_full)
 template <int M, int P, int MK>
-__global__ void __launch_bounds__(128, M <= 16 ? KFB_ROWSH_MINB : 1) kf_rowsDfull_kernel(const __grid_constant__ KfArgs A) {
+__global__ void __launch_bounds__(128, M <= 16 ? ROWSH_MIN_BLOCKS : 1) kf_rowsDfull_kernel(const __grid_constant__ KfArgs A) {
   extern __shared__ __align__(16) double kf_dyn_smem[];
   constexpr int per_unit = RowsDLayout<M, P, false>::fwd_doubles;
   const int warp = threadIdx.x >> 5;
@@ -299,25 +263,10 @@ template <bool BWD, bool WARP>
 __global__ void kf_dare_kernel(const __grid_constant__ DareArgs D, int arena_doubles) {
   extern __shared__ __align__(16) double kf_dyn_smem[];
   CoopCtx x;
-  x.set_dims(D.m, D.p);
-  x.off = 0;
-  x.cap = arena_doubles;
-  x.overflow = false;
-  long long u;
-  const long long count = BWD ? D.U : D.nD;
-  if (WARP) {
-    const int warp = threadIdx.x >> 5;
-    x.lane_ = threadIdx.x & 31;
-    x.G_ = 32;
-    x.arena = kf_dyn_smem + (size_t)warp * arena_doubles;
-    u = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
-    if (u >= count) return;
-  } else {
-    x.lane_ = threadIdx.x;
-    x.G_ = blockDim.x;
-    x.arena = kf_dyn_smem;
-    u = blockIdx.x;
-  }
+  x.init(D.m, D.p, WARP ? kf_dyn_smem + (size_t)(threadIdx.x >> 5) * arena_doubles : kf_dyn_smem, arena_doubles,
+         WARP ? threadIdx.x & 31 : threadIdx.x, WARP ? 32 : blockDim.x);
+  const long long u = coop_unit<WARP>();
+  if (WARP && u >= (BWD ? D.U : D.nD)) return;
   x.red = x.bump(34);
   if (BWD) {
     const long long d = u / D.n_series;
@@ -353,24 +302,10 @@ template <bool WARP>
 __global__ void __launch_bounds__(WARP ? 128 : 256) kf_smoother_kernel(const __grid_constant__ SmoothArgs S, int arena_doubles) {
   extern __shared__ __align__(16) double kf_dyn_smem[];
   CoopCtx x;
-  x.set_dims(S.m, 1);
-  x.off = 0;
-  x.cap = arena_doubles;
-  x.overflow = false;
-  long long u;
-  if (WARP) {
-    const int warp = threadIdx.x >> 5;
-    x.lane_ = threadIdx.x & 31;
-    x.G_ = 32;
-    x.arena = kf_dyn_smem + (size_t)warp * arena_doubles;
-    u = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
-    if (u >= S.U) return;
-  } else {
-    x.lane_ = threadIdx.x;
-    x.G_ = blockDim.x;
-    x.arena = kf_dyn_smem;
-    u = blockIdx.x;
-  }
+  x.init(S.m, 1, WARP ? kf_dyn_smem + (size_t)(threadIdx.x >> 5) * arena_doubles : kf_dyn_smem, arena_doubles,
+         WARP ? threadIdx.x & 31 : threadIdx.x, WARP ? 32 : blockDim.x);
+  const long long u = coop_unit<WARP>();
+  if (WARP && u >= S.U) return;
   x.red = x.bump(34);
   smoother_unit(x, S, u);
   if (x.overflow) __trap();
@@ -388,7 +323,7 @@ __global__ void __launch_bounds__(128) kf_smoother_thread_kernel(const __grid_co
 typedef cudaError_t (*smoother_launch_fn)(const SmoothArgs& S, cudaStream_t s);
 smoother_launch_fn find_smoother_thread_launcher(int m);
 
-// launchers implemented in kf_thread_m*.cu / kf_coop.cu
+// launchers implemented in kf_thread.cu / kf_coopT.cu / kf_coop.cu
 typedef cudaError_t (*thread_launch_fn)(const KfArgs& A, bool bwd, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 thread_launch_fn find_thread_launcher(int m, int p, int mk, bool tv = false);
 cudaError_t launch_coop(const KfArgs& A, bool bwd, cudaStream_t s);

@@ -202,8 +202,7 @@ KFB_HD void forward_unit_pred(X& x, const KfArgs& A, long long u) {
 // adjoint
 // ------------------------------------------------------------------------------------------------
 // One step's inputs for the adjoint: predicted moments of step t and everything that depends only on them
-// (innovation, gain, closed-loop matrix).  None of it depends on the adjoint state, so with X::PIPELINE the set of
-// step t-1 is computed while the adjoint of step t is in flight (two independent dependency chains per thread).
+// (innovation, gain, closed-loop matrix).  None of it depends on the adjoint state.
 template <class X>
 struct StepSet {
   typename X::template Buf<SZ_M> a;
@@ -224,7 +223,6 @@ KFB_HD void backward_unit_pred(X& x, const KfArgs& A, long long u) {
   typename X::template Buf<SZ_PP> Hb(x), Fb(x), Gb(x), Q1(x);
   typename X::template Buf<SZ_P> db(x), vb(x);
   StepSet<X> S0(x);
-  StepSet<X> S1(X::PIPELINE ? StepSet<X>(x) : S0);
 
   const double* Tp = A.T.p + draw * A.T.bs;
   const double* Zp = A.Z.p + draw * A.Z.bs;
@@ -423,21 +421,9 @@ KFB_HD void backward_unit_pred(X& x, const KfArgs& A, long long u) {
     }
   };
 
-  if (!X::PIPELINE) {
-    for (int t = n - 1; t >= 0; --t) {
-      prepare(t, S0);
-      adjoint(t, S0);
-    }
-  } else {
-    prepare(n - 1, S0);
-    for (int t = n - 1; t >= 0; t -= 2) {
-      if (t >= 1) prepare(t - 1, S1);
-      adjoint(t, S0);
-      if (t >= 1) {
-        if (t >= 2) prepare(t - 2, S0);
-        adjoint(t - 1, S1);
-      }
-    }
+  for (int t = n - 1; t >= 0; --t) {
+    prepare(t, S0);
+    adjoint(t, S0);
   }
   if (A.ga0) KFB_FOR(i, m) A.ga0[u * m + i] = ab[i];
   if (MK == MK_STEADY) {

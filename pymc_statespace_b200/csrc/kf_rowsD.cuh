@@ -30,7 +30,7 @@ namespace kfb {
 //    fragment patterns and the 16-byte tile stores are all conflict free.  These kernels run 12-16 warps per SM and sat ON
 //    the shared-memory wavefront roof (93-96 % of the LSU peak), a quarter of it bank conflicts at LD = 18: 478 -> 323
 //    (forward) / 696 -> 537 (adjoint) wavefronts per step together with the predicated row loads; the full-output forward
-//    gained 14 %, the adjoint little (it is then bound by spills at 128 registers: see KFB_ROWSH_MINB).
+//    gained 14 %, the adjoint little (it is then bound by spills at 128 registers: see ROWSH_MIN_BLOCKS in kf_kernels.cuh).
 __host__ __device__ constexpr int rowsD_nt(int m) { return m <= 16 ? 2 : 4; }
 __host__ __device__ constexpr int rowsD_ld(int m) { return m <= 16 ? 16 : 34; }
 template <int LD>

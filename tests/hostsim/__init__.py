@@ -22,7 +22,7 @@ MK = {"standard": 0, "single": 0, "cholesky": 0, "univariate": 1, "steady_state"
 
 def build(force=False):
     src = os.path.join(HERE, "hostsim.cpp")
-    deps = [src] + [os.path.join(ROOT, "pymc_statespace_b200", "csrc", f) for f in ("kf_core.cuh", "kf_ctx.cuh", "kf_dare.cuh", "kf_pred.cuh", "kf_smooth.cuh", "kf_p1.cuh")]
+    deps = [src] + [os.path.join(ROOT, "pymc_statespace_b200", "csrc", f) for f in ("kf_core.cuh", "kf_ctx.cuh", "kf_dare.cuh", "kf_pred.cuh", "kf_smooth.cuh", "kf_p1.cuh", "kf_run.cuh")]
     if force or not os.path.exists(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
         subprocess.check_call(
             ["g++", "-O1", "-std=c++17", "-shared", "-fPIC", "-Wno-unknown-pragmas",

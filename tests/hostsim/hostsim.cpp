@@ -10,6 +10,7 @@
 #include "kf_dare.cuh"
 #include "kf_p1.cuh"
 #include "kf_pred.cuh"
+#include "kf_run.cuh"
 #include "kf_smooth.cuh"
 
 using namespace kfb;
@@ -17,16 +18,21 @@ using namespace kfb;
 static int g_p1 = 0;    // k_endog = 1: 1: forward + adjoint of kf_p1.cuh, 2: generic forward + kf_p1.cuh adjoint
 static int g_pred = 0;  // 1: run the one-step-predictor programs (kf_pred.cuh) where they exist
 
+// g_pred: the kernels' programs (kf_run.cuh: run_unit); otherwise the two-stage programs, the reference the
+// one-step-predictor form is checked against.
 template <int MK, class X>
-static void run_both(X& x, KfArgs& A, int do_bwd) {
-  constexpr bool PRED = (MK == MK_STD || MK == MK_STEADY);
-  if (A.ll_obs || A.fs) forward_unit<MK, true>(x, A, 0);
-  else if (g_pred && PRED) forward_unit_pred<MK == MK_STEADY ? MK_STEADY : MK_STD>(x, A, 0);
+static void run_adjoint(X& x, const KfArgs& A) {
+  if (g_pred) run_unit<MK, 2>(x, A, 0);
+  else backward_unit<MK>(x, A, 0);
+}
+
+// With per-step outputs requested the forward pass is the kernels' full-output one, `full`.
+template <int MK, class X, class Full>
+static void run_both(X& x, KfArgs& A, int do_bwd, Full&& full) {
+  if (kernel_mode(A, false) == 1) full();
+  else if (g_pred) run_unit<MK, 0>(x, A, 0);
   else forward_unit<MK, false>(x, A, 0);
-  if (do_bwd) {
-    if (g_pred && PRED) backward_unit_pred<MK == MK_STEADY ? MK_STEADY : MK_STD>(x, A, 0);
-    else backward_unit<MK>(x, A, 0);
-  }
+  if (do_bwd) run_adjoint<MK>(x, A);
 }
 
 // The k_endog = 1 kernels' instantiation choice (kf_p1.cuh: with_forward_variant / with_adjoint_variant), with the tape
@@ -53,12 +59,10 @@ static void run_p1(KfArgs& A, int do_bwd) {
   });
 }
 
-template <class X>
-static void run_kind(X& x, KfArgs& A, int do_bwd) {
-  if (A.math_kind == MK_STD) run_both<MK_STD>(x, A, do_bwd);
-  else if (A.math_kind == MK_UNIV) run_both<MK_UNIV>(x, A, do_bwd);
-  else if (A.math_kind == MK_STEADY) run_both<MK_STEADY>(x, A, do_bwd);
-  else if (A.math_kind == MK_CHOLS) run_both<MK_CHOLS>(x, A, do_bwd);
+// run-time dims: the generic kernels' full-output forward is run_unit<MK, 1>
+template <int MK>
+static void run_coop(CoopCtx& x, KfArgs& A) {
+  run_both<MK>(x, A, 0, [&] { run_unit<MK, 1>(x, A, 0); });
 }
 
 extern "C" int hostsim_run(int mk, int m, int p, int n, const double* y, const double* a0, const double* P0,
@@ -100,40 +104,32 @@ extern "C" int hostsim_run(int mk, int m, int p, int n, const double* y, const d
     return 2;
   }
   const bool tv_any = ts[0] || ts[1] || ts[2] || ts[3] || ts[4] || ts[5];
-  if (static_dims) {
-#define KFB_CASE(MM, PP)                                   \
-  if (m == MM && p == PP) {                                \
-    if (tv_any) { /* the time-varying instantiation (standard filter only, kf_thread_inst.inc pick_kind) */ \
-      if (mk != MK_STD) return 7;                          \
-      ThreadCtx<MM, PP, true> x{nullptr, nullptr, 0, 1};   \
-      run_both<MK_STD>(x, A, do_bwd);                      \
-      return 0;                                            \
-    }                                                      \
-    ThreadCtx<MM, PP> x{nullptr, nullptr, 0, 1};                         \
-    run_kind(x, A, do_bwd);                                \
-    return 0;                                              \
-  }
-    KFB_CASE(1, 1) KFB_CASE(2, 1) KFB_CASE(2, 2) KFB_CASE(3, 1) KFB_CASE(3, 2) KFB_CASE(3, 3)
-    KFB_CASE(4, 1) KFB_CASE(4, 2) KFB_CASE(4, 3)
-#undef KFB_CASE
-    return 2;
+  if (static_dims) {  // the thread-per-unit kernels' instantiations
+    const bool ok = with_thread_instance(m, p, mk, tv_any, [&](auto v) {
+      using V = decltype(v);
+      ThreadCtx<V::M, V::P, V::TV> x{nullptr, nullptr, 0, 1};
+      run_both<V::MK>(x, A, do_bwd, [&] { run_unit_full<V::M, V::P, V::MK, V::TV>(x, A, 0); });
+    });
+    return ok ? 0 : 2;
   }
   const int cap = coop_arena_doubles(m, p, true) + coop_arena_doubles(m, p, false);
   std::vector<double> arena((size_t)cap);
   CoopCtx x;
-  x.set_dims(m, p); x.lane_ = 0; x.G_ = 1; x.arena = arena.data(); x.cap = cap; x.overflow = false;
-  x.off = 0;
-  run_kind(x, A, 0);
+  x.init(m, p, arena.data(), cap, 0, 1);
+  if (mk == MK_STD) run_coop<MK_STD>(x, A);
+  else if (mk == MK_UNIV) run_coop<MK_UNIV>(x, A);
+  else if (mk == MK_STEADY) run_coop<MK_STEADY>(x, A);
+  else if (mk == MK_CHOLS) run_coop<MK_CHOLS>(x, A);
   const int fwd_used = x.off;
   if (fwd_used > coop_arena_doubles(m, p, false)) return 3;
   if (do_bwd) {
     x.off = 0;  // the adjoint re-uses the arena; the tape written by the forward pass lives in A.tape
     KfArgs B = A;
     B.loglik = nullptr; B.ll_obs = nullptr; B.fs = B.ps = B.fc = B.pc = nullptr; B.info = nullptr;
-    if (A.math_kind == MK_STD) { if (g_pred) backward_unit_pred<MK_STD>(x, B, 0); else backward_unit<MK_STD>(x, B, 0); }
-    else if (A.math_kind == MK_UNIV) backward_unit<MK_UNIV>(x, B, 0);
-    else if (A.math_kind == MK_CHOLS) backward_unit<MK_CHOLS>(x, B, 0);
-    else { if (g_pred) backward_unit_pred<MK_STEADY>(x, B, 0); else backward_unit<MK_STEADY>(x, B, 0); }
+    if (mk == MK_STD) run_adjoint<MK_STD>(x, B);
+    else if (mk == MK_UNIV) run_adjoint<MK_UNIV>(x, B);
+    else if (mk == MK_CHOLS) run_adjoint<MK_CHOLS>(x, B);
+    else run_adjoint<MK_STEADY>(x, B);
     if (x.off > coop_arena_doubles(m, p, true)) return 4;
   }
   return x.overflow ? 5 : 0;
@@ -145,7 +141,7 @@ extern "C" int hostsim_dare(int m, int p, const double* T, const double* Z, cons
   const int cap = dare_arena_doubles(m, p);
   std::vector<double> arena((size_t)cap);
   CoopCtx x;
-  x.set_dims(m, p); x.lane_ = 0; x.G_ = 1; x.arena = arena.data(); x.cap = cap; x.overflow = false; x.off = 0;
+  x.init(m, p, arena.data(), cap, 0, 1);
   x.red = x.bump(34);
   int info = dare_unit(x, T, Z, H, C, Pss, Gss);
   if (x.overflow) return 5;
@@ -165,7 +161,7 @@ extern "C" int hostsim_smoother(int n, int m, const double* T, const double* C, 
   const int cap = smoother_arena_doubles(m);
   std::vector<double> arena((size_t)cap);
   CoopCtx x;
-  x.set_dims(m, 1); x.lane_ = 0; x.G_ = 1; x.arena = arena.data(); x.cap = cap; x.overflow = false; x.off = 0;
+  x.init(m, 1, arena.data(), cap, 0, 1);
   x.red = x.bump(34);
   smoother_unit(x, S, 0);
   return x.overflow ? 5 : 0;
