@@ -64,6 +64,7 @@ enum {
 #define KFB_INFO_BAD_STRUCTURE 0x40000003   /* a KFB_FLAG_Z_UNIT0 / _H_ZERO / _T_COMPANION promise does not hold for this unit */
 #define KFB_INFO_NOT_STATIONARY 0x40000002 /* set by the host layer (KalmanLogp): stationary P0 requested but the      */
                                            /* Lyapunov doubling did not converge (spectral radius of T >= 1)            */
+#define KFB_INFO_NOT_PSD 0x40000004        /* kfb_simulation_smoother: P0, Q or H is not positive semi-definite         */
 
 /* flags */
 #define KFB_FLAG_CORRECTED 1u  /* strict_reference=False: fix SURVEY.md A.2 quirks Q1,Q4,Q5,Q6 */
@@ -231,6 +232,33 @@ kfb_status kfb_simulate(int64_t n_draws, int64_t sims_per_draw, int32_t n, int32
 kfb_status kfb_mvn_draws(int64_t n_units, int64_t sims_per_unit, int32_t n, int32_t k, const double *mus,
                          const double *covs, const double *z, const double *jitter, double *out, int32_t *info,
                          void *stream);
+
+/* Simulation smoother (Durbin & Koopman 2002, mean correction; not on the logp/grad path): joint draws of the state
+ * paths x_0..x_{n-1} from p(x | y, theta), sims_per_unit of them per unit.  Model: x_0 ~ N(a0, P0), y_t = Z x_t + d +
+ * eps_t (eps_t ~ N(0, H), t = 0..n-1), x_{t+1} = T x_t + c + R eta_t (eta_t ~ N(0, Q), t = 0..n-2) - the filters' model;
+ * NOT kfb_simulate's shifted convention obs[t] = Z states[t-1].  Per simulation:
+ *   1. x+_0 = a0 + S_P0 z_init, x+_{t+1} = T x+_t + c + R S_Q z_state_t, y+_t = Z x+_t + d + S_H z_obs_t
+ *      (S_A S_A^T = A: lower Cholesky that accepts PSD input - a pivot at or below 1e-10 times the largest diagonal
+ *      entry is zero and its column is zeroed, a pivot below -1e-10 times it is an error; H = 0: no observation noise);
+ *   2. y* = y - y+; a*_0 = 0, v_t = y*_t - Z a*_t, a*_{t+1} = T a*_t + K_t v_t, K_t = T P_t Z^T F_t^-1;
+ *   3. r_{n-1} = 0, r_{t-1} = Z^T F_t^-1 v_t + L_t^T r_t, L_t = T - K_t Z;
+ *   4. xhat_0 = P0 r_{-1}, xhat_{t+1} = T xhat_t + R Q R^T r_t;   5. states[s, t] = x+_t + xhat_t.
+ * A missing row (all of y_t NaN) has F_t^-1 = 0, K_t = 0.
+ * Inputs: desc gives sizes and batch strides; every time stride must be 0 (else KFB_ERR_UNSUPPORTED); filter_kind and
+ * flags are ignored.  k_states, k_endog, k_posdef <= 32 (else KFB_ERR_UNSUPPORTED).  predicted_covs[U, n+1, m, m] is
+ * the output of a preceding kfb_forward (standard filter, KFB_FLAG_CORRECTED) on the same desc and inputs
+ * (its row 0 is not read: P_0 is the input P0).  Simulation
+ * s = unit * sims_per_unit + k (S = U * sims_per_unit).  Normals, time-major: z_init[S, m], z_state[n-1, S, r] (may be
+ * NULL if n = 1), z_obs[n, S, p].  c, d may be NULL.  Output states[S, n, m]; info[U] (written, no zeroing needed):
+ * 0 ok, t+1 F_t not positive definite, -(t+1) y_t partly missing, KFB_INFO_NOT_PSD; a failing unit's paths are NaN.
+ * Workspace (kfb_simulation_smoother_workspace_bytes), each term rounded up to 256 bytes, with U = n_draws * n_series
+ * and S32 = S rounded up to a multiple of 32:  8 U n (m p + p p)  +  8 U (2 m m + m r + p p + r r)  +  8 n S32 p
+ *   +  8 (n - 1) S32 m  +  4 U. */
+kfb_status kfb_simulation_smoother_workspace_bytes(const kfb_desc *desc, int64_t sims_per_unit, size_t *bytes);
+kfb_status kfb_simulation_smoother(const kfb_desc *desc, const kfb_inputs *in, const double *predicted_covs,
+                                   int64_t sims_per_unit, const double *z_init, const double *z_state,
+                                   const double *z_obs, double *states, int32_t *info, void *workspace,
+                                   size_t workspace_bytes, void *stream);
 
 /* FP64 roofline denominator: `iters` dependent-chain DFMA rounds on every SM.  Returns through
  * h_flops the number of floating-point operations the launch executes (2 per FMA); the caller

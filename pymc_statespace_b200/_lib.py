@@ -29,6 +29,7 @@ KFB_FLAG_TIME_PARALLEL = 128
 KFB_INFO_DARE_FAILED = 0x40000001
 KFB_INFO_NOT_STATIONARY = 0x40000002
 KFB_INFO_BAD_STRUCTURE = 0x40000003
+KFB_INFO_NOT_PSD = 0x40000004
 
 KFB_OK, KFB_ERR_INVALID_ARG, KFB_ERR_UNSUPPORTED, KFB_ERR_WORKSPACE, KFB_ERR_CUDA = range(5)
 
@@ -92,6 +93,9 @@ EXPORTS = {
     "kfb_simulate": (_c_i32, [_c_i64, _c_i64, _c_i32, _c_i32, _c_i32, _c_i32, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _c_i64,
                               _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "kfb_mvn_draws": (_c_i32, [_c_i64, _c_i64, _c_i32, _c_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "kfb_simulation_smoother_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), _c_i64, ctypes.POINTER(ctypes.c_size_t)]),
+    "kfb_simulation_smoother": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _c_i64, _vp, _vp, _vp, _vp,
+                                         _vp, _vp, ctypes.c_size_t, _vp]),
     "kfb_fp64_peak": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),
     "kfb_fp64_peak_distinct": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),
 }

@@ -5,6 +5,7 @@
 #include "../../include/kfb200.h"
 #include "kf_aux.cuh"
 #include "kf_kernels.cuh"
+#include "kf_simsmooth.cuh"
 
 namespace kfb {
 
@@ -20,6 +21,7 @@ bool tpar_supported(int m, int p, int mk);
 cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
 bool tpar_smoother_supported(int m);
 cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
+cudaError_t launch_simulation_smoother(const ss::Args& A, cudaStream_t s);
 
 // k_states with launchers of their own, one object per size (kf_thread.cu: thread-per-unit filters and smoother;
 // kf_coopT.cu: compile-time-dims kernels; the tensor-core DARE in kf_coopT.cu from k_states 10).  The Makefile repeats
@@ -215,6 +217,30 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
     if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   }
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
+// Workspace of kfb_simulation_smoother: gain tape, per-unit factors, the u and r scratch of every simulation and the
+// per-unit status, each region rounded up to 256 bytes (the rule kfb200.h states).
+struct SsPlan {
+  size_t off_gain, off_fac, off_u, off_r, off_stat, total;
+};
+
+static kfb_status make_ss_plan(const kfb_desc* d, int64_t sims_per_unit, SsPlan* pl) {
+  if (!d || d->n_draws <= 0 || d->n_series <= 0 || d->n <= 0 || d->m <= 0 || d->p <= 0 || d->r <= 0 || sims_per_unit <= 0)
+    return KFB_ERR_INVALID_ARG;
+  if (d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts) return KFB_ERR_UNSUPPORTED;
+  if (d->m > ss::SS_MAX || d->p > ss::SS_MAX || d->r > ss::SS_MAX || d->n >= (1 << 29)) return KFB_ERR_UNSUPPORTED;
+  const long long U = d->n_draws * d->n_series;
+  const long long lanes = ss::warps_of(U * sims_per_unit) * 32;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+  pl->off_gain = take((size_t)U * d->n * ss::gain_stride(d->m, d->p) * 8);
+  pl->off_fac = take((size_t)U * ss::fac_stride(d->m, d->p, d->r) * 8);
+  pl->off_u = take((size_t)d->n * lanes * d->p * 8);
+  pl->off_r = take((size_t)(d->n - 1) * lanes * d->m * 8);
+  pl->off_stat = take((size_t)U * 4);
+  pl->total = off;
+  return KFB_OK;
 }
 
 }  // namespace kfb
@@ -464,6 +490,45 @@ kfb_status kfb_mvn_draws(int64_t n_units, int64_t sims_per_unit, int32_t n, int3
   if (k > 32) return KFB_ERR_UNSUPPORTED;
   cudaError_t e = launch_mvn_draws(n_units * sims_per_unit, sims_per_unit, n, k, mus, covs, z, jitter, out, info,
                                    (cudaStream_t)stream);
+  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
+kfb_status kfb_simulation_smoother_workspace_bytes(const kfb_desc* desc, int64_t sims_per_unit, size_t* bytes) {
+  if (!bytes) return KFB_ERR_INVALID_ARG;
+  SsPlan pl;
+  kfb_status st = make_ss_plan(desc, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  *bytes = pl.total;
+  return KFB_OK;
+}
+
+kfb_status kfb_simulation_smoother(const kfb_desc* desc, const kfb_inputs* in, const double* predicted_covs,
+                                   int64_t sims_per_unit, const double* z_init, const double* z_state,
+                                   const double* z_obs, double* states, int32_t* info, void* workspace,
+                                   size_t workspace_bytes, void* stream) {
+  SsPlan pl;
+  kfb_status st = make_ss_plan(desc, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  if (!in || !in->y || !in->a0 || !in->P0 || !in->T || !in->Z || !in->R || !in->H || !in->Q || !predicted_covs ||
+      !z_init || (desc->n > 1 && !z_state) || !z_obs || !states || !info)
+    return KFB_ERR_INVALID_ARG;
+  if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
+  char* ws = (char*)workspace;
+  ss::Args A;
+  std::memset(&A, 0, sizeof(A));
+  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
+  A.n = desc->n; A.m = desc->m; A.p = desc->p; A.r = desc->r;
+  A.y = {in->y, desc->y_bs, 0}; A.a0 = {in->a0, desc->a0_bs, 0}; A.P0 = {in->P0, desc->P0_bs, 0};
+  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
+  A.H = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
+  A.pc = predicted_covs; A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs; A.states = states; A.info = info;
+  A.gain = (double*)(ws + pl.off_gain); A.fac = (double*)(ws + pl.off_fac);
+  A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r); A.ustat = (int*)(ws + pl.off_stat);
+  cudaStream_t s = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(A.ustat, 0x7f, (size_t)A.U * 4, s);  // every word = ss::KEY_NONE
+  if (e != cudaSuccess) return cuda_fail(e);
+  e = launch_simulation_smoother(A, s);
+  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
 }
 

@@ -295,6 +295,45 @@ class KalmanLogp:
             out["filtered_covs"] = out["filtered_covs"][..., :m, :m].contiguous()
         return ss, sc, out
 
+    def sample_states(self, theta, n_simulations: int = 1, generator: Optional[torch.Generator] = None,
+                      z_init=None, z_state=None, z_obs=None) -> torch.Tensor:
+        """Joint draws of the latent state paths from p(x_0..x_{n-1} | y, theta) for every draw: the simulation smoother
+        of ``simulation.simulation_smoother`` (Durbin & Koopman 2002) after the theta scatter (and stationary P0), as
+        ``smooth()`` does.  Returns states [B * n_simulations, n, k_states] (draw-major); the paths of a failing draw are
+        NaN and ``sample_states_info`` holds the per-draw status.
+
+        Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
+        built with: the posterior of the states does not depend on the reference's as-coded likelihood quirks.  Normals
+        may be given as in ``simulation_smoother``, sized for the model's own k_states."""
+        from .simulation import _simulation_smoother
+
+        mats = self._scatter(self._check_theta(theta))
+        sp = self.spec
+        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
+        if getattr(self, "_ss_kalman", None) is None:
+            self._ss_kalman = BatchedKalman("standard", self.n, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
+                                            strict_reference=False, device=self.device)
+        if z_init is not None and m != m0:  # padded model: the extra states are identically zero, their normals unused
+            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
+        if z_init is None and m != m0:
+            z_init = torch.nn.functional.pad(
+                torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator), (0, m - m0))
+        states, info = _simulation_smoother(self._ss_kalman, self.y, mats, int(n_simulations), z_init, z_state, z_obs,
+                                            generator)
+        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
+            bad = self._lyap[2] != 0
+            info = torch.where(bad, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
+            states.view(self.B, -1)[bad] = float("nan")
+        self._ss_info = info
+        return states[..., :m0].contiguous() if m != m0 else states
+
+    @property
+    def sample_states_info(self) -> torch.Tensor:
+        """Per-draw status of the last ``sample_states`` (int32, 0 = ok; t+1: F_t not positive definite; -(t+1): y_t
+        partly missing; KFB_INFO_NOT_PSD: P0, Q or H not positive semi-definite; KFB_INFO_NOT_STATIONARY as in
+        ``info``).  A failing draw's paths are NaN."""
+        return self._ss_info
+
     def logp(self, theta) -> torch.Tensor:
         mats = self._scatter(self._check_theta(theta))
         out = self.kalman.forward(self.y, *[mats[k] for k in MATRICES], outputs=("loglik",))
