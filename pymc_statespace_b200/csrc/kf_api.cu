@@ -6,6 +6,7 @@
 #include "kf_aux.cuh"
 #include "kf_kernels.cuh"
 #include "kf_simsmooth.cuh"
+#include "kf_tpar.cuh"
 
 namespace kfb {
 
@@ -17,9 +18,7 @@ bool p1_adjoint_supported(int m, int p, int mk);
 cudaError_t launch_p1_adjoint(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 cudaError_t launch_p1_forward(const KfArgs& A, int y_smem_doubles, int bulk_ok, cudaStream_t s);
 
-bool tpar_supported(int m, int p, int mk);
 cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
-bool tpar_smoother_supported(int m);
 cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
 cudaError_t launch_simulation_smoother(const ss::Args& A, cudaStream_t s);
 
@@ -80,7 +79,8 @@ struct Plan {
   int mk;
   double ll_const, d_sign;
   bool tv_any, use_thread;
-  bool compressed;   // k_endog = 1 kernels with all four structure promises: the compressed tape (CTape, kf_core.cuh)
+  bool p1;           // k_endog = 1 with shared observations on the thread-per-unit path: the kernels of kf_p1.cu
+  int struct_flags;  // KfArgs::struct_flags; KF_STRUCT_COMPRESSED: the compressed tape (CTape, kf_core.cuh)
   bool tpar;         // KFB_FLAG_TIME_PARALLEL: one CTA per unit, scans over time (kf_tpar.cu); tape [u][t][a_t, P_t]
   long long U, nD;
   int nTC;           // time entries of C = R Q R^T (1 or n)
@@ -91,28 +91,12 @@ struct Plan {
 static kfb_status make_plan(const kfb_desc* d, bool save, Plan* pl) {
   if (!d || d->n_draws <= 0 || d->n_series <= 0 || d->n <= 0 || d->m <= 0 || d->p <= 0 || d->r <= 0)
     return KFB_ERR_INVALID_ARG;
-  const bool corrected = (d->flags & KFB_FLAG_CORRECTED) != 0;
-  const double l2pi = KF_LOG_2PI;
-  switch (d->filter_kind) {
-    case KFB_STANDARD:
-      pl->mk = MK_STD; pl->ll_const = corrected ? d->p * l2pi : l2pi; pl->d_sign = 1.0; break;
-    case KFB_SINGLE:
-      if (d->p != 1) return KFB_ERR_INVALID_ARG;  // assert_data_is_1d, kalman_filter.py:19,329
-      pl->mk = MK_STD; pl->ll_const = l2pi; pl->d_sign = corrected ? 1.0 : -1.0; break;
-    case KFB_CHOLESKY:
-      // as coded the filter is exact only for p = 1 (SURVEY A.2-Q4); p > 1 strict = bug-compatible MK_CHOLS
-      pl->mk = (d->p != 1 && !corrected) ? MK_CHOLS : MK_STD; pl->ll_const = d->p * l2pi; pl->d_sign = 1.0; break;
-    case KFB_UNIVARIATE:
-      pl->mk = MK_UNIV; pl->ll_const = 0.0; pl->d_sign = 1.0; break;
-    case KFB_STEADY_STATE:
-      pl->mk = MK_STEADY; pl->ll_const = corrected ? d->p * l2pi : l2pi; pl->d_sign = corrected ? 1.0 : 0.0; break;
-    default: return KFB_ERR_INVALID_ARG;
-  }
+  if (!filter_rule(d->filter_kind, d->p, d->flags, &pl->mk, &pl->ll_const, &pl->d_sign)) return KFB_ERR_INVALID_ARG;
   pl->tv_any = d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts;
   if (pl->tv_any && (pl->mk == MK_UNIV || pl->mk == MK_STEADY)) return KFB_ERR_UNSUPPORTED;
   // time-parallel form: k_endog = 1, k_states <= 4, standard-family filters only
   pl->tpar = (d->flags & KFB_FLAG_TIME_PARALLEL) != 0;
-  if (pl->tpar && !tpar_supported(d->m, d->p, pl->mk)) return KFB_ERR_UNSUPPORTED;
+  if (pl->tpar && !tpar::supported(d->m, d->p, pl->mk)) return KFB_ERR_UNSUPPORTED;
   pl->U = d->n_draws * d->n_series;
   pl->nD = d->n_draws;
   pl->nTC = (d->R_ts || d->Q_ts) ? d->n : 1;
@@ -131,17 +115,18 @@ static kfb_status make_plan(const kfb_desc* d, bool save, Plan* pl) {
     pl->off_dinfo = take((size_t)(pl->nD + 1) / 2);
   }
   // decided from the descriptor alone, so that workspace sizing, the forward pass and the adjoint always agree
-  constexpr uint32_t kPromises = KFB_FLAG_Z_UNIT0 | KFB_FLAG_H_ZERO | KFB_FLAG_T_COMPANION | KFB_FLAG_NO_MISSING;
-  pl->compressed = pl->use_thread && !pl->tv_any && d->y_bs == 0 && d->n_series == 1 && (d->flags & kPromises) == kPromises &&
-                   !(d->flags & KFB_FLAG_GENERIC_ADJOINT) && p1_adjoint_supported(d->m, d->p, pl->mk);
+  pl->p1 = pl->use_thread && !pl->tv_any && d->y_bs == 0 && d->n_series == 1 && !(d->flags & KFB_FLAG_GENERIC_ADJOINT) &&
+           p1_adjoint_supported(d->m, d->p, pl->mk);
+  pl->struct_flags = struct_flags_of(d->flags, d->p, d->Z_ts || d->H_ts, pl->p1);
+  const bool compressed = (pl->struct_flags & KF_STRUCT_COMPRESSED) != 0;
   pl->off_tape = pl->off_gC = 0;
   if (pl->tpar) {
     // the forward pass always writes the tape (its parallel map reads the predicted moments back from it)
     pl->off_tape = take((size_t)pl->U * d->n * (d->m + d->m * d->m));
     if (save) pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
   } else if (save) {
-    const size_t entries = pl->compressed ? (size_t)ctape_steps_padded(d->n) * ctape_entry_doubles(d->m)
-                                          : (size_t)(d->n > 1 ? d->n - 1 : 0) * tape_width(d->m);
+    const size_t entries = compressed ? (size_t)ctape_steps_padded(d->n) * ctape_entry_doubles(d->m)
+                                      : (size_t)(d->n > 1 ? d->n - 1 : 0) * tape_width(d->m);
     pl->off_tape = take((size_t)tape_units_padded(pl->U) * entries);
     pl->off_gC = take((size_t)pl->U * pl->nTC * d->m * d->m);
     if (pl->mk == MK_STEADY) {
@@ -172,10 +157,7 @@ static void fill_args(const kfb_desc* d, const kfb_inputs* in, const Plan& pl, c
   }
   A->ll_const = pl.ll_const;
   A->d_sign = pl.d_sign;
-  if (d->p == 1 && !d->Z_ts && !d->H_ts)
-    A->struct_flags = ((d->flags & KFB_FLAG_Z_UNIT0) ? KF_STRUCT_Z_UNIT0 : 0) |
-                      ((d->flags & KFB_FLAG_H_ZERO) ? KF_STRUCT_H_ZERO : 0) |
-                      ((d->flags & KFB_FLAG_T_COMPANION) ? KF_STRUCT_T_COMPANION : 0);
+  A->struct_flags = pl.struct_flags;
 }
 
 static kfb_status cuda_fail(cudaError_t e) {
@@ -193,20 +175,14 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
       ysm = (int)ydoubles;
       bulk_ok = ((uintptr_t)A.y.p % 16 == 0) ? 1 : 0;
     }
+    if ((A.struct_flags & KF_STRUCT_COMPRESSED) && bwd && (A.gZ || A.gH)) return KFB_ERR_UNSUPPORTED;  // Z, H constant
     // k_endog = 1, shared observations: the specialised adjoint with the TMA tape ring (kf_p1.cu)
-    const bool p1_ok = !pl.tv_any && d->y_bs == 0 && d->n_series == 1 && !(d->flags & KFB_FLAG_GENERIC_ADJOINT) &&
-                       p1_adjoint_supported(d->m, d->p, pl.mk);
-    // all four structure promises on the k_endog = 1 kernels: compressed tape entries (kf_p1.cuh, ZU_REDUCED) - decided
-    // from the descriptor alone (make_plan), so that the forward pass and the adjoint always agree on the format
-    KfArgs B = A;
-    if (pl.compressed) B.struct_flags |= KF_STRUCT_COMPRESSED;
-    if (pl.compressed && bwd && (A.gZ || A.gH)) return KFB_ERR_UNSUPPORTED;  // Z, H were promised constant
-    if (p1_ok && bwd)
-      e = launch_p1_adjoint(B, ysm, bulk_ok, s);
-    else if (p1_ok && !wants_step_outputs(A))
-      e = launch_p1_forward(B, ysm, bulk_ok, s);
+    if (pl.p1 && bwd)
+      e = launch_p1_adjoint(A, ysm, bulk_ok, s);
+    else if (pl.p1 && !wants_step_outputs(A))
+      e = launch_p1_forward(A, ysm, bulk_ok, s);
     else
-      e = find_thread_launcher(d->m, d->p, pl.mk, pl.tv_any)(B, bwd, ysm, bulk_ok, s);
+      e = find_thread_launcher(d->m, d->p, pl.mk, pl.tv_any)(A, bwd, ysm, bulk_ok, s);
   } else {
     // sub-warp kernels with compile-time dims need uniform control flow across the units of a warp:
     // static matrices and ONE observation stream shared by every unit
@@ -383,7 +359,7 @@ kfb_status kfb_smoother_ex(int64_t n_draws, int64_t n_series, int32_t n, int32_t
     return KFB_ERR_INVALID_ARG;
   if (flags & ~KFB_FLAG_TIME_PARALLEL) return KFB_ERR_INVALID_ARG;
   const bool tpar = (flags & KFB_FLAG_TIME_PARALLEL) != 0;
-  if (tpar && !tpar_smoother_supported(m)) return KFB_ERR_UNSUPPORTED;
+  if (tpar && !tpar::with_instance(m, [](auto) {})) return KFB_ERR_UNSUPPORTED;  // k_states 1..4
   const bool C_batched = R_bs || Q_bs;
   const long long nDC = C_batched ? n_draws : 1;
   const size_t need = (size_t)nDC * m * m * sizeof(double);

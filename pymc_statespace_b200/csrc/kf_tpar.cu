@@ -132,16 +132,10 @@ cudaError_t launch_tpar_m(const KfArgs& A, bool bwd, cudaStream_t s) {
 
 }  // namespace
 
-bool tpar_supported(int m, int p, int mk) { return p == 1 && mk == MK_STD && m >= 1 && m <= 4; }
-
 cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s) {
-  switch (A.m) {
-    case 1: return launch_tpar_m<1>(A, bwd, s);
-    case 2: return launch_tpar_m<2>(A, bwd, s);
-    case 3: return launch_tpar_m<3>(A, bwd, s);
-    case 4: return launch_tpar_m<4>(A, bwd, s);
-    default: return cudaErrorInvalidConfiguration;
-  }
+  cudaError_t e = cudaErrorInvalidConfiguration;
+  tpar::with_instance(A.m, [&](auto M) { e = launch_tpar_m<M>(A, bwd, s); });
+  return e;
 }
 
 }  // namespace kfb

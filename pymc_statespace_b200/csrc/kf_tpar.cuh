@@ -31,9 +31,10 @@
 //
 // Each phase of a pass is a function over one chunk [lo, hi) of one unit (filt_fold_chunk .. adjoint_chunk); the kernels
 // of kf_tpar.cu add only the CTA scans, the fallback decisions and the reductions.  Everything here is KFB_HD so that
-// tests/tpar_host runs the same chunk functions on the host, with its own scans, and checks them against the oracle.
+// the host build (tests/hostsim) runs the same chunk functions, with its own scans, and checks them against the oracle.
 #pragma once
 #include <climits>
+#include <type_traits>
 
 #include "kf_ctx.cuh"
 #include "kf_pred.cuh"
@@ -49,6 +50,22 @@ using TX = ThreadCtx<M, 1, false>;
 // longer fit either, so those run 128 threads (a few more steps per thread, one scan level less).
 template <int M>
 KFB_HD constexpr int tpar_threads() { return M <= 2 ? 256 : 128; }
+
+// The one list of k_states of the time-parallel kernels (filter and smoother), for their launchers and the host build:
+// run(std::integral_constant<int, M>{}) for M = m in 1..4; false for any other m.
+template <class Run>
+bool with_instance(int m, Run&& run) {
+  switch (m) {
+    case 1: run(std::integral_constant<int, 1>{}); return true;
+    case 2: run(std::integral_constant<int, 2>{}); return true;
+    case 3: run(std::integral_constant<int, 3>{}); return true;
+    case 4: run(std::integral_constant<int, 4>{}); return true;
+    default: return false;
+  }
+}
+
+// The filters of the time-parallel form: k_endog = 1 and the standard-family update.
+inline bool supported(int m, int p, int mk) { return p == 1 && mk == MK_STD && with_instance(m, [](auto) {}); }
 
 // Steps [lo, hi) of chunk k of K over n steps: contiguous chunks of ceil(n / K) steps; the last ones may be short or empty.
 struct Chunk {

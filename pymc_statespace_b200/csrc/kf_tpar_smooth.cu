@@ -43,16 +43,10 @@ cudaError_t launch_tpar_smoother_m(const SmoothArgs& S, cudaStream_t s) {
 
 }  // namespace
 
-bool tpar_smoother_supported(int m) { return m >= 1 && m <= 4; }
-
 cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s) {
-  switch (S.m) {
-    case 1: return launch_tpar_smoother_m<1>(S, s);
-    case 2: return launch_tpar_smoother_m<2>(S, s);
-    case 3: return launch_tpar_smoother_m<3>(S, s);
-    case 4: return launch_tpar_smoother_m<4>(S, s);
-    default: return cudaErrorInvalidConfiguration;
-  }
+  cudaError_t e = cudaErrorInvalidConfiguration;
+  tpar::with_instance(S.m, [&](auto M) { e = launch_tpar_smoother_m<M>(S, s); });
+  return e;
 }
 
 }  // namespace kfb

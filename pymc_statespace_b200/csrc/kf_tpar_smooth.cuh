@@ -21,8 +21,8 @@
 //     A scan over products of gains has no accuracy guarantee, so on any drift the whole unit is re-run by the
 //     sequential recursion (smoother_unit's steps) - this smoother never returns what the sequential one would not.
 //
-// Everything here is KFB_HD so that tests/tpar_host runs the same fold and walk on the host and checks them against the
-// oracle.
+// Everything here is KFB_HD so that the host build of the kernels (tests/hostsim) runs the same fold and walk and checks
+// them against the oracle.
 #pragma once
 #include "kf_smooth.cuh"
 #include "kf_tpar.cuh"

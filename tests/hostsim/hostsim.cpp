@@ -1,9 +1,8 @@
-// hostsim.cpp - TEST-ONLY host build of the device step programs in
-// pymc_statespace_b200/csrc/kf_core.cuh.  The container that builds this repo has no GPU, so the
-// Kalman/adjoint math is debugged here against the oracle before it is run on a B200.  This file is
-// NOT part of the product: the package never loads it, and it cannot be reached from any public API.
-//
-//   g++ -O1 -shared -fPIC -I pymc_statespace_b200/csrc tests/hostsim/hostsim.cpp -o tests/hostsim/_hostsim.so
+// hostsim.cpp - TEST-ONLY host build of the device step programs in pymc_statespace_b200/csrc/kf_core.cuh, kf_pred.cuh
+// and kf_p1.cuh, the DARE and the RTS smoother.  The container that builds this repo has no GPU, so the Kalman/adjoint
+// math is debugged here against the oracle before it is run on a B200.  This file is NOT part of the product: the package
+// never loads it, and it cannot be reached from any public API.  tests/hostsim/__init__.py builds it.
+#include <algorithm>
 #include <vector>
 
 #include "kf_ctx.cuh"
@@ -55,7 +54,7 @@ static void run_p1(KfArgs& A, int do_bwd) {
     constexpr int KT = p1::tape_doubles<M, V::ZU>;
     using Tape = p1::DirectTape<M, KT>;
     Tape tape{A.tape + (long long)(A.n - 2) * KT * 32, (long long)KT * 32, 32};
-    p1::backward_unit_p1<M, V::NEED_Z, V::NEED_H, V::HAS_GOBS, Tape, V::ZU, V::H0>(A, 0, true, A.y.p, tape);
+    p1::backward_unit_p1<M, V::NEED_Z, V::NEED_H, V::HAS_GOBS, Tape, V::ZU, V::H0, V::CD>(A, 0, true, A.y.p, tape);
   });
 }
 
@@ -65,32 +64,38 @@ static void run_coop(CoopCtx& x, KfArgs& A) {
   run_both<MK>(x, A, 0, [&] { run_unit<MK, 1>(x, A, 0); });
 }
 
-extern "C" int hostsim_run(int mk, int m, int p, int n, const double* y, const double* a0, const double* P0,
-                           const double* T, const double* Z, const double* H, const double* C, const double* c,
-                           const double* d, const double* Pss, const double* Gss, const long long* ts /*T,Z,H,C,c,d*/,
-                           double ll_const, double d_sign, int static_dims, double* loglik, double* ll_obs, double* fs,
-                           double* ps, double* fc, double* pc, int* info, int do_bwd, const double* g_loglik,
-                           const double* g_ll_obs, double* ga0, double* gP0, double* gT, double* gZ, double* gH,
-                           double* gC, double* gc, double* gd, double* gPss, double* gGss) {
+// kind, flags: the C ABI's filter kind and KFB_FLAG_* bits, applied by the library's rules (kf_run.cuh).  The other
+// choices exist for the tests only: static_dims, the thread-per-unit instantiations (else the run-time-dims context);
+// pred, the one-step-predictor programs (else the two-stage reference programs); p1, the k_endog = 1 kernels (g_p1).
+extern "C" int hostsim_run(int kind, unsigned flags, int m, int p, int n, const double* y, const double* a0,
+                           const double* P0, const double* T, const double* Z, const double* H, const double* C,
+                           const double* c, const double* d, const double* Pss, const double* Gss,
+                           const long long* ts /*T,Z,H,C,c,d*/, int static_dims, int pred, int p1, double* loglik,
+                           double* ll_obs, double* fs, double* ps, double* fc, double* pc, int* info, int do_bwd,
+                           const double* g_loglik, const double* g_ll_obs, double* ga0, double* gP0, double* gT,
+                           double* gZ, double* gH, double* gC, double* gc, double* gd, double* gPss, double* gGss) {
   KfArgs A;
   std::memset(&A, 0, sizeof(A));
-  A.U = 1; A.n_series = 1; A.n = n; A.m = m; A.p = p; A.math_kind = mk;
+  if (!filter_rule(kind, p, flags, &A.math_kind, &A.ll_const, &A.d_sign)) return 1;
+  const int mk = A.math_kind;
+  A.U = 1; A.n_series = 1; A.n = n; A.m = m; A.p = p;
   A.y = {y, 0, 0}; A.a0 = {a0, 0, 0}; A.P0 = {P0, 0, 0};
   A.T = {T, 0, ts[0]}; A.Z = {Z, 0, ts[1]}; A.H = {H, 0, ts[2]}; A.C = {C, 0, ts[3]};
   A.c = {c, 0, ts[4]}; A.d = {d, 0, ts[5]};
   A.Pss = {Pss, 0, 0}; A.Gss = {Gss, 0, 0};
-  A.ll_const = ll_const; A.d_sign = d_sign;
   A.loglik = loglik; A.ll_obs = ll_obs; A.fs = fs; A.ps = ps; A.fc = fc; A.pc = pc; A.info = info;
-  std::vector<double> tape((size_t)(n > 1 ? n - 1 : 1) * tape_width(m) * 32);  // ThreadCtx layout: whole warps of units
+  A.struct_flags = struct_flags_of(flags, p, ts[1] || ts[2], p1 != 0);
+  // either tape format (g_p1 == 2 writes full entries under the compressed flag), in whole warps of units
+  const long long entries =
+      std::max((long long)std::max(n - 1, 1) * tape_width(m), ctape_steps_padded(n) * ctape_entry_doubles(m));
+  std::vector<double> tape((size_t)entries * 32);
   A.tape = tape.data();
   A.g_loglik = g_loglik; A.g_ll_obs = g_ll_obs;
   A.ga0 = ga0; A.gP0 = gP0; A.gT = gT; A.gZ = gZ; A.gH = gH; A.gC = gC; A.gc = gc; A.gd = gd;
   A.gPss = gPss; A.gGss = gGss;
 
-  g_pred = (static_dims >> 1) & 1;
-  A.struct_flags = (static_dims >> 4) & 15;  // bits 4..7: KF_STRUCT_Z_UNIT0, _H_ZERO, _T_COMPANION, _COMPRESSED
-  g_p1 = (static_dims >> 2) & 3;  // 1: specialised forward + adjoint, 2: generic forward + specialised adjoint
-  static_dims &= 1;
+  g_pred = pred;
+  g_p1 = p1;
   if (g_p1) {
     if (p != 1 || mk != MK_STD || ts[0] || ts[1] || ts[2] || ts[3] || ts[4] || ts[5]) return 7;
     if ((A.struct_flags & p1::REDUCED_FLAGS) == p1::REDUCED_FLAGS && (gZ || gH)) return 7;  // the C ABI refuses it too

@@ -76,25 +76,17 @@ def test_as_coded_cholesky_filter_multivariate(dims):
 
 
 def test_dare_solver_and_adjoint_on_host():
-    import ctypes
-
     import scipy.linalg
     import torch
 
     from pymc_statespace_b200.models import arma_spec, trend_seasonal_spec
 
-    lib = hostsim.build()
-    vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
-
     def run(T, Z, H, C, grad_tol):
         m, p = T.shape[0], Z.shape[0]
         T, Z, H, C = [np.ascontiguousarray(v, dtype=float) for v in (T, Z, H, C)]
-        Pss, Gss = np.zeros((m, m)), np.zeros((p, p))
         gP, gG = np.random.default_rng(0).normal(size=(m, m)), np.random.default_rng(1).normal(size=(p, p))
-        gT, gZ, gH, gC = np.zeros((m, m)), np.zeros((p, m)), np.zeros((p, p)), np.zeros((m, m))
-        rc = lib.hostsim_dare(m, p, vp(T), vp(Z), vp(H), vp(C), vp(Pss), vp(Gss), 1, vp(gP), vp(gG), vp(gT), vp(gZ),
-                              vp(gH), vp(gC))
-        assert rc == 0
+        Pss, Gss, gs = hostsim.dare(T, Z, H, C, gP, gG)  # raises unless the solve succeeds
+        gT, gZ, gH, gC = (gs[k] for k in ("T", "Z", "H", "C"))
         ref = scipy.linalg.solve_discrete_are(T.T, Z.T, C, H)
         assert rel_err(Pss, ref) < 1e-12
         ts = [torch.tensor(v, requires_grad=True) for v in (T, Z, H, C)]
@@ -181,10 +173,6 @@ def test_predictor_form_steady_state_and_time_varying():
 
 
 def test_rts_smoother_on_host():
-    import ctypes
-
-    lib = hostsim.build()
-    vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
     rng = np.random.default_rng(0)
     from tests.helpers import make_test_inputs
 
@@ -192,11 +180,9 @@ def test_rts_smoother_on_host():
                        (make_test_inputs(1, 5, 2, 10, missing_data=1), 0), (random_system(rng, 6, 3, 3, 30, n_missing=2), 0)):
         o = kn.kalman_filter("standard", *args)
         T, R, Q = (np.ascontiguousarray(args[i]) for i in (3, 5, 7))
-        n, m = o[0].shape[0], T.shape[0]
-        fs, fc = np.ascontiguousarray(o[0][..., 0]), np.ascontiguousarray(o[2])
-        ss, sc = np.zeros_like(fs), np.zeros_like(fc)
-        C = np.ascontiguousarray(R @ Q @ R.T)
-        assert lib.hostsim_smoother(n, m, vp(T), vp(C), vp(fs), vp(fc), vp(ss), vp(sc)) == 0
+        fs = o[0][..., 0]
+        ss, sc = hostsim.smoother(T, R, Q, o[0], o[2])
+        ss = ss[..., 0]
         rs, rc = kn.kalman_smoother(T, R, Q, o[0], o[2])
         assert rel_err(ss, rs[..., 0]) < 1e-10
         # reference tests/test_kalman_filter.py:236-238: the first few smoothed covariances of the P0 = 1e6 fixture are
@@ -394,10 +380,6 @@ def test_device_math_moments_and_smoother_equal_dense_conditional_moments():
     """Full-output device math (filtered / predicted moments) and the device RTS smoother, compiled for the host, against
     the dense conditional moments of the joint Gaussian (oracle.kalman_numpy.dense_gaussian_state_moments) - a known answer
     that shares no recursion with them."""
-    import ctypes
-
-    lib = hostsim.build()
-    vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
     rng = np.random.default_rng(77)
     for (m, p, r), static in (((2, 1, 1), True), ((3, 2, 2), True), ((4, 3, 2), False)):
         n = 10
@@ -410,10 +392,8 @@ def test_device_math_moments_and_smoother_equal_dense_conditional_moments():
         for t in range(n):
             for (got_a, got_P), (a, P) in (((fs[t], fc[t]), cond(t, t)), ((ps[t + 1], pc[t + 1]), cond(t + 1, t))):
                 assert rel_err(got_a, a) < 1e-10 and rel_err(got_P, P) < 1e-10, (m, t)
-        T, R, Q = (np.ascontiguousarray(args[i]) for i in (3, 5, 7))
-        f1, f2 = np.ascontiguousarray(fs[..., 0]), np.ascontiguousarray(fc)
-        ss, sc = np.zeros_like(f1), np.zeros_like(f2)
-        assert lib.hostsim_smoother(n, m, vp(T), vp(np.ascontiguousarray(R @ Q @ R.T)), vp(f1), vp(f2), vp(ss), vp(sc)) == 0
+        ss, sc = hostsim.smoother(args[3], args[5], args[7], fs, fc)
+        ss = ss[..., 0]
         for t in range(n):
             a, P = cond(t, n - 1)
             assert rel_err(ss[t], a[:, 0]) < 1e-10 and rel_err(sc[t], P) < 1e-10, (m, t)

@@ -55,26 +55,25 @@ def test_p1_ctape_block_edges_on_host(m):
 @pytest.mark.parametrize("m", [1, 2, 3, 4])
 def test_p1_ctape_skipping_c_d_keeps_other_cotangents_bitwise_on_host(m):
     """KalmanLogp for BayesianARMA requests a0, P0, T, R, Q only: the reduced sweep then drops c-bar and d-bar (the
-    instantiation with_adjoint_variant picks for the request, built for the host by tests/p1ctape_host).  The cotangents
+    instantiation with_adjoint_variant picks for the request, run on the host by tests/hostsim).  The cotangents
     that are requested are bit-identical to a run that requests everything, and agree with the oracle."""
-    from tests import p1ctape_host
-
     rng = np.random.default_rng(950 + m)
     for n in (2, S + 2, 25):
         y, a0, P0, T, Z, R, H, Q = _arma_like(rng, m, n)
-        C = R @ Q @ R.T
         c, d = rng.normal(size=(m, 1)), rng.normal(size=(1, 1))
         for w in (None, rng.normal(size=n)):
-            ll1, i1, g_all = p1ctape_host.run(y, a0, P0, T, C, c, d, g_ll_obs=w, want_cd=True)
-            ll0, i0, g_some = p1ctape_host.run(y, a0, P0, T, C, c, d, g_ll_obs=w, want_cd=False)
+            kw = dict(c=c, d=d, static_dims=True, full=False, pred=True, p1=True, g_ll_obs=w, z_unit0=True, h_zero=True,
+                      t_companion=True, no_missing=True)
+            o1, g_all, i1 = hostsim.run("standard", y, a0, P0, T, Z, R, H, Q, skip=("Z", "H"), **kw)
+            o0, g_some, i0 = hostsim.run("standard", y, a0, P0, T, Z, R, H, Q, skip=("Z", "H", "c", "d"), **kw)
+            ll0, ll1 = o0[4], o1[4]
             assert i0 == 0 and i1 == 0 and ll0 == ll1
-            assert np.abs(g_all["c"]).max() > 0.0 and set(g_some) == {"a0", "P0", "T", "C"}
-            for k in g_some:
+            assert np.abs(g_all["c"]).max() > 0.0 and not np.any(g_some["c"]) and not np.any(g_some["d"])
+            for k in ("a0", "P0", "T", "R", "Q"):
                 assert np.array_equal(g_some[k], g_all[k]), (k, n)
             _, gt = kt.loglik_and_grads("standard", y, a0, P0, T, Z, R, H, Q, c=c, d=d,
                                         g_ll_obs=None if w is None else 1.0 + w)
-            Cb = g_some["C"]
-            got = {"a0": g_some["a0"], "P0": g_some["P0"], "T": g_some["T"][:, 0], "Q": R.T @ Cb @ R,
+            got = {"a0": g_some["a0"], "P0": g_some["P0"], "T": g_some["T"][:, 0], "Q": g_some["Q"],
                    "c": g_all["c"], "d": g_all["d"]}
             ref = {"a0": np.ravel(gt["a0"]), "P0": gt["P0"], "T": np.asarray(gt["T"])[:, 0], "Q": gt["Q"],
                    "c": np.ravel(gt["c"]), "d": np.ravel(gt["d"])}

@@ -1,6 +1,6 @@
 """CPU checks of the simulation smoother: the numpy restatement (oracle/simsmooth.py) pins itself against dense
 joint-Gaussian algebra through the affine map from normals to paths, the host build of the kernels' KFB_HD code
-(tests/simsmooth_host) equals the restatement, and the C ABI validates its arguments without a device."""
+(tests/hostsim) equals the restatement, and the C ABI validates its arguments without a device."""
 import ctypes
 
 import numpy as np
@@ -159,7 +159,7 @@ def test_oracle_factor_rule():
 @pytest.mark.parametrize("force_dyn", [False, True], ids=["instantiation", "runtime_dims"])
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 def test_host_build_equals_oracle(case, force_dyn):
-    from tests import simsmooth_host as sh
+    from tests import hostsim
 
     name, y, a0, P0, T, Z, R, H, Q, c, d, _ = case
     n, p, m, r = y.shape[0], Z.shape[0], T.shape[0], R.shape[1]
@@ -169,13 +169,13 @@ def test_host_build_equals_oracle(case, force_dyn):
     pc = oss.predicted_covs(y, P0, T, Z, R, H, Q)
     want, info = oss.simulation_smoother(y, a0, P0, T, Z, R, H, Q, c, d, zi, zs, zo, P=pc)
     assert info == 0
-    got, hinfo = sh.run(y[..., 0], mats_of(case), pc[None], S, zi, zs.reshape(-1), zo, force_dyn=force_dyn)
+    got, hinfo = hostsim.simsmooth(y[..., 0], mats_of(case), pc[None], S, zi, zs.reshape(-1), zo, force_dyn=force_dyn)
     assert (hinfo == 0).all()
     assert np.abs(got - want).max() <= 1e-13 * (np.abs(want).max() + 1.0), name
 
 
 def test_host_build_nile():
-    from tests import simsmooth_host as sh
+    from tests import hostsim
 
     y, a0, P0, T, Z, R, H, Q = nile_inputs(n_missing=5)
     rng = np.random.default_rng(2)
@@ -183,14 +183,14 @@ def test_host_build_nile():
     zi, zs, zo = random_normals(rng, S, n, 2, 1, 2)
     pc = oss.predicted_covs(y, P0, T, Z, R, H, Q)
     want, _ = oss.simulation_smoother(y, a0, P0, T, Z, R, H, Q, None, None, zi, zs, zo, P=pc)
-    got, info = sh.run(y[..., 0], dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q), pc[None], S, zi, zs, zo)
+    got, info = hostsim.simsmooth(y[..., 0], dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q), pc[None], S, zi, zs, zo)
     assert (info == 0).all()
     # P0 = 1e6 I: xhat_0 = P0 r_{-1} scales the rounding of r_{-1} (different F^-1 and summation orders) by 1e6
     assert np.abs(got - want).max() <= 1e-8 * np.abs(want).max()
 
 
 def test_host_build_info_codes():
-    from tests import simsmooth_host as sh
+    from tests import hostsim
     from pymc_statespace_b200._lib import KFB_INFO_NOT_PSD
 
     rng = np.random.default_rng(5)
@@ -200,24 +200,24 @@ def test_host_build_info_codes():
     mats = dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q)
     yp = y.copy()
     yp[3, 1] = np.nan  # partly missing row 3
-    got, info = sh.run(yp[..., 0], dict(mats), pc[None], 2, zi, zs, zo)
+    got, info = hostsim.simsmooth(yp[..., 0], dict(mats), pc[None], 2, zi, zs, zo)
     assert info[0] == -4 and np.isnan(got).all()
-    got, info = sh.run(y[..., 0], dict(mats, Q=-Q), pc[None], 2, zi, zs, zo)
+    got, info = hostsim.simsmooth(y[..., 0], dict(mats, Q=-Q), pc[None], 2, zi, zs, zo)
     assert info[0] == KFB_INFO_NOT_PSD and np.isnan(got).all()
     pc_bad = pc.copy()
     pc_bad[2] = -10 * np.eye(2)  # F_2 = Z P_2 Z^T + H not PD
-    got, info = sh.run(y[..., 0], dict(mats), pc_bad[None], 2, zi, zs, zo)
+    got, info = hostsim.simsmooth(y[..., 0], dict(mats), pc_bad[None], 2, zi, zs, zo)
     assert info[0] == 3 and np.isnan(got).all()
 
 
 def test_instantiation_choice():
-    from tests import simsmooth_host as sh
+    from tests import hostsim
 
     for m in range(1, 5):
         for p in range(1, 4):
-            assert sh.is_static(m, p, 1) and sh.is_static(m, p, m)
-    assert not sh.is_static(2, 1, 3) and not sh.is_static(5, 1, 1) and not sh.is_static(13, 1, 3)
-    assert not sh.is_static(2, 4, 1)
+            assert hostsim.simsmooth_is_static(m, p, 1) and hostsim.simsmooth_is_static(m, p, m)
+    assert not hostsim.simsmooth_is_static(2, 1, 3) and not hostsim.simsmooth_is_static(5, 1, 1) and not hostsim.simsmooth_is_static(13, 1, 3)
+    assert not hostsim.simsmooth_is_static(2, 4, 1)
 
 
 # ---------------------------------------------------------------------------------------------------- C ABI

@@ -1,7 +1,7 @@
 """Time-parallel form (KFB_FLAG_TIME_PARALLEL) without a GPU.
 
 * The filtering-element, affine and congruence combination operators of csrc/kf_tpar.cuh, compiled for the host
-  (tests/tpar_host), folded in chunks and scanned in several tree shapes, give the oracle's sequential moments and
+  (tests/hostsim), folded in chunks and scanned in several tree shapes, give the oracle's sequential moments and
   cotangents: m = 1..4, missing rows (first and last included), c / d, time-varying matrices, non-symmetric P0.
 * The plan logic of the C ABI: the flag on a geometry outside the time-parallel form is KFB_ERR_UNSUPPORTED, and
   kfb_workspace_bytes sizes the per-unit tape the forward pass always writes.
@@ -13,7 +13,7 @@ import pytest
 
 from oracle import kalman_numpy as kn
 from oracle import kalman_torch as kt
-from tests import tpar_host
+from tests import hostsim
 from tests.helpers import nile_inputs, random_system, rel_err
 
 TOL = 1e-11
@@ -25,7 +25,7 @@ def _check(kind, args, c=None, d=None, strict=True, w=None, chunks=(1, 3, 8, 64)
     _, gt = kt.loglik_and_grads(kind, *args, c=c, d=d, strict_reference=strict, g_ll_obs=w)
     for nch in chunks:
         for tree in trees:
-            outs, g, info, seq = tpar_host.run(kind, *args, c=c, d=d, strict=strict, nchunks=nch, tree=tree,
+            outs, g, info, seq = hostsim.tpar_run(kind, *args, c=c, d=d, strict=strict, nchunks=nch, tree=tree,
                                                seed=nch * 7 + tree, g_ll_obs=w, g_loglik=(0.0 if w is not None else None))
             assert info == 0 and not seq
             for name, a, b in zip(("fs", "ps", "fc", "pc", "loglik", "ll_obs"), outs, ref):
@@ -90,7 +90,7 @@ def test_undefined_element_takes_the_sequential_walk():
     args = (y, a0, P0, T, Z, R, H, Q)
     ref = kn.kalman_filter("standard", *args)
     _, gt = kt.loglik_and_grads("standard", *args)
-    outs, g, info, seq = tpar_host.run("standard", *args, nchunks=8)
+    outs, g, info, seq = hostsim.tpar_run("standard", *args, nchunks=8)
     assert seq == 1 and info == 0
     for a, b in zip(outs, ref):
         assert rel_err(a, b) < TOL
@@ -114,7 +114,7 @@ def test_expanding_elements_fail_the_check_and_take_the_sequential_walk():
     args = (y, a0.reshape(-1, 1), P0, T, Z, R, H, Q)
     ref = kn.kalman_filter("standard", *args)
     _, gt = kt.loglik_and_grads("standard", *args)
-    outs, g, info, walk = tpar_host.run("standard", *args, nchunks=256)
+    outs, g, info, walk = hostsim.tpar_run("standard", *args, nchunks=256)
     assert walk == 2 and info == 0
     for a, b in zip(outs, ref):
         assert rel_err(a, b) < TOL
@@ -127,7 +127,7 @@ def test_info_when_F0_is_not_positive():
     y, a0, P0, T, Z, R, H, Q = random_system(rng, 2, 1, 1, 20)
     Z = np.array([[1.0, 0.0]])
     P0 = np.diag([0.0, 1.0])
-    _, _, info, _ = tpar_host.run("standard", y, a0, P0, T, Z, R, np.zeros((1, 1)), Q, do_bwd=False)
+    _, _, info, _ = hostsim.tpar_run("standard", y, a0, P0, T, Z, R, np.zeros((1, 1)), Q, do_bwd=False)
     assert info == 1
 
 

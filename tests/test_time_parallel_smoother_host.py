@@ -1,6 +1,6 @@
 """Time-parallel RTS smoother (kfb_smoother_ex with KFB_FLAG_TIME_PARALLEL) without a GPU.
 
-* The fold, suffix scan and checked walk of csrc/kf_tpar_smooth.cuh, compiled for the host (tests/tpar_host), in
+* The fold, suffix scan and checked walk of csrc/kf_tpar_smooth.cuh, compiled for the host (tests/hostsim), in
   several chunk counts and scan-tree shapes, give the oracle's smoothed moments: m = 1..4, missing rows in the filtered
   series, non-symmetric filtered covariances, singular predicted covariances (the pinv branch), the Nile fixture.
 * With a zero drift tolerance the unit falls back to the sequential recursion and reproduces it bit for bit.
@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 from oracle import kalman_numpy as kn
-from tests import tpar_host
+from tests import hostsim
 from tests.helpers import nile_inputs, random_system, rel_err
 
 TOL = 1e-12  # the sequential smoother itself agrees with the oracle (SVD pinv) to ~1e-13
@@ -31,7 +31,7 @@ def _check(T, R, Q, fs, fc, tol=TOL, chunks=CHUNKS, trees=TREES, skip=0):
     rs, rc = kn.kalman_smoother(T, R, Q, fs, fc)
     for nch in chunks:
         for tree in trees:
-            ss, sc, fb = tpar_host.smooth_run(T, R, Q, fs, fc, nchunks=nch, tree=tree, seed=nch * 7 + tree)
+            ss, sc, fb = hostsim.tpar_smooth(T, R, Q, fs, fc, nchunks=nch, tree=tree, seed=nch * 7 + tree)
             assert fb == 0, (nch, tree)
             assert rel_err(ss, rs) < tol, (nch, tree, rel_err(ss, rs))
             assert rel_err(sc[skip:], rc[skip:]) < tol, (nch, tree, rel_err(sc, rc))
@@ -51,11 +51,11 @@ def test_nonsymmetric_filtered_covariances(m):
     rng = np.random.default_rng(3 + m)
     T, R, Q, fs, fc = _filtered(rng, m, 60)
     fc = fc + 1e-3 * rng.normal(size=fc.shape)
-    rs, rc = tpar_host.smooth_sequential(T, R, Q, fs, fc)
+    rs, rc = hostsim.smoother(T, R, Q, fs, fc, static_dims=True)
     assert np.abs(rc - np.swapaxes(rc, -1, -2)).max() > 1e-4
     for nch in CHUNKS:
         for tree in TREES:
-            ss, sc, fb = tpar_host.smooth_run(T, R, Q, fs, fc, nchunks=nch, tree=tree, seed=nch * 7 + tree)
+            ss, sc, fb = hostsim.tpar_smooth(T, R, Q, fs, fc, nchunks=nch, tree=tree, seed=nch * 7 + tree)
             assert fb == 0
             assert rel_err(ss, rs) < TOL and rel_err(sc, rc) < TOL, (nch, tree)
 
@@ -90,13 +90,13 @@ def test_nile_diffuse_start():
 def test_zero_tolerance_falls_back_to_the_sequential_recursion(m):
     rng = np.random.default_rng(70 + m)
     args = _filtered(rng, m, 200, n_missing=10)
-    seq_s, seq_c = tpar_host.smooth_sequential(*args)
-    ss, sc, fb = tpar_host.smooth_run(*args, nchunks=16, tol=0.0)
+    seq_s, seq_c = hostsim.smoother(*args, static_dims=True)
+    ss, sc, fb = hostsim.tpar_smooth(*args, nchunks=16, tol=0.0)
     assert fb == 1 or m == 1  # at k_states 1 the scan may meet the walk in every bit
     np.testing.assert_array_equal(ss, seq_s)
     np.testing.assert_array_equal(sc, seq_c)
     # one chunk: the walk is the sequential recursion itself, so even a zero tolerance passes
-    ss, sc, fb = tpar_host.smooth_run(*args, nchunks=1, tol=0.0)
+    ss, sc, fb = hostsim.tpar_smooth(*args, nchunks=1, tol=0.0)
     assert fb == 0
     np.testing.assert_array_equal(ss, seq_s)
     np.testing.assert_array_equal(sc, seq_c)
@@ -111,7 +111,7 @@ def test_dense_gaussian_smoothed_moments(m):
     out = kn.kalman_filter("standard", y, a0, P0, T, Z, R, H, Q)
     cond = kn.dense_gaussian_state_moments(y, a0, P0, T, Z, R, H, Q)
     for nch, tree in ((1, 1), (4, 1), (14, 2)):
-        ss, sc, fb = tpar_host.smooth_run(T, R, Q, out[0], out[2], nchunks=nch, tree=tree, seed=nch)
+        ss, sc, fb = hostsim.tpar_smooth(T, R, Q, out[0], out[2], nchunks=nch, tree=tree, seed=nch)
         assert fb == 0
         for t in range(n):
             mu, cov = cond(t, n - 1)
