@@ -65,6 +65,7 @@ enum {
 #define KFB_INFO_NOT_STATIONARY 0x40000002 /* set by the host layer (KalmanLogp): stationary P0 requested but the      */
                                            /* Lyapunov doubling did not converge (spectral radius of T >= 1)            */
 #define KFB_INFO_NOT_PSD 0x40000004        /* kfb_simulation_smoother: P0, Q or H is not positive semi-definite         */
+                                           /* (kfb_forecast_paths: the start covariance, Q or H; kfb_impulse_response: Q) */
 
 /* flags */
 #define KFB_FLAG_CORRECTED 1u  /* strict_reference=False: fix SURVEY.md A.2 quirks Q1,Q4,Q5,Q6 */
@@ -259,6 +260,40 @@ kfb_status kfb_simulation_smoother(const kfb_desc *desc, const kfb_inputs *in, c
                                    int64_t sims_per_unit, const double *z_init, const double *z_state,
                                    const double *z_obs, double *states, int32_t *info, void *workspace,
                                    size_t workspace_bytes, void *stream);
+
+/* Forecast paths from the end of the sample (not on the logp/grad path): joint draws of x_n..x_{n+H-1} and
+ * y_n..y_{n+H-1} given y_0..y_{n-1}, sims_per_unit of them per unit.  Same model as kfb_simulation_smoother.  The start
+ * (a, P) of a unit is the state's distribution at the first forecast time: the predicted moments a_n, P_n of a
+ * preceding kfb_forward (standard filter, KFB_FLAG_CORRECTED), copied into start_mean[U, m], start_cov[U, m, m].  (Run
+ * that filter on y extended by H all-NaN rows and its predicted moments n..n+H-1 are the forecast's moments.)
+ * Simulation s = unit * sims_per_unit + k with (a, P) = (start_mean[unit], start_cov[unit]):
+ *   x_0 = a + S_P z_init[s];  for h = 0..H-1:  states[h, s] = x_h,  obs[h, s] = Z x_h + d + S_H z_obs[h, s],
+ *                                              x_{h+1} = T x_h + c + R S_Q z_state[h, s]  (h < H-1)
+ * with S_A the PSD lower factor of kfb_simulation_smoother.  Normals and outputs are time-major: z_init[S, m],
+ * z_state[H-1, S, r] (may be NULL if H = 1), z_obs[H, S, p], states[H, S, m], obs[H, S, p]; either output may be NULL,
+ * not both.  desc gives U = n_draws * n_series, m, p, r and the batch strides of T, Z, R, H, Q, c, d (c, d may be NULL);
+ * desc->n, filter_kind, flags and in->y, a0, P0 are not read.  Every time stride must be 0 and k_states, k_endog,
+ * k_posdef <= 32 (else KFB_ERR_UNSUPPORTED); horizon < 1, sims_per_unit < 1, a null required pointer or both outputs
+ * NULL: KFB_ERR_INVALID_ARG.  info[U] (written, no zeroing needed): 0, or KFB_INFO_NOT_PSD if P, Q or H is not positive
+ * semi-definite or the start has a NaN; a failing unit's paths are NaN.  Workspace
+ * (kfb_forecast_paths_workspace_bytes), each term rounded up to 256 bytes:  8 U (m m + m r + p p + r r)  +  4 U. */
+kfb_status kfb_forecast_paths_workspace_bytes(const kfb_desc *desc, int64_t sims_per_unit, size_t *bytes);
+kfb_status kfb_forecast_paths(const kfb_desc *desc, const kfb_inputs *in, const double *start_mean,
+                              const double *start_cov, int32_t horizon, int64_t sims_per_unit, const double *z_init,
+                              const double *z_state, const double *z_obs, double *states, double *obs, int32_t *info,
+                              void *workspace, size_t workspace_bytes, void *stream);
+
+/* Impulse responses for every draw: column j of horizon h is T^h R S e_j (states[n_draws, H, m, r]) and Z T^h R S e_j
+ * (obs[n_draws, H, p, r]), the response to shock j at time 0.  Either output may be NULL, not both.  desc gives
+ * n_draws, m, p, r and the batch strides of T, Z, R, Q (every time stride 0, sizes <= 32, else KFB_ERR_UNSUPPORTED);
+ * nothing else of desc or in is read.  A bad `shock` or horizon < 1: KFB_ERR_INVALID_ARG.  info[n_draws] (written):
+ * 0, or KFB_INFO_NOT_PSD if Q is not positive semi-definite under KFB_SHOCK_STD / _CHOLESKY; that draw's responses
+ * are NaN. */
+#define KFB_SHOCK_UNIT 0     /* S = I                                        */
+#define KFB_SHOCK_STD 1      /* S = diag(sqrt(diag Q)): one standard deviation */
+#define KFB_SHOCK_CHOLESKY 2 /* S = PSD lower factor of Q: orthogonalised     */
+kfb_status kfb_impulse_response(const kfb_desc *desc, const kfb_inputs *in, int32_t horizon, int32_t shock,
+                                double *states, double *obs, int32_t *info, void *stream);
 
 /* FP64 roofline denominator: `iters` dependent-chain DFMA rounds on every SM.  Returns through
  * h_flops the number of floating-point operations the launch executes (2 per FMA); the caller

@@ -30,6 +30,8 @@ KFB_INFO_DARE_FAILED = 0x40000001
 KFB_INFO_NOT_STATIONARY = 0x40000002
 KFB_INFO_BAD_STRUCTURE = 0x40000003
 KFB_INFO_NOT_PSD = 0x40000004
+KFB_SHOCK_UNIT, KFB_SHOCK_STD, KFB_SHOCK_CHOLESKY = range(3)  # kfb_impulse_response: S = I, diag(sqrt(diag Q)), chol(Q)
+SHOCK_KIND = {"unit": KFB_SHOCK_UNIT, "std": KFB_SHOCK_STD, "cholesky": KFB_SHOCK_CHOLESKY}
 
 KFB_OK, KFB_ERR_INVALID_ARG, KFB_ERR_UNSUPPORTED, KFB_ERR_WORKSPACE, KFB_ERR_CUDA = range(5)
 
@@ -96,6 +98,11 @@ EXPORTS = {
     "kfb_simulation_smoother_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), _c_i64, ctypes.POINTER(ctypes.c_size_t)]),
     "kfb_simulation_smoother": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _c_i64, _vp, _vp, _vp, _vp,
                                          _vp, _vp, ctypes.c_size_t, _vp]),
+    "kfb_forecast_paths_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), _c_i64, ctypes.POINTER(ctypes.c_size_t)]),
+    "kfb_forecast_paths": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _vp, _c_i32, _c_i64, _vp, _vp,
+                                    _vp, _vp, _vp, _vp, _vp, ctypes.c_size_t, _vp]),
+    "kfb_impulse_response": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _c_i32, _c_i32, _vp, _vp, _vp,
+                                      _vp]),
     "kfb_fp64_peak": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),
     "kfb_fp64_peak_distinct": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),
 }

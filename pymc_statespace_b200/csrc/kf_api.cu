@@ -4,6 +4,7 @@
 
 #include "../../include/kfb200.h"
 #include "kf_aux.cuh"
+#include "kf_forecast.cuh"
 #include "kf_kernels.cuh"
 #include "kf_simsmooth.cuh"
 #include "kf_tpar.cuh"
@@ -21,6 +22,8 @@ cudaError_t launch_p1_forward(const KfArgs& A, int y_smem_doubles, int bulk_ok, 
 cudaError_t launch_tpar(const KfArgs& A, bool bwd, cudaStream_t s);
 cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
 cudaError_t launch_simulation_smoother(const ss::Args& A, cudaStream_t s);
+cudaError_t launch_forecast_paths(const fc::Args& A, cudaStream_t s);
+cudaError_t launch_impulse_response(const fc::IrfArgs& A, cudaStream_t s);
 
 // k_states with launchers of their own, one object per size (kf_thread.cu: thread-per-unit filters and smoother;
 // kf_coopT.cu: compile-time-dims kernels; the tensor-core DARE in kf_coopT.cu from k_states 10).  The Makefile repeats
@@ -214,6 +217,37 @@ static kfb_status make_ss_plan(const kfb_desc* d, int64_t sims_per_unit, SsPlan*
   pl->off_fac = take((size_t)U * ss::fac_stride(d->m, d->p, d->r) * 8);
   pl->off_u = take((size_t)d->n * lanes * d->p * 8);
   pl->off_r = take((size_t)(d->n - 1) * lanes * d->m * 8);
+  pl->off_stat = take((size_t)U * 4);
+  pl->total = off;
+  return KFB_OK;
+}
+
+// Sizes and strides of kfb_forecast_paths / kfb_impulse_response: static matrices, dims up to ss::SS_MAX (desc->n,
+// filter_kind and flags are not read).
+static kfb_status check_forecast_desc(const kfb_desc* d) {
+  if (!d || d->n_draws <= 0 || d->n_series <= 0 || d->m <= 0 || d->p <= 0 || d->r <= 0) return KFB_ERR_INVALID_ARG;
+  if (d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts) return KFB_ERR_UNSUPPORTED;
+  if (d->m > ss::SS_MAX || d->p > ss::SS_MAX || d->r > ss::SS_MAX) return KFB_ERR_UNSUPPORTED;
+  return KFB_OK;
+}
+
+static_assert(fc::SHOCK_UNIT == KFB_SHOCK_UNIT && fc::SHOCK_STD == KFB_SHOCK_STD &&
+                  fc::SHOCK_CHOLESKY == KFB_SHOCK_CHOLESKY && ss::INFO_NOT_PSD == KFB_INFO_NOT_PSD,
+              "kf_forecast.cuh / kf_simsmooth.cuh constants differ from include/kfb200.h");
+
+// Workspace of kfb_forecast_paths: per-unit factors and status, each region rounded up to 256 bytes (kfb200.h).
+struct FcPlan {
+  size_t off_fac, off_stat, total;
+};
+
+static kfb_status make_fc_plan(const kfb_desc* d, int64_t sims_per_unit, FcPlan* pl) {
+  kfb_status st = check_forecast_desc(d);
+  if (st != KFB_OK) return st;
+  if (sims_per_unit <= 0) return KFB_ERR_INVALID_ARG;
+  const long long U = d->n_draws * d->n_series;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+  pl->off_fac = take((size_t)U * fc::fac_stride(d->m, d->p, d->r) * 8);
   pl->off_stat = take((size_t)U * 4);
   pl->total = off;
   return KFB_OK;
@@ -504,6 +538,59 @@ kfb_status kfb_simulation_smoother(const kfb_desc* desc, const kfb_inputs* in, c
   cudaError_t e = cudaMemsetAsync(A.ustat, 0x7f, (size_t)A.U * 4, s);  // every word = ss::KEY_NONE
   if (e != cudaSuccess) return cuda_fail(e);
   e = launch_simulation_smoother(A, s);
+  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
+  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
+kfb_status kfb_forecast_paths_workspace_bytes(const kfb_desc* desc, int64_t sims_per_unit, size_t* bytes) {
+  if (!bytes) return KFB_ERR_INVALID_ARG;
+  FcPlan pl;
+  kfb_status st = make_fc_plan(desc, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  *bytes = pl.total;
+  return KFB_OK;
+}
+
+kfb_status kfb_forecast_paths(const kfb_desc* desc, const kfb_inputs* in, const double* start_mean,
+                              const double* start_cov, int32_t horizon, int64_t sims_per_unit, const double* z_init,
+                              const double* z_state, const double* z_obs, double* states, double* obs, int32_t* info,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  FcPlan pl;
+  kfb_status st = make_fc_plan(desc, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  if (horizon < 1 || !in || !in->T || !in->Z || !in->R || !in->H || !in->Q || !start_mean || !start_cov || !z_init ||
+      (horizon > 1 && !z_state) || !z_obs || (!states && !obs) || !info)
+    return KFB_ERR_INVALID_ARG;
+  if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
+  char* ws = (char*)workspace;
+  fc::Args A;
+  std::memset(&A, 0, sizeof(A));
+  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
+  A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r;
+  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
+  A.Hm = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
+  A.mean = start_mean; A.cov = start_cov; A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs;
+  A.states = states; A.obs = obs; A.info = info;
+  A.vec = (uintptr_t)states % 16 == 0 && (uintptr_t)obs % 16 == 0;
+  A.fac = (double*)(ws + pl.off_fac); A.ustat = (int*)(ws + pl.off_stat);
+  const cudaError_t e = launch_forecast_paths(A, (cudaStream_t)stream);
+  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
+  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
+kfb_status kfb_impulse_response(const kfb_desc* desc, const kfb_inputs* in, int32_t horizon, int32_t shock,
+                                double* states, double* obs, int32_t* info, void* stream) {
+  kfb_status st = check_forecast_desc(desc);
+  if (st != KFB_OK) return st;
+  if (horizon < 1 || shock < KFB_SHOCK_UNIT || shock > KFB_SHOCK_CHOLESKY || !in || !in->T || !in->Z || !in->R ||
+      !in->Q || (!states && !obs) || !info)
+    return KFB_ERR_INVALID_ARG;
+  fc::IrfArgs A;
+  std::memset(&A, 0, sizeof(A));
+  A.nD = desc->n_draws; A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r; A.shock = shock;
+  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0};
+  A.states = states; A.obs = obs; A.info = info;
+  const cudaError_t e = launch_impulse_response(A, (cudaStream_t)stream);
   if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
 }

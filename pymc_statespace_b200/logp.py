@@ -327,6 +327,68 @@ class KalmanLogp:
         self._ss_info = info
         return states[..., :m0].contiguous() if m != m0 else states
 
+    def forecast(self, theta, horizon: int, n_simulations: int = 0, generator: Optional[torch.Generator] = None,
+                 z_init=None, z_state=None, z_obs=None) -> Dict[str, torch.Tensor]:
+        """Forecasts from the end of the sample for every draw: ``simulation.forecast`` after the theta scatter (and
+        stationary P0), as ``sample_states`` does.  Returns its dict (state_mean [B, H, k_states], state_cov, obs_mean,
+        obs_cov and, with n_simulations > 0, state_paths [B * n_simulations, H, k_states] and obs_paths, draw-major)
+        plus "info" [B] (int32): KFB_INFO_NOT_STATIONARY for a draw whose stationary P0 does not exist (it replaces the
+        forward's follow-on code, as in ``sample_states``), else the forward's code (t+1: F_t not positive definite;
+        -(t+1): y_t partly missing), else the paths' code (KFB_INFO_NOT_PSD: P_n, Q or H not positive semi-definite).
+        Every output of a failing draw is NaN.
+
+        Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
+        built with.  Normals may be given as in ``simulation.forecast``, sized for the model's own k_states."""
+        from .simulation import _forecast
+
+        H = int(horizon)
+        if H < 1:
+            raise ValueError("horizon must be >= 1")
+        mats = self._scatter(self._check_theta(theta))
+        sp = self.spec
+        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
+        kal = getattr(self, "_fc_kalman", None)
+        if kal is None or kal.n != self.n + H:
+            self._fc_kalman = kal = BatchedKalman("standard", self.n + H, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
+                                                  strict_reference=False, device=self.device)
+        if S > 0 and m != m0:  # padded model: the extra states are identically zero, their normals unused
+            if z_init is None:
+                z_init = torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator)
+            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
+        res, info, pinfo = _forecast(kal, self.y, mats, H, int(n_simulations), z_init, z_state, z_obs, generator)
+        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
+            info = torch.where(self._lyap[2] != 0, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
+        if pinfo is not None:
+            info = torch.where(info == 0, pinfo, info)
+        bad = info != 0
+        for k, v in res.items():
+            if k.endswith("_paths"):  # [S, H, .] views of the time-major buffers, draw-major
+                v.unflatten(0, (self.B, -1))[bad] = float("nan")
+            else:
+                v[bad] = float("nan")
+        if m != m0:
+            for k in ("state_mean", "state_paths"):
+                if k in res:
+                    res[k] = res[k][..., :m0]
+            res["state_cov"] = res["state_cov"][..., :m0, :m0]
+        res["info"] = info
+        return res
+
+    def impulse_responses(self, theta, horizon: int, shock: str = "cholesky") -> Dict[str, torch.Tensor]:
+        """``simulation.impulse_responses`` for every draw after the theta scatter: {"states" [B, H, k_states, k_posdef],
+        "obs" [B, H, k_endog, k_posdef], "info" [B]} (info KFB_INFO_NOT_PSD and NaN responses where Q is not positive
+        semi-definite under shock "std" / "cholesky")."""
+        from .simulation import _impulse_responses
+
+        mats = self._scatter(self._check_theta(theta))
+        states, obs, info = _impulse_responses(mats["T"], mats["Z"], mats["R"], mats["Q"], horizon, shock)
+        if states.shape[0] != self.B:  # every matrix shared by the draws
+            states, obs, info = (t.expand((self.B,) + t.shape[1:]).contiguous() for t in (states, obs, info))
+        m0 = self.k_states_model
+        if m0 != self.spec.k_states:
+            states = states[:, :, :m0]
+        return {"states": states, "obs": obs, "info": info}
+
     @property
     def sample_states_info(self) -> torch.Tensor:
         """Per-draw status of the last ``sample_states`` (int32, 0 = ok; t+1: F_t not positive definite; -(t+1): y_t

@@ -3,7 +3,9 @@
 Mirrors reference ``pymc_statespace/utils/simulation.py`` (numba): ``simulate_statespace`` (:29-62),
 ``unconditional_simulations`` (:65-79) and ``conditional_simulation`` (:17-26).  ``simulation_smoother`` goes beyond the
 reference: joint draws of the whole state path from p(x_0..x_{n-1} | y, theta) (Durbin & Koopman 2002), where
-``conditional_simulation`` draws every time step on its own from the smoothed marginal.  The reference draws its normals from
+``conditional_simulation`` draws every time step on its own from the smoothed marginal.  ``forecast`` gives the
+forecast moments and joint draws of the paths after the end of the sample, and ``impulse_responses`` the responses of
+states and observations to one shock.  The reference draws its normals from
 NumPy's global RNG inside numba, so its trajectories are not reproducible from outside; here the standard-normal draws
 come from ``torch.randn`` on the device (or are passed in, which makes the result exactly checkable) and the CUDA kernels
 are deterministic transforms of them.
@@ -16,7 +18,7 @@ import ctypes
 
 import torch
 
-from ._lib import check, load
+from ._lib import SHOCK_KIND, KfbInputs, check, load
 from .engine import BatchedKalman, _ptr, _stream_ptr
 
 
@@ -145,3 +147,145 @@ def simulation_smoother(y, a0, P0, T, Z, R, H, Q, c=None, d=None, n_simulations:
         u = int(bad[0, 0])
         raise RuntimeError(f"simulation_smoother: unit {u} failed with info {int(info[u])} (codes in include/kfb200.h)")
     return states
+
+
+def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_state, z_obs, generator):
+    """Forecast moments (and paths if n_simulations > 0) on ``kalman``'s geometry: the standard corrected filter of
+    length n + horizon, run on y extended by ``horizon`` all-NaN rows.  Returns (result dict, forward info [U], paths
+    info [U] or None) without raising on a non-zero info."""
+    lib = load()
+    dev = kalman.device
+    H, m, p, r, U = int(horizon), kalman.m, kalman.p, kalman.r, kalman.units
+    n = kalman.n - H
+    f64 = dict(dtype=torch.float64, device=dev)
+    yx = torch.cat([y, torch.full(y.shape[:-2] + (H, p), float("nan"), **f64)], dim=-2)
+    out = kalman.forward(yx, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
+                         outputs=("predicted_states", "predicted_covs"))
+    a, P = out["predicted_states"][:, n:n + H], out["predicted_covs"][:, n:n + H]
+    ns = kalman.n_series
+
+    def per_unit(t, base_ndim):  # [..] shared or [B, ..] per draw -> broadcastable against [U, H, ..]
+        t = t if t.ndim == base_ndim else t.repeat_interleave(ns, dim=0)[:, None]
+        return t
+
+    Zu, Hu = per_unit(mats["Z"], 2), per_unit(mats["H"], 2)
+    ya = torch.matmul(Zu, a[..., None])[..., 0]
+    if mats.get("d") is not None:
+        ya = ya + per_unit(mats["d"], 1)
+    res = {"state_mean": a, "state_cov": P, "obs_mean": ya,
+           "obs_cov": torch.matmul(torch.matmul(Zu, P), Zu.transpose(-1, -2)) + Hu}
+    if n_simulations <= 0:
+        return res, out["info"], None
+    S = U * n_simulations
+    z_init = torch.randn((S, m), generator=generator, **f64) if z_init is None else z_init
+    z_state = torch.randn((H - 1, S, r), generator=generator, **f64) if z_state is None else z_state
+    z_obs = torch.randn((H, S, p), generator=generator, **f64) if z_obs is None else z_obs
+    for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (H - 1, S, r)), ("z_obs", z_obs, (H, S, p))):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
+            raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
+    z_init, z_state, z_obs = z_init.contiguous(), z_state.contiguous(), z_obs.contiguous()
+    start_mean, start_cov = a[:, 0].contiguous(), P[:, 0].contiguous()
+    desc = kalman._desc
+    nbytes = ctypes.c_size_t(0)
+    check(lib.kfb_forecast_paths_workspace_bytes(ctypes.byref(desc), n_simulations, ctypes.byref(nbytes)),
+          "kfb_forecast_paths_workspace_bytes")
+    ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
+    states = torch.empty((H, S, m), **f64)
+    obs = torch.empty((H, S, p), **f64)
+    info = torch.empty(U, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.kfb_forecast_paths(ctypes.byref(desc), ctypes.byref(kalman._inputs), _ptr(start_mean), _ptr(start_cov),
+                                     H, n_simulations, _ptr(z_init), _ptr(z_state) if H > 1 else None, _ptr(z_obs),
+                                     _ptr(states), _ptr(obs), _ptr(info), _ptr(ws), ws.numel(), _stream_ptr(dev)),
+              "kfb_forecast_paths")
+    res["state_paths"], res["obs_paths"] = states.permute(1, 0, 2), obs.permute(1, 0, 2)
+    return res, out["info"], info
+
+
+def _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y):
+    mats = {"a0": a0, "P0": P0, "T": T, "Z": Z, "R": R, "H": H, "Q": Q, "c": c, "d": d}
+    for k, t in mats.items():
+        if t is not None and k in ("a0", "c", "d") and t.ndim >= 2 and t.shape[-1] == 1:
+            mats[k] = t = t[..., 0]
+        if t is not None and t.ndim > _BASE_NDIM[k] + 1:
+            raise NotImplementedError("time-varying matrices are not supported")
+    if y is not None and y.ndim == 3 and y.shape[-1] == 1 and y.shape[-2] == Z.shape[-2]:
+        y = y[..., 0]  # reference layout [n, p, 1]
+    B = max([t.shape[0] for k, t in mats.items() if t is not None and t.ndim == _BASE_NDIM[k] + 1] + [1])
+    return mats, y, B
+
+
+def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simulations: int = 0, z_init=None,
+             z_state=None, z_obs=None, generator: Optional[torch.Generator] = None):
+    """Forecasts from the end of the sample: the distribution of x_n..x_{n+H-1} and y_n..y_{n+H-1} given y_0..y_{n-1}
+    (H = ``horizon``; output index h is time n + h), and with ``n_simulations`` > 0 joint draws of those paths.
+
+    Arguments and conventions as in ``simulation_smoother``: float64 CUDA tensors, each matrix shared or one per draw,
+    y [n, p] or [n_series, n, p], draw-major units (u = draw * n_series + series) and simulations
+    (s = u * n_simulations + k).  The moments are the predicted moments of the exact (corrected standard) filter run
+    on y extended by H all-NaN rows.  Each path starts from x_n ~ N(a_n, P_n) and follows the model with its own state
+    and observation noise (include/kfb200.h, kfb_forecast_paths), so the paths have the joint law of the future,
+    cross-horizon covariances included.  Normals may be given, time-major: z_init [S, m], z_state [H-1, S, r],
+    z_obs [H, S, p] for S = U * n_simulations; otherwise they are drawn with ``torch.randn``.
+
+    Returns a dict: state_mean [U, H, m], state_cov [U, H, m, m], obs_mean [U, H, p], obs_cov [U, H, p, p], and with
+    n_simulations > 0 state_paths [S, H, m] and obs_paths [S, H, p].  The paths are ``permute(1, 0, 2)`` views of the
+    kernel's time-major [H, S, .] buffers (no copy): call ``.contiguous()`` for path-major storage.  Raises
+    RuntimeError if some unit fails (F_t not positive definite, a partly missing row, P_n / Q / H not positive
+    semi-definite) and NotImplementedError for time-varying matrices."""
+    mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
+    n_series = 1 if y.ndim == 2 else y.shape[0]
+    m, p, r = T.shape[-1], Z.shape[-2], R.shape[-1]
+    if int(horizon) < 1:
+        raise ValueError("horizon must be >= 1")
+    kalman = BatchedKalman("standard", y.shape[-2] + int(horizon), m, p, r, n_draws=B, n_series=n_series,
+                           strict_reference=False, device=T.device)
+    res, finfo, pinfo = _forecast(kalman, y, mats, int(horizon), int(n_simulations), z_init, z_state, z_obs, generator)
+    for info in (finfo, pinfo):
+        bad = torch.nonzero(info != 0) if info is not None else None
+        if bad is not None and bad.numel():
+            u = int(bad[0, 0])
+            raise RuntimeError(f"forecast: unit {u} failed with info {int(info[u])} (codes in include/kfb200.h)")
+    return res
+
+
+def _impulse_responses(T, Z, R, Q, horizon, shock):
+    """kfb_impulse_response for shared or per-draw T, Z, R, Q.  Returns (states [B, H, m, r], obs [B, H, p, r],
+    info [B]) without raising on a non-zero info."""
+    if shock not in SHOCK_KIND:
+        raise ValueError(f"shock must be one of {sorted(SHOCK_KIND)}")
+    if int(horizon) < 1:
+        raise ValueError("horizon must be >= 1")
+    lib = load()
+    dev = T.device
+    mats, _, B = _canon_matrices(T, Z, R, None, Q, None, None, None, None, None)
+    m, p, r = T.shape[-1], Z.shape[-2], R.shape[-1]
+    kal = BatchedKalman("standard", 1, m, p, r, n_draws=B, device=dev)
+    held, strides = {}, {}
+    for k in ("T", "Z", "R", "Q"):
+        held[k], bs, _ = kal._canon(k, mats[k])
+        strides[k] = (bs, 0)
+    desc = kal._make_desc(strides)
+    ins = KfbInputs(*[_ptr(held.get(k)) for k in ("y", "a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")])
+    H = int(horizon)
+    states = torch.empty((B, H, m, r), dtype=torch.float64, device=dev)
+    obs = torch.empty((B, H, p, r), dtype=torch.float64, device=dev)
+    info = torch.empty(B, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.kfb_impulse_response(ctypes.byref(desc), ctypes.byref(ins), H, SHOCK_KIND[shock], _ptr(states),
+                                       _ptr(obs), _ptr(info), _stream_ptr(dev)), "kfb_impulse_response")
+    return states, obs, info
+
+
+def impulse_responses(T, Z, R, Q, horizon: int, shock: str = "cholesky"):
+    """Responses to one shock at time 0, for every draw: column j of horizon h is T^h R S e_j (states) and
+    Z T^h R S e_j (observations), with S = I (``shock="unit"``), diag(sqrt(diag Q)) (``"std"``: one standard
+    deviation) or the lower factor of Q (``"cholesky"``: orthogonalised).  Float64 CUDA tensors, shared or with a
+    leading draw axis B (B = 1 if all are shared).  Returns (states [B, H, m, r], obs [B, H, p, r]).  Raises
+    RuntimeError if Q is not positive semi-definite for some draw under "std" / "cholesky"."""
+    states, obs, info = _impulse_responses(T, Z, R, Q, horizon, shock)
+    bad = torch.nonzero(info != 0)
+    if bad.numel():
+        b = int(bad[0, 0])
+        raise RuntimeError(f"impulse_responses: draw {b} failed with info {int(info[b])} (Q not positive semi-definite)")
+    return states, obs
