@@ -283,6 +283,43 @@ kfb_status kfb_forecast_paths(const kfb_desc *desc, const kfb_inputs *in, const 
                               const double *z_state, const double *z_obs, double *states, double *obs, int32_t *info,
                               void *workspace, size_t workspace_bytes, void *stream);
 
+/* Conditional forecasts from the end of the sample (not on the logp/grad path): the law of x_n..x_{n+H-1} and
+ * y_n..y_{n+H-1} given y_0..y_{n-1} AND the known future values cond[h, i] = y_{n+h, i} (NaN = free), and joint draws
+ * of those paths (Banbura, Giannone & Lenza 2015: the simulation smoother over the window, with partly observed rows).
+ * Same model and start as kfb_forecast_paths: (a, P) = (start_mean[u], start_cov[u]) are a_n, P_n of a preceding
+ * kfb_forward (standard filter, KFB_FLAG_CORRECTED) over the n observations.  cond is [H, p] shared by every unit
+ * (cond_bs = 0) or [U, H, p] (cond_bs = H p).  Per unit, with o / u the conditioned / free entries of step h and every
+ * product in the masked p x p form:
+ *   window filter  F = Z_o P Z_o^T + H_oo, K = T P Z^T F^-1, v = cond - Z a - d (0 on free entries), u_h = F^-1 v,
+ *                  a <- T a + c + K v, P <- T P L^T + R Q R^T (L = T - K Z);
+ *   smoother       r_{h-1} = Z^T (u_h - K^T r_h) + T^T r_h, N_{h-1} = Z^T F^-1 Z + L^T N_h L  (r = N = 0 after H-1);
+ *   state_mean[u, h] = a_h + P_h r_{h-1}, state_cov[u, h] = P_h - P_h N_{h-1} P_h;
+ *   G = H_uo H_oo^- (generalised inverse by the PSD factor's zero-pivot rule; 0 for a diagonal H), D = Z_u - G Z_o;
+ *   obs_mean[u, h] = cond on conditioned entries, D x^ + d_u + G (cond_o - d_o) on free ones; obs_cov[u, h] =
+ *   D V D^T + H_uu - G H_ou on the free block, 0 on every row and column of a conditioned entry.
+ * Paths (sims_per_unit > 0; simulation s = unit * sims_per_unit + k): Durbin & Koopman's mean correction over the
+ * window from x+_0 = a + S_P z_init[s] with the normals of kfb_forecast_paths (time-major z_init[S, m],
+ * z_state[H-1, S, r] (may be NULL if H = 1), z_obs[H, S, p]); states[h, s] = x~_h, obs[h, s] = cond on conditioned
+ * entries and Z_u x~ + d_u + eps+_u + G (cond_o - Z_o x~ - d_o - eps+_o) on free ones (eps+_h = S_H z_obs[h, s]).
+ * With no condition these are kfb_forecast_paths' paths on the same normals.  sims_per_unit = 0: moments only (no
+ * normal or path pointer is read).  Any moment output [U, H, m], [U, H, m, m], [U, H, p], [U, H, p, p] may be NULL; with
+ * paths, states[H, S, m] or obs[H, S, p] may be NULL, not both.  desc as in kfb_forecast_paths, plus desc->n >= 0 (the
+ * number of observations, used for info codes only).  info[U] (written): 0; n + h + 1 if F_o is not positive definite
+ * at window step h (the numbering of a filter over n + H steps; e.g. a condition the model already determines without
+ * noise); KFB_INFO_NOT_PSD if P, Q or H is not positive semi-definite or the start has a NaN.  Every output of a failing
+ * unit is NaN.  Workspace (kfb_conditional_forecast_workspace_bytes), each term rounded up to 256 bytes, with
+ * U = n_draws * n_series and S32 = U * sims_per_unit rounded up to a multiple of 32:
+ *   8 U H (m p + 2 p p + p + m + m m)  +  8 U (2 m m + m r + p p + r r)  +  8 U (3 m m + 2 m p + 4 p p)  +  4 U
+ *   +  8 H S32 p  +  8 (H - 1) S32 m. */
+kfb_status kfb_conditional_forecast_workspace_bytes(const kfb_desc *desc, int32_t horizon, int64_t sims_per_unit,
+                                                    size_t *bytes);
+kfb_status kfb_conditional_forecast(const kfb_desc *desc, const kfb_inputs *in, const double *start_mean,
+                                    const double *start_cov, int32_t horizon, const double *cond, int64_t cond_bs,
+                                    int64_t sims_per_unit, const double *z_init, const double *z_state,
+                                    const double *z_obs, double *state_mean, double *state_cov, double *obs_mean,
+                                    double *obs_cov, double *states, double *obs, int32_t *info, void *workspace,
+                                    size_t workspace_bytes, void *stream);
+
 /* Impulse responses for every draw: column j of horizon h is T^h R S e_j (states[n_draws, H, m, r]) and Z T^h R S e_j
  * (obs[n_draws, H, p, r]), the response to shock j at time 0.  Either output may be NULL, not both.  desc gives
  * n_draws, m, p, r and the batch strides of T, Z, R, Q (every time stride 0, sizes <= 32, else KFB_ERR_UNSUPPORTED);

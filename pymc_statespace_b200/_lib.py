@@ -101,6 +101,11 @@ EXPORTS = {
     "kfb_forecast_paths_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), _c_i64, ctypes.POINTER(ctypes.c_size_t)]),
     "kfb_forecast_paths": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _vp, _c_i32, _c_i64, _vp, _vp,
                                     _vp, _vp, _vp, _vp, _vp, ctypes.c_size_t, _vp]),
+    "kfb_conditional_forecast_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), _c_i32, _c_i64,
+                                                          ctypes.POINTER(ctypes.c_size_t)]),
+    "kfb_conditional_forecast": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _vp, _c_i32, _vp, _c_i64,
+                                          _c_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_size_t,
+                                          _vp]),
     "kfb_impulse_response": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _c_i32, _c_i32, _vp, _vp, _vp,
                                       _vp]),
     "kfb_fp64_peak": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),

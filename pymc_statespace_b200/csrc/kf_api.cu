@@ -4,6 +4,7 @@
 
 #include "../../include/kfb200.h"
 #include "kf_aux.cuh"
+#include "kf_condfc.cuh"
 #include "kf_forecast.cuh"
 #include "kf_kernels.cuh"
 #include "kf_simsmooth.cuh"
@@ -24,6 +25,7 @@ cudaError_t launch_tpar_smoother(const SmoothArgs& S, cudaStream_t s);
 cudaError_t launch_simulation_smoother(const ss::Args& A, cudaStream_t s);
 cudaError_t launch_forecast_paths(const fc::Args& A, cudaStream_t s);
 cudaError_t launch_impulse_response(const fc::IrfArgs& A, cudaStream_t s);
+cudaError_t launch_conditional_forecast(const cf::Args& A, cudaStream_t s);
 
 // k_states with launchers of their own, one object per size (kf_thread.cu: thread-per-unit filters and smoother;
 // kf_coopT.cu: compile-time-dims kernels; the tensor-core DARE in kf_coopT.cu from k_states 10).  The Makefile repeats
@@ -249,6 +251,31 @@ static kfb_status make_fc_plan(const kfb_desc* d, int64_t sims_per_unit, FcPlan*
   auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
   pl->off_fac = take((size_t)U * fc::fac_stride(d->m, d->p, d->r) * 8);
   pl->off_stat = take((size_t)U * 4);
+  pl->total = off;
+  return KFB_OK;
+}
+
+// Workspace of kfb_conditional_forecast: window tape, per-unit factors, run-time-dims scratch, per-unit status and the
+// u and r scratch of the paths, each region rounded up to 256 bytes (kfb200.h).
+struct CfPlan {
+  size_t off_tape, off_fac, off_wscr, off_stat, off_u, off_r, total;
+};
+
+static kfb_status make_cf_plan(const kfb_desc* d, int32_t horizon, int64_t sims_per_unit, CfPlan* pl) {
+  kfb_status st = check_forecast_desc(d);
+  if (st != KFB_OK) return st;
+  if (horizon < 1 || sims_per_unit < 0 || d->n < 0) return KFB_ERR_INVALID_ARG;
+  if (d->n >= (1 << 29) || horizon >= (1 << 29)) return KFB_ERR_UNSUPPORTED;
+  const long long U = d->n_draws * d->n_series;
+  const long long lanes = ss::warps_of(U * sims_per_unit) * 32;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+  pl->off_tape = take((size_t)U * horizon * cf::tape_stride(d->m, d->p) * 8);
+  pl->off_fac = take((size_t)U * ss::fac_stride(d->m, d->p, d->r) * 8);
+  pl->off_wscr = take((size_t)U * cf::wscr_stride(d->m, d->p) * 8);
+  pl->off_stat = take((size_t)U * 4);
+  pl->off_u = take((size_t)horizon * lanes * d->p * 8);
+  pl->off_r = take((size_t)(horizon - 1) * lanes * d->m * 8);
   pl->total = off;
   return KFB_OK;
 }
@@ -574,6 +601,50 @@ kfb_status kfb_forecast_paths(const kfb_desc* desc, const kfb_inputs* in, const 
   A.vec = (uintptr_t)states % 16 == 0 && (uintptr_t)obs % 16 == 0;
   A.fac = (double*)(ws + pl.off_fac); A.ustat = (int*)(ws + pl.off_stat);
   const cudaError_t e = launch_forecast_paths(A, (cudaStream_t)stream);
+  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
+  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
+kfb_status kfb_conditional_forecast_workspace_bytes(const kfb_desc* desc, int32_t horizon, int64_t sims_per_unit,
+                                                    size_t* bytes) {
+  if (!bytes) return KFB_ERR_INVALID_ARG;
+  CfPlan pl;
+  kfb_status st = make_cf_plan(desc, horizon, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  *bytes = pl.total;
+  return KFB_OK;
+}
+
+kfb_status kfb_conditional_forecast(const kfb_desc* desc, const kfb_inputs* in, const double* start_mean,
+                                    const double* start_cov, int32_t horizon, const double* cond, int64_t cond_bs,
+                                    int64_t sims_per_unit, const double* z_init, const double* z_state,
+                                    const double* z_obs, double* state_mean, double* state_cov, double* obs_mean,
+                                    double* obs_cov, double* states, double* obs, int32_t* info, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  CfPlan pl;
+  kfb_status st = make_cf_plan(desc, horizon, sims_per_unit, &pl);
+  if (st != KFB_OK) return st;
+  const bool paths = sims_per_unit > 0;
+  if (!in || !in->T || !in->Z || !in->R || !in->H || !in->Q || !start_mean || !start_cov || !cond || cond_bs < 0 ||
+      !info || (paths && (!z_init || (horizon > 1 && !z_state) || !z_obs || (!states && !obs))))
+    return KFB_ERR_INVALID_ARG;
+  if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
+  char* ws = (char*)workspace;
+  cf::Args A;
+  std::memset(&A, 0, sizeof(A));
+  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
+  A.n = desc->n; A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r;
+  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
+  A.Hm = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
+  A.mean = start_mean; A.cov = start_cov; A.cond = cond; A.cond_bs = cond_bs;
+  A.state_mean = state_mean; A.state_cov = state_cov; A.obs_mean = obs_mean; A.obs_cov = obs_cov; A.info = info;
+  if (paths) {
+    A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs; A.states = states; A.obs = obs;
+    A.vec = (uintptr_t)states % 16 == 0 && (uintptr_t)obs % 16 == 0;
+  }
+  A.tape = (double*)(ws + pl.off_tape); A.fac = (double*)(ws + pl.off_fac); A.wscr = (double*)(ws + pl.off_wscr);
+  A.ustat = (int*)(ws + pl.off_stat); A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r);
+  const cudaError_t e = launch_conditional_forecast(A, (cudaStream_t)stream);
   if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
 }

@@ -374,6 +374,49 @@ class KalmanLogp:
         res["info"] = info
         return res
 
+    def conditional_forecast(self, theta, conditions, n_simulations: int = 0,
+                             generator: Optional[torch.Generator] = None, z_init=None, z_state=None,
+                             z_obs=None) -> Dict[str, torch.Tensor]:
+        """Conditional forecasts for every draw: ``simulation.conditional_forecast`` after the theta scatter (and
+        stationary P0), as ``forecast`` does.  conditions [H, k_endog] shared by every draw or [B, H, k_endog] (NaN =
+        free).  Returns ``forecast``'s dict plus "info" [B] (int32): KFB_INFO_NOT_STATIONARY for a draw whose stationary
+        P0 does not exist, else the forward's code, else the window / paths code (n + h + 1: F_o not positive definite
+        at window step h; KFB_INFO_NOT_PSD).  Every output of a failing draw is NaN.
+
+        Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
+        built with.  Normals may be given as in ``simulation.conditional_forecast``, sized for the model's own
+        k_states."""
+        from .simulation import _conditional_forecast
+
+        mats = self._scatter(self._check_theta(theta))
+        sp = self.spec
+        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
+        if getattr(self, "_ss_kalman", None) is None:
+            self._ss_kalman = BatchedKalman("standard", self.n, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
+                                            strict_reference=False, device=self.device)
+        if S > 0 and m != m0:  # padded model: the extra states are identically zero, their normals unused
+            if z_init is None:
+                z_init = torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator)
+            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
+        res, info, winfo = _conditional_forecast(self._ss_kalman, self.y, mats, conditions, int(n_simulations), z_init,
+                                                 z_state, z_obs, generator)
+        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
+            info = torch.where(self._lyap[2] != 0, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
+        info = torch.where(info == 0, winfo, info)
+        bad = info != 0
+        for k, v in res.items():
+            if k.endswith("_paths"):  # [S, H, .] views of the time-major buffers, draw-major
+                v.unflatten(0, (self.B, -1))[bad] = float("nan")
+            else:
+                v[bad] = float("nan")
+        if m != m0:
+            for k in ("state_mean", "state_paths"):
+                if k in res:
+                    res[k] = res[k][..., :m0]
+            res["state_cov"] = res["state_cov"][..., :m0, :m0]
+        res["info"] = info
+        return res
+
     def impulse_responses(self, theta, horizon: int, shock: str = "cholesky") -> Dict[str, torch.Tensor]:
         """``simulation.impulse_responses`` for every draw after the theta scatter: {"states" [B, H, k_states, k_posdef],
         "obs" [B, H, k_endog, k_posdef], "info" [B]} (info KFB_INFO_NOT_PSD and NaN responses where Q is not positive

@@ -4,11 +4,11 @@ Mirrors reference ``pymc_statespace/utils/simulation.py`` (numba): ``simulate_st
 ``unconditional_simulations`` (:65-79) and ``conditional_simulation`` (:17-26).  ``simulation_smoother`` goes beyond the
 reference: joint draws of the whole state path from p(x_0..x_{n-1} | y, theta) (Durbin & Koopman 2002), where
 ``conditional_simulation`` draws every time step on its own from the smoothed marginal.  ``forecast`` gives the
-forecast moments and joint draws of the paths after the end of the sample, and ``impulse_responses`` the responses of
-states and observations to one shock.  The reference draws its normals from
-NumPy's global RNG inside numba, so its trajectories are not reproducible from outside; here the standard-normal draws
-come from ``torch.randn`` on the device (or are passed in, which makes the result exactly checkable) and the CUDA kernels
-are deterministic transforms of them.
+forecast moments and joint draws of the paths after the end of the sample, ``conditional_forecast`` the same given
+known future values of some series, and ``impulse_responses`` the responses of states and observations to one shock.
+The reference draws its normals from NumPy's global RNG inside numba, so its trajectories are not reproducible from
+outside; here the standard-normal draws come from ``torch.randn`` on the device (or are passed in, which makes the
+result exactly checkable) and the CUDA kernels are deterministic transforms of them.
 """
 from __future__ import annotations
 
@@ -246,6 +246,88 @@ def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simul
         if bad is not None and bad.numel():
             u = int(bad[0, 0])
             raise RuntimeError(f"forecast: unit {u} failed with info {int(info[u])} (codes in include/kfb200.h)")
+    return res
+
+
+def _conditional_forecast(kalman: BatchedKalman, y, mats, conditions, n_simulations, z_init, z_state, z_obs,
+                          generator):
+    """Conditional forecast on ``kalman``'s geometry (the standard corrected filter over the n observations): its
+    predicted moments at index n start kfb_conditional_forecast.  conditions [H, p] shared or [U, H, p].  Returns
+    (result dict, forward info [U], window / paths info [U]) without raising on a non-zero info."""
+    lib = load()
+    dev = kalman.device
+    m, p, r, U, n = kalman.m, kalman.p, kalman.r, kalman.units, kalman.n
+    f64 = dict(dtype=torch.float64, device=dev)
+    if not (isinstance(conditions, torch.Tensor) and conditions.is_cuda and conditions.dtype == torch.float64
+            and conditions.ndim in (2, 3) and conditions.shape[-1] == p and conditions.shape[-2] >= 1
+            and (conditions.ndim == 2 or conditions.shape[0] == U)):
+        raise ValueError(f"conditions: expected a float64 CUDA tensor of shape [H, {p}] or [{U}, H, {p}]")
+    H = conditions.shape[-2]
+    cond = conditions.contiguous()
+    out = kalman.forward(y, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
+                         outputs=("predicted_states", "predicted_covs"))
+    start_mean, start_cov = out["predicted_states"][:, n].contiguous(), out["predicted_covs"][:, n].contiguous()
+    S = U * n_simulations
+    if S > 0:
+        z_init = torch.randn((S, m), generator=generator, **f64) if z_init is None else z_init
+        z_state = torch.randn((H - 1, S, r), generator=generator, **f64) if z_state is None else z_state
+        z_obs = torch.randn((H, S, p), generator=generator, **f64) if z_obs is None else z_obs
+        for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (H - 1, S, r)),
+                               ("z_obs", z_obs, (H, S, p))):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
+                raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
+        z_init, z_state, z_obs = z_init.contiguous(), z_state.contiguous(), z_obs.contiguous()
+    desc = kalman._desc
+    nbytes = ctypes.c_size_t(0)
+    check(lib.kfb_conditional_forecast_workspace_bytes(ctypes.byref(desc), H, n_simulations, ctypes.byref(nbytes)),
+          "kfb_conditional_forecast_workspace_bytes")
+    ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
+    res = {"state_mean": torch.empty((U, H, m), **f64), "state_cov": torch.empty((U, H, m, m), **f64),
+           "obs_mean": torch.empty((U, H, p), **f64), "obs_cov": torch.empty((U, H, p, p), **f64)}
+    states = torch.empty((H, S, m), **f64) if S > 0 else None
+    obs = torch.empty((H, S, p), **f64) if S > 0 else None
+    info = torch.empty(U, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.kfb_conditional_forecast(
+            ctypes.byref(desc), ctypes.byref(kalman._inputs), _ptr(start_mean), _ptr(start_cov), H, _ptr(cond),
+            H * p if cond.ndim == 3 else 0, n_simulations, _ptr(z_init) if S > 0 else None,
+            _ptr(z_state) if S > 0 and H > 1 else None, _ptr(z_obs) if S > 0 else None,
+            *[_ptr(res[k]) for k in ("state_mean", "state_cov", "obs_mean", "obs_cov")], _ptr(states), _ptr(obs),
+            _ptr(info), _ptr(ws), ws.numel(), _stream_ptr(dev)), "kfb_conditional_forecast")
+    if S > 0:
+        res["state_paths"], res["obs_paths"] = states.permute(1, 0, 2), obs.permute(1, 0, 2)
+    return res, out["info"], info
+
+
+def conditional_forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, conditions=None, n_simulations: int = 0,
+                         z_init=None, z_state=None, z_obs=None, generator: Optional[torch.Generator] = None):
+    """Conditional forecasts from the end of the sample: the law of x_n..x_{n+H-1} and y_n..y_{n+H-1} given
+    y_0..y_{n-1} and the known future values ``conditions[h, i]`` = y_{n+h, i} (NaN = free), and with ``n_simulations``
+    > 0 joint draws of those paths (the simulation smoother over the window with partly observed rows; include/kfb200.h,
+    kfb_conditional_forecast).  The horizon H is ``conditions.shape[-2]``; conditions is [H, p] shared by every unit or
+    [U, H, p] per unit (float64 CUDA, U = n_draws * n_series).
+
+    Arguments and conventions otherwise as in ``forecast``; the normals have the same shapes: z_init [S, m], z_state
+    [H-1, S, r], z_obs [H, S, p] for S = U * n_simulations.  Returns ``forecast``'s dict (same keys, same views):
+    state_mean [U, H, m], state_cov, obs_mean [U, H, p], obs_cov and with n_simulations > 0 state_paths [S, H, m],
+    obs_paths [S, H, p].  Conditioned entries of obs_mean and obs_paths equal the condition exactly and have zero rows
+    and columns in obs_cov.  With every entry NaN this is ``forecast`` (the paths bit for bit on the same normals).
+    Raises RuntimeError if some unit fails (F_t not positive definite in the sample or at a window step (n + h + 1),
+    a partly missing row in the sample, P_n / Q / H not positive semi-definite) and NotImplementedError for
+    time-varying matrices."""
+    mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
+    n_series = 1 if y.ndim == 2 else y.shape[0]
+    m, p, r = T.shape[-1], Z.shape[-2], R.shape[-1]
+    kalman = BatchedKalman("standard", y.shape[-2], m, p, r, n_draws=B, n_series=n_series, strict_reference=False,
+                           device=T.device)
+    res, finfo, winfo = _conditional_forecast(kalman, y, mats, conditions, int(n_simulations), z_init, z_state, z_obs,
+                                              generator)
+    for info in (finfo, winfo):
+        bad = torch.nonzero(info != 0)
+        if bad.numel():
+            u = int(bad[0, 0])
+            raise RuntimeError(f"conditional_forecast: unit {u} failed with info {int(info[u])} "
+                               "(codes in include/kfb200.h)")
     return res
 
 
