@@ -4,10 +4,8 @@
 
 #include "../../include/kfb200.h"
 #include "kf_aux.cuh"
-#include "kf_condfc.cuh"
-#include "kf_forecast.cuh"
+#include "kf_draws_run.cuh"
 #include "kf_kernels.cuh"
-#include "kf_simsmooth.cuh"
 #include "kf_tpar.cuh"
 
 namespace kfb {
@@ -170,6 +168,12 @@ static kfb_status cuda_fail(cudaError_t e) {
   return KFB_ERR_CUDA;
 }
 
+// The status of a launcher's result: cudaErrorInvalidConfiguration means the request needs more than a launch allows.
+static kfb_status launch_status(cudaError_t e) {
+  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
+  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+}
+
 static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A, bool bwd, cudaStream_t s) {
   cudaError_t e;
   if (pl.use_thread) {
@@ -198,86 +202,6 @@ static kfb_status launch_main(const kfb_desc* d, const Plan& pl, const KfArgs& A
     if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
   }
   return e == cudaSuccess ? KFB_OK : cuda_fail(e);
-}
-
-// Workspace of kfb_simulation_smoother: gain tape, per-unit factors, the u and r scratch of every simulation and the
-// per-unit status, each region rounded up to 256 bytes (the rule kfb200.h states).
-struct SsPlan {
-  size_t off_gain, off_fac, off_u, off_r, off_stat, total;
-};
-
-static kfb_status make_ss_plan(const kfb_desc* d, int64_t sims_per_unit, SsPlan* pl) {
-  if (!d || d->n_draws <= 0 || d->n_series <= 0 || d->n <= 0 || d->m <= 0 || d->p <= 0 || d->r <= 0 || sims_per_unit <= 0)
-    return KFB_ERR_INVALID_ARG;
-  if (d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts) return KFB_ERR_UNSUPPORTED;
-  if (d->m > ss::SS_MAX || d->p > ss::SS_MAX || d->r > ss::SS_MAX || d->n >= (1 << 29)) return KFB_ERR_UNSUPPORTED;
-  const long long U = d->n_draws * d->n_series;
-  const long long lanes = ss::warps_of(U * sims_per_unit) * 32;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  pl->off_gain = take((size_t)U * d->n * ss::gain_stride(d->m, d->p) * 8);
-  pl->off_fac = take((size_t)U * ss::fac_stride(d->m, d->p, d->r) * 8);
-  pl->off_u = take((size_t)d->n * lanes * d->p * 8);
-  pl->off_r = take((size_t)(d->n - 1) * lanes * d->m * 8);
-  pl->off_stat = take((size_t)U * 4);
-  pl->total = off;
-  return KFB_OK;
-}
-
-// Sizes and strides of kfb_forecast_paths / kfb_impulse_response: static matrices, dims up to ss::SS_MAX (desc->n,
-// filter_kind and flags are not read).
-static kfb_status check_forecast_desc(const kfb_desc* d) {
-  if (!d || d->n_draws <= 0 || d->n_series <= 0 || d->m <= 0 || d->p <= 0 || d->r <= 0) return KFB_ERR_INVALID_ARG;
-  if (d->T_ts || d->Z_ts || d->R_ts || d->H_ts || d->Q_ts || d->c_ts || d->d_ts) return KFB_ERR_UNSUPPORTED;
-  if (d->m > ss::SS_MAX || d->p > ss::SS_MAX || d->r > ss::SS_MAX) return KFB_ERR_UNSUPPORTED;
-  return KFB_OK;
-}
-
-static_assert(fc::SHOCK_UNIT == KFB_SHOCK_UNIT && fc::SHOCK_STD == KFB_SHOCK_STD &&
-                  fc::SHOCK_CHOLESKY == KFB_SHOCK_CHOLESKY && ss::INFO_NOT_PSD == KFB_INFO_NOT_PSD,
-              "kf_forecast.cuh / kf_simsmooth.cuh constants differ from include/kfb200.h");
-
-// Workspace of kfb_forecast_paths: per-unit factors and status, each region rounded up to 256 bytes (kfb200.h).
-struct FcPlan {
-  size_t off_fac, off_stat, total;
-};
-
-static kfb_status make_fc_plan(const kfb_desc* d, int64_t sims_per_unit, FcPlan* pl) {
-  kfb_status st = check_forecast_desc(d);
-  if (st != KFB_OK) return st;
-  if (sims_per_unit <= 0) return KFB_ERR_INVALID_ARG;
-  const long long U = d->n_draws * d->n_series;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  pl->off_fac = take((size_t)U * fc::fac_stride(d->m, d->p, d->r) * 8);
-  pl->off_stat = take((size_t)U * 4);
-  pl->total = off;
-  return KFB_OK;
-}
-
-// Workspace of kfb_conditional_forecast: window tape, per-unit factors, run-time-dims scratch, per-unit status and the
-// u and r scratch of the paths, each region rounded up to 256 bytes (kfb200.h).
-struct CfPlan {
-  size_t off_tape, off_fac, off_wscr, off_stat, off_u, off_r, total;
-};
-
-static kfb_status make_cf_plan(const kfb_desc* d, int32_t horizon, int64_t sims_per_unit, CfPlan* pl) {
-  kfb_status st = check_forecast_desc(d);
-  if (st != KFB_OK) return st;
-  if (horizon < 1 || sims_per_unit < 0 || d->n < 0) return KFB_ERR_INVALID_ARG;
-  if (d->n >= (1 << 29) || horizon >= (1 << 29)) return KFB_ERR_UNSUPPORTED;
-  const long long U = d->n_draws * d->n_series;
-  const long long lanes = ss::warps_of(U * sims_per_unit) * 32;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  pl->off_tape = take((size_t)U * horizon * cf::tape_stride(d->m, d->p) * 8);
-  pl->off_fac = take((size_t)U * ss::fac_stride(d->m, d->p, d->r) * 8);
-  pl->off_wscr = take((size_t)U * cf::wscr_stride(d->m, d->p) * 8);
-  pl->off_stat = take((size_t)U * 4);
-  pl->off_u = take((size_t)horizon * lanes * d->p * 8);
-  pl->off_r = take((size_t)(horizon - 1) * lanes * d->m * 8);
-  pl->total = off;
-  return KFB_OK;
 }
 
 }  // namespace kfb
@@ -439,8 +363,7 @@ kfb_status kfb_smoother_ex(int64_t n_draws, int64_t n_series, int32_t n, int32_t
     const smoother_launch_fn per_thread = find_smoother_thread_launcher(m);
     e = per_thread ? per_thread(S, s) : launch_smoother(S, s);
   }
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(e);
 }
 
 kfb_status kfb_lyapunov_forward(int64_t B, int32_t m, int32_t r, const double* A, int64_t A_bs, const double* R,
@@ -448,8 +371,7 @@ kfb_status kfb_lyapunov_forward(int64_t B, int32_t m, int32_t r, const double* A
   if (B <= 0 || m <= 0 || r <= 0 || !A || !R || !Q || !X) return KFB_ERR_INVALID_ARG;
   cudaError_t e = launch_lyapunov_forward(B, m, r, MatArg{A, A_bs, 0}, MatArg{R, R_bs, 0}, MatArg{Q, Q_bs, 0}, X, info,
                                           (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(e);
 }
 
 kfb_status kfb_lyapunov_backward(int64_t B, int32_t m, int32_t r, const double* A, int64_t A_bs, const double* R,
@@ -458,8 +380,7 @@ kfb_status kfb_lyapunov_backward(int64_t B, int32_t m, int32_t r, const double* 
   if (B <= 0 || m <= 0 || r <= 0 || !A || !R || !Q || !X || !Xbar) return KFB_ERR_INVALID_ARG;
   cudaError_t e = launch_lyapunov_backward(B, m, r, MatArg{A, A_bs, 0}, MatArg{R, R_bs, 0}, MatArg{Q, Q_bs, 0}, X, Xbar,
                                            Abar, Rbar, Qbar, (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(e);
 }
 
 kfb_status kfb_scatter_forward(int64_t B, int32_t n_theta, int32_t block, int32_t n_map, const double* theta,
@@ -502,8 +423,7 @@ kfb_status kfb_scatter_backward_multi(int64_t B, int32_t n_theta, int32_t n_seg,
                                       double* gtheta, void* stream) {
   if (B <= 0 || n_theta <= 0 || !gtheta || !scatter_segs_ok(n_seg, segs, false)) return KFB_ERR_INVALID_ARG;
   cudaError_t e = launch_scatter_backward_multi(B, n_theta, n_seg, segs, gtheta, (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;  // mapped elements exceed shared memory
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(e);  // UNSUPPORTED: the mapped elements exceed shared memory
 }
 
 kfb_status kfb_simulate(int64_t n_draws, int64_t sims_per_draw, int32_t n, int32_t m, int32_t p, int32_t r, const double* T,
@@ -532,8 +452,8 @@ kfb_status kfb_mvn_draws(int64_t n_units, int64_t sims_per_unit, int32_t n, int3
 
 kfb_status kfb_simulation_smoother_workspace_bytes(const kfb_desc* desc, int64_t sims_per_unit, size_t* bytes) {
   if (!bytes) return KFB_ERR_INVALID_ARG;
-  SsPlan pl;
-  kfb_status st = make_ss_plan(desc, sims_per_unit, &pl);
+  draws::SsPlan pl;
+  kfb_status st = draws::plan_ss(desc, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   *bytes = pl.total;
   return KFB_OK;
@@ -543,36 +463,26 @@ kfb_status kfb_simulation_smoother(const kfb_desc* desc, const kfb_inputs* in, c
                                    int64_t sims_per_unit, const double* z_init, const double* z_state,
                                    const double* z_obs, double* states, int32_t* info, void* workspace,
                                    size_t workspace_bytes, void* stream) {
-  SsPlan pl;
-  kfb_status st = make_ss_plan(desc, sims_per_unit, &pl);
+  draws::SsPlan pl;
+  kfb_status st = draws::plan_ss(desc, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   if (!in || !in->y || !in->a0 || !in->P0 || !in->T || !in->Z || !in->R || !in->H || !in->Q || !predicted_covs ||
       !z_init || (desc->n > 1 && !z_state) || !z_obs || !states || !info)
     return KFB_ERR_INVALID_ARG;
   if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
-  char* ws = (char*)workspace;
-  ss::Args A;
-  std::memset(&A, 0, sizeof(A));
-  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
-  A.n = desc->n; A.m = desc->m; A.p = desc->p; A.r = desc->r;
-  A.y = {in->y, desc->y_bs, 0}; A.a0 = {in->a0, desc->a0_bs, 0}; A.P0 = {in->P0, desc->P0_bs, 0};
-  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
-  A.H = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
-  A.pc = predicted_covs; A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs; A.states = states; A.info = info;
-  A.gain = (double*)(ws + pl.off_gain); A.fac = (double*)(ws + pl.off_fac);
-  A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r); A.ustat = (int*)(ws + pl.off_stat);
+  const ss::Args A =
+      draws::ss_args(desc, in, predicted_covs, sims_per_unit, z_init, z_state, z_obs, states, info, workspace, pl);
+  const draws::Fill f = draws::ss_status_init(A);
   cudaStream_t s = (cudaStream_t)stream;
-  cudaError_t e = cudaMemsetAsync(A.ustat, 0x7f, (size_t)A.U * 4, s);  // every word = ss::KEY_NONE
+  const cudaError_t e = cudaMemsetAsync(f.p, f.value, f.bytes, s);
   if (e != cudaSuccess) return cuda_fail(e);
-  e = launch_simulation_smoother(A, s);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(launch_simulation_smoother(A, s));
 }
 
 kfb_status kfb_forecast_paths_workspace_bytes(const kfb_desc* desc, int64_t sims_per_unit, size_t* bytes) {
   if (!bytes) return KFB_ERR_INVALID_ARG;
-  FcPlan pl;
-  kfb_status st = make_fc_plan(desc, sims_per_unit, &pl);
+  draws::FcPlan pl;
+  kfb_status st = draws::plan_fc(desc, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   *bytes = pl.total;
   return KFB_OK;
@@ -582,34 +492,23 @@ kfb_status kfb_forecast_paths(const kfb_desc* desc, const kfb_inputs* in, const 
                               const double* start_cov, int32_t horizon, int64_t sims_per_unit, const double* z_init,
                               const double* z_state, const double* z_obs, double* states, double* obs, int32_t* info,
                               void* workspace, size_t workspace_bytes, void* stream) {
-  FcPlan pl;
-  kfb_status st = make_fc_plan(desc, sims_per_unit, &pl);
+  draws::FcPlan pl;
+  kfb_status st = draws::plan_fc(desc, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   if (horizon < 1 || !in || !in->T || !in->Z || !in->R || !in->H || !in->Q || !start_mean || !start_cov || !z_init ||
       (horizon > 1 && !z_state) || !z_obs || (!states && !obs) || !info)
     return KFB_ERR_INVALID_ARG;
   if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
-  char* ws = (char*)workspace;
-  fc::Args A;
-  std::memset(&A, 0, sizeof(A));
-  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
-  A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r;
-  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
-  A.Hm = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
-  A.mean = start_mean; A.cov = start_cov; A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs;
-  A.states = states; A.obs = obs; A.info = info;
-  A.vec = (uintptr_t)states % 16 == 0 && (uintptr_t)obs % 16 == 0;
-  A.fac = (double*)(ws + pl.off_fac); A.ustat = (int*)(ws + pl.off_stat);
-  const cudaError_t e = launch_forecast_paths(A, (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  const fc::Args A = draws::fc_args(desc, in, start_mean, start_cov, horizon, sims_per_unit, z_init, z_state, z_obs,
+                                    states, obs, info, workspace, pl);
+  return launch_status(launch_forecast_paths(A, (cudaStream_t)stream));
 }
 
 kfb_status kfb_conditional_forecast_workspace_bytes(const kfb_desc* desc, int32_t horizon, int64_t sims_per_unit,
                                                     size_t* bytes) {
   if (!bytes) return KFB_ERR_INVALID_ARG;
-  CfPlan pl;
-  kfb_status st = make_cf_plan(desc, horizon, sims_per_unit, &pl);
+  draws::CfPlan pl;
+  kfb_status st = draws::plan_cf(desc, horizon, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   *bytes = pl.total;
   return KFB_OK;
@@ -621,49 +520,29 @@ kfb_status kfb_conditional_forecast(const kfb_desc* desc, const kfb_inputs* in, 
                                     const double* z_obs, double* state_mean, double* state_cov, double* obs_mean,
                                     double* obs_cov, double* states, double* obs, int32_t* info, void* workspace,
                                     size_t workspace_bytes, void* stream) {
-  CfPlan pl;
-  kfb_status st = make_cf_plan(desc, horizon, sims_per_unit, &pl);
+  draws::CfPlan pl;
+  kfb_status st = draws::plan_cf(desc, horizon, sims_per_unit, &pl);
   if (st != KFB_OK) return st;
   const bool paths = sims_per_unit > 0;
   if (!in || !in->T || !in->Z || !in->R || !in->H || !in->Q || !start_mean || !start_cov || !cond || cond_bs < 0 ||
       !info || (paths && (!z_init || (horizon > 1 && !z_state) || !z_obs || (!states && !obs))))
     return KFB_ERR_INVALID_ARG;
   if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
-  char* ws = (char*)workspace;
-  cf::Args A;
-  std::memset(&A, 0, sizeof(A));
-  A.U = desc->n_draws * desc->n_series; A.n_series = desc->n_series; A.spu = sims_per_unit; A.S = A.U * sims_per_unit;
-  A.n = desc->n; A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r;
-  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0};
-  A.Hm = {in->H, desc->H_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0}; A.c = {in->c, desc->c_bs, 0}; A.d = {in->d, desc->d_bs, 0};
-  A.mean = start_mean; A.cov = start_cov; A.cond = cond; A.cond_bs = cond_bs;
-  A.state_mean = state_mean; A.state_cov = state_cov; A.obs_mean = obs_mean; A.obs_cov = obs_cov; A.info = info;
-  if (paths) {
-    A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs; A.states = states; A.obs = obs;
-    A.vec = (uintptr_t)states % 16 == 0 && (uintptr_t)obs % 16 == 0;
-  }
-  A.tape = (double*)(ws + pl.off_tape); A.fac = (double*)(ws + pl.off_fac); A.wscr = (double*)(ws + pl.off_wscr);
-  A.ustat = (int*)(ws + pl.off_stat); A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r);
-  const cudaError_t e = launch_conditional_forecast(A, (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  const cf::Args A = draws::cf_args(desc, in, start_mean, start_cov, horizon, cond, cond_bs, sims_per_unit, z_init,
+                                    z_state, z_obs, state_mean, state_cov, obs_mean, obs_cov, states, obs, info,
+                                    workspace, pl);
+  return launch_status(launch_conditional_forecast(A, (cudaStream_t)stream));
 }
 
 kfb_status kfb_impulse_response(const kfb_desc* desc, const kfb_inputs* in, int32_t horizon, int32_t shock,
                                 double* states, double* obs, int32_t* info, void* stream) {
-  kfb_status st = check_forecast_desc(desc);
+  kfb_status st = draws::check_desc(desc);
   if (st != KFB_OK) return st;
   if (horizon < 1 || shock < KFB_SHOCK_UNIT || shock > KFB_SHOCK_CHOLESKY || !in || !in->T || !in->Z || !in->R ||
       !in->Q || (!states && !obs) || !info)
     return KFB_ERR_INVALID_ARG;
-  fc::IrfArgs A;
-  std::memset(&A, 0, sizeof(A));
-  A.nD = desc->n_draws; A.H = horizon; A.m = desc->m; A.p = desc->p; A.r = desc->r; A.shock = shock;
-  A.T = {in->T, desc->T_bs, 0}; A.Z = {in->Z, desc->Z_bs, 0}; A.R = {in->R, desc->R_bs, 0}; A.Q = {in->Q, desc->Q_bs, 0};
-  A.states = states; A.obs = obs; A.info = info;
-  const cudaError_t e = launch_impulse_response(A, (cudaStream_t)stream);
-  if (e == cudaErrorInvalidConfiguration) return KFB_ERR_UNSUPPORTED;
-  return e == cudaSuccess ? KFB_OK : cuda_fail(e);
+  return launch_status(launch_impulse_response(draws::irf_args(desc, in, horizon, shock, states, obs, info),
+                                               (cudaStream_t)stream));
 }
 
 kfb_status kfb_fp64_peak_distinct(int32_t iters, int32_t blocks, int32_t threads, double* sink, double* h_flops,

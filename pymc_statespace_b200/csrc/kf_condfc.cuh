@@ -1,5 +1,6 @@
 // kf_condfc.cuh - conditional forecasts from the end of the sample, written once as KFB_HD functions: kf_condfc.cu runs
-// them as kernels and the host build of the kernels (tests/hostsim) runs them on the host.
+// them as kernels and the host build of the kernels (tests/hostsim/draws.cpp, requests from kf_draws_run.cuh) runs them
+// on the host.
 //
 // Model (the filters', as in kf_forecast.cuh): y_t = Z x_t + d + eps_t, eps_t ~ N(0, H); x_{t+1} = T x_t + c + R eta_t,
 // eta_t ~ N(0, Q); static matrices.  Window index h is time n + h, h = 0..H-1.  cond[h][i] is the known value of

@@ -1,5 +1,6 @@
 // kf_forecast.cuh - forecast paths and impulse responses from the end of the sample, written once as KFB_HD functions:
-// kf_forecast.cu runs them as kernels and the host build of the kernels (tests/hostsim) runs them on the host.
+// kf_forecast.cu runs them as kernels and the host build of the kernels (tests/hostsim/draws.cpp, requests from
+// kf_draws_run.cuh) runs them on the host.
 //
 // Model (the filters', as in kf_simsmooth.cuh): y_t = Z x_t + d + eps_t, eps_t ~ N(0, H); x_{t+1} = T x_t + c + R eta_t,
 // eta_t ~ N(0, Q); static matrices.  Given the state's distribution N(a, P) at the first forecast time (a_n, P_n: the

@@ -1,6 +1,6 @@
 // kf_simsmooth.cuh - the simulation smoother (Durbin & Koopman 2002, mean correction, with the fast state smoother of
 // Durbin & Koopman's book, section 4.6.2), written once as KFB_HD functions: kf_simsmooth.cu runs them as kernels and
-// the host build of the kernels (tests/hostsim) runs them on the host.
+// the host build of the kernels (tests/hostsim/draws.cpp, requests from kf_draws_run.cuh) runs them on the host.
 //
 // Model (the one the filters evaluate): x_0 ~ N(a0, P0); y_t = Z x_t + d + eps_t, eps_t ~ N(0, H), t = 0..n-1;
 // x_{t+1} = T x_t + c + R eta_t, eta_t ~ N(0, Q), t = 0..n-2.  (kfb_simulate's shifted convention obs[t] = Z x_{t-1} is

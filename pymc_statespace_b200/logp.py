@@ -295,6 +295,65 @@ class KalmanLogp:
             out["filtered_covs"] = out["filtered_covs"][..., :m, :m].contiguous()
         return ss, sc, out
 
+    def _exact_kalman(self, n):
+        """The exact (corrected standard) filter over n steps for the per-draw calls: one cached for the sample's n
+        and one for the last other n (n + horizon of ``forecast``)."""
+        slot = "_ss_kalman" if n == self.n else "_fc_kalman"
+        kal = getattr(self, slot, None)
+        if kal is None or kal.n != n:
+            sp = self.spec
+            kal = BatchedKalman("standard", n, sp.k_states, sp.k_endog, sp.k_posdef, n_draws=self.B,
+                                strict_reference=False, device=self.device)
+            setattr(self, slot, kal)
+        return kal
+
+    def _not_stationary(self):
+        """[B] bool: the draws of the last scatter whose stationary P0 does not exist (None without a stationary P0)."""
+        if self.spec.stationary_initialization and getattr(self, "_lyap", None) is not None:
+            return self._lyap[2] != 0
+        return None
+
+    def _stationary_info(self, info):
+        """``info`` with KFB_INFO_NOT_STATIONARY for every draw whose stationary P0 does not exist (it replaces the
+        follow-on code of that draw)."""
+        bad = self._not_stationary()
+        return info if bad is None else torch.where(bad, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
+
+    def _per_draw(self, theta, n, n_simulations, generator, z_init, run, kernel_nans=False):
+        """A per-draw call of ``simulation`` after the theta scatter (and stationary P0):
+        ``run(kalman, mats, z_init)`` on the exact filter over n steps returns (outputs dict, info tensors in order of
+        precedence).  z_init is padded for a padded model (the extra states are identically zero, their normals
+        unused).  Returns (outputs, info [B]): info is the stationarity code, else the first non-zero code of the
+        tensors; every output of a failing draw is NaN and the padded states are sliced off (views).  ``kernel_nans``:
+        the outputs are already NaN for every non-zero code of the tensors, so only the non-stationary draws are
+        masked (a mask is a full pass over the outputs)."""
+        mats = self._scatter(self._check_theta(theta))
+        m, m0, S = self.spec.k_states, self.k_states_model, self.B * int(n_simulations)
+        kal = self._exact_kalman(n)
+        if S > 0 and m != m0:
+            if z_init is None:
+                z_init = torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator)
+            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
+        res, infos = run(kal, mats, z_init)
+        info = self._stationary_info(infos[0])
+        for later in infos[1:]:
+            if later is not None:
+                info = torch.where(info == 0, later, info)
+        bad = self._not_stationary() if kernel_nans else info != 0
+        if bad is not None:
+            for k, v in res.items():
+                if k.endswith("_paths"):  # [S, ., .] draw-major (views of the time-major buffers for the forecasts)
+                    v.unflatten(0, (self.B, -1))[bad] = float("nan")
+                else:
+                    v[bad] = float("nan")
+        if m != m0:
+            for k in ("state_mean", "state_paths"):
+                if k in res:
+                    res[k] = res[k][..., :m0]
+            if "state_cov" in res:
+                res["state_cov"] = res["state_cov"][..., :m0, :m0]
+        return res, info
+
     def sample_states(self, theta, n_simulations: int = 1, generator: Optional[torch.Generator] = None,
                       z_init=None, z_state=None, z_obs=None) -> torch.Tensor:
         """Joint draws of the latent state paths from p(x_0..x_{n-1} | y, theta) for every draw: the simulation smoother
@@ -307,25 +366,14 @@ class KalmanLogp:
         may be given as in ``simulation_smoother``, sized for the model's own k_states."""
         from .simulation import _simulation_smoother
 
-        mats = self._scatter(self._check_theta(theta))
-        sp = self.spec
-        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
-        if getattr(self, "_ss_kalman", None) is None:
-            self._ss_kalman = BatchedKalman("standard", self.n, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
-                                            strict_reference=False, device=self.device)
-        if z_init is not None and m != m0:  # padded model: the extra states are identically zero, their normals unused
-            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
-        if z_init is None and m != m0:
-            z_init = torch.nn.functional.pad(
-                torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator), (0, m - m0))
-        states, info = _simulation_smoother(self._ss_kalman, self.y, mats, int(n_simulations), z_init, z_state, z_obs,
-                                            generator)
-        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
-            bad = self._lyap[2] != 0
-            info = torch.where(bad, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
-            states.view(self.B, -1)[bad] = float("nan")
-        self._ss_info = info
-        return states[..., :m0].contiguous() if m != m0 else states
+        def run(kal, mats, z_init):
+            states, info = _simulation_smoother(kal, self.y, mats, int(n_simulations), z_init, z_state, z_obs,
+                                                generator)
+            return {"state_paths": states}, (info,)
+
+        # the kernel writes NaN paths for its own failures
+        res, self._ss_info = self._per_draw(theta, self.n, n_simulations, generator, z_init, run, kernel_nans=True)
+        return res["state_paths"].contiguous()
 
     def forecast(self, theta, horizon: int, n_simulations: int = 0, generator: Optional[torch.Generator] = None,
                  z_init=None, z_state=None, z_obs=None) -> Dict[str, torch.Tensor]:
@@ -344,34 +392,13 @@ class KalmanLogp:
         H = int(horizon)
         if H < 1:
             raise ValueError("horizon must be >= 1")
-        mats = self._scatter(self._check_theta(theta))
-        sp = self.spec
-        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
-        kal = getattr(self, "_fc_kalman", None)
-        if kal is None or kal.n != self.n + H:
-            self._fc_kalman = kal = BatchedKalman("standard", self.n + H, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
-                                                  strict_reference=False, device=self.device)
-        if S > 0 and m != m0:  # padded model: the extra states are identically zero, their normals unused
-            if z_init is None:
-                z_init = torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator)
-            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
-        res, info, pinfo = _forecast(kal, self.y, mats, H, int(n_simulations), z_init, z_state, z_obs, generator)
-        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
-            info = torch.where(self._lyap[2] != 0, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
-        if pinfo is not None:
-            info = torch.where(info == 0, pinfo, info)
-        bad = info != 0
-        for k, v in res.items():
-            if k.endswith("_paths"):  # [S, H, .] views of the time-major buffers, draw-major
-                v.unflatten(0, (self.B, -1))[bad] = float("nan")
-            else:
-                v[bad] = float("nan")
-        if m != m0:
-            for k in ("state_mean", "state_paths"):
-                if k in res:
-                    res[k] = res[k][..., :m0]
-            res["state_cov"] = res["state_cov"][..., :m0, :m0]
-        res["info"] = info
+
+        def run(kal, mats, z_init):
+            res, info, pinfo = _forecast(kal, self.y, mats, H, int(n_simulations), z_init, z_state, z_obs, generator)
+            return res, (info, pinfo)
+
+        res, res_info = self._per_draw(theta, self.n + H, n_simulations, generator, z_init, run)
+        res["info"] = res_info
         return res
 
     def conditional_forecast(self, theta, conditions, n_simulations: int = 0,
@@ -388,33 +415,13 @@ class KalmanLogp:
         k_states."""
         from .simulation import _conditional_forecast
 
-        mats = self._scatter(self._check_theta(theta))
-        sp = self.spec
-        m, m0, S = sp.k_states, self.k_states_model, self.B * int(n_simulations)
-        if getattr(self, "_ss_kalman", None) is None:
-            self._ss_kalman = BatchedKalman("standard", self.n, m, sp.k_endog, sp.k_posdef, n_draws=self.B,
-                                            strict_reference=False, device=self.device)
-        if S > 0 and m != m0:  # padded model: the extra states are identically zero, their normals unused
-            if z_init is None:
-                z_init = torch.randn((S, m0), dtype=torch.float64, device=self.device, generator=generator)
-            z_init = torch.nn.functional.pad(z_init, (0, m - m0))
-        res, info, winfo = _conditional_forecast(self._ss_kalman, self.y, mats, conditions, int(n_simulations), z_init,
-                                                 z_state, z_obs, generator)
-        if sp.stationary_initialization and getattr(self, "_lyap", None) is not None:
-            info = torch.where(self._lyap[2] != 0, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
-        info = torch.where(info == 0, winfo, info)
-        bad = info != 0
-        for k, v in res.items():
-            if k.endswith("_paths"):  # [S, H, .] views of the time-major buffers, draw-major
-                v.unflatten(0, (self.B, -1))[bad] = float("nan")
-            else:
-                v[bad] = float("nan")
-        if m != m0:
-            for k in ("state_mean", "state_paths"):
-                if k in res:
-                    res[k] = res[k][..., :m0]
-            res["state_cov"] = res["state_cov"][..., :m0, :m0]
-        res["info"] = info
+        def run(kal, mats, z_init):
+            res, info, winfo = _conditional_forecast(kal, self.y, mats, conditions, int(n_simulations), z_init,
+                                                     z_state, z_obs, generator)
+            return res, (info, winfo)
+
+        res, res_info = self._per_draw(theta, self.n, n_simulations, generator, z_init, run)
+        res["info"] = res_info
         return res
 
     def impulse_responses(self, theta, horizon: int, shock: str = "cholesky") -> Dict[str, torch.Tensor]:
@@ -452,11 +459,7 @@ class KalmanLogp:
         bilinear solve returns a finite non-PSD matrix there and carries on, here logp is NaN) is reported as
         KFB_INFO_NOT_STATIONARY instead of the follow-on "F_0 not positive definite".  Merged lazily: nothing is added
         to the per-evaluation launch sequence."""
-        info = self._kf_info
-        if self.spec.stationary_initialization and getattr(self, "_lyap", None) is not None:
-            bad = self._lyap[2] != 0
-            info = torch.where(bad, torch.full_like(info, KFB_INFO_NOT_STATIONARY), info)
-        return info
+        return self._stationary_info(self._kf_info)
 
     def capture_host_step(self, theta_host: torch.Tensor, out_host: torch.Tensor, chunks: int = 1,
                           sequential: bool = False) -> "HostStepGraph":

@@ -84,6 +84,50 @@ def conditional_simulation(mus, covs, n_simulations: int = 100, z=None, jitter=N
 _BASE_NDIM = {"a0": 1, "P0": 2, "T": 2, "Z": 2, "R": 2, "H": 2, "Q": 2, "c": 1, "d": 1}
 
 
+def _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y):
+    mats = {"a0": a0, "P0": P0, "T": T, "Z": Z, "R": R, "H": H, "Q": Q, "c": c, "d": d}
+    for k, t in mats.items():
+        if t is not None and k in ("a0", "c", "d") and t.ndim >= 2 and t.shape[-1] == 1:
+            mats[k] = t = t[..., 0]
+        if t is not None and t.ndim > _BASE_NDIM[k] + 1:
+            raise NotImplementedError("time-varying matrices are not supported")
+    if y is not None and y.ndim == 3 and y.shape[-1] == 1 and y.shape[-2] == Z.shape[-2]:
+        y = y[..., 0]  # reference layout [n, p, 1]
+    B = max([t.shape[0] for k, t in mats.items() if t is not None and t.ndim == _BASE_NDIM[k] + 1] + [1])
+    return mats, y, B
+
+
+def _normals(S, steps, m, p, r, z_init, z_state, z_obs, generator, dev):
+    """Time-major standard normals of S simulations over ``steps`` steps: z_init [S, m], z_state [steps-1, S, r],
+    z_obs [steps, S, p], each drawn with ``torch.randn`` if None, else checked.  Returns them contiguous."""
+    out = []
+    for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (max(steps - 1, 0), S, r)),
+                           ("z_obs", z_obs, (steps, S, p))):
+        if t is None:
+            t = torch.randn(shape, generator=generator, dtype=torch.float64, device=dev)
+        elif not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
+            raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
+        out.append(t.contiguous())
+    return out
+
+
+def _workspace(lib, call, desc, dev, *args):
+    """The workspace of ``call`` for ``desc`` on ``dev`` (``call``_workspace_bytes with ``args``), at least 256 bytes."""
+    nbytes = ctypes.c_size_t(0)
+    check(getattr(lib, call + "_workspace_bytes")(ctypes.byref(desc), *args, ctypes.byref(nbytes)),
+          call + "_workspace_bytes")
+    return torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
+
+
+def _raise_on_failure(what, infos, unit="unit", codes="codes in include/kfb200.h"):
+    """RuntimeError naming the first failing unit of the first info tensor (None: skipped) that has one."""
+    for info in infos:
+        bad = torch.nonzero(info != 0) if info is not None else None
+        if bad is not None and bad.numel():
+            u = int(bad[0, 0])
+            raise RuntimeError(f"{what}: {unit} {u} failed with info {int(info[u])} ({codes})")
+
+
 def _simulation_smoother(kalman: BatchedKalman, y, mats, n_simulations, z_init, z_state, z_obs, generator):
     """kfb_forward (predicted covariances) then kfb_simulation_smoother on ``kalman``'s geometry.  Returns
     (states [U*S, n, m], info [U]) without raising on a non-zero info."""
@@ -93,21 +137,10 @@ def _simulation_smoother(kalman: BatchedKalman, y, mats, n_simulations, z_init, 
     S = U * n_simulations
     pc = kalman.forward(y, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
                         outputs=("predicted_covs",))["predicted_covs"]
-    f64 = dict(dtype=torch.float64, device=dev)
-    z_init = torch.randn((S, m), generator=generator, **f64) if z_init is None else z_init
-    z_state = torch.randn((max(n - 1, 0), S, r), generator=generator, **f64) if z_state is None else z_state
-    z_obs = torch.randn((n, S, p), generator=generator, **f64) if z_obs is None else z_obs
-    for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (max(n - 1, 0), S, r)),
-                           ("z_obs", z_obs, (n, S, p))):
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
-            raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
-    z_init, z_state, z_obs = z_init.contiguous(), z_state.contiguous(), z_obs.contiguous()
+    z_init, z_state, z_obs = _normals(S, n, m, p, r, z_init, z_state, z_obs, generator, dev)
     desc = kalman._desc
-    nbytes = ctypes.c_size_t(0)
-    check(lib.kfb_simulation_smoother_workspace_bytes(ctypes.byref(desc), n_simulations, ctypes.byref(nbytes)),
-          "kfb_simulation_smoother_workspace_bytes")
-    ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
-    states = torch.empty((S, n, m), **f64)
+    ws = _workspace(lib, "kfb_simulation_smoother", desc, dev, n_simulations)
+    states = torch.empty((S, n, m), dtype=torch.float64, device=dev)
     info = torch.empty(U, dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
         check(lib.kfb_simulation_smoother(ctypes.byref(desc), ctypes.byref(kalman._inputs), _ptr(pc), n_simulations,
@@ -128,24 +161,13 @@ def simulation_smoother(y, a0, P0, T, Z, R, H, Q, c=None, d=None, n_simulations:
     [n-1, S, r], z_obs [n, S, p] for S = U * n_simulations; otherwise they are drawn with ``torch.randn``.
     Returns states [S, n, m].  Raises RuntimeError if some unit fails (F_t not positive definite, a partly missing row,
     P0 / Q / H not positive semi-definite) and NotImplementedError for time-varying matrices."""
-    mats = {"a0": a0, "P0": P0, "T": T, "Z": Z, "R": R, "H": H, "Q": Q, "c": c, "d": d}
-    for k, t in mats.items():
-        if t is not None and k in ("a0", "c", "d") and t.ndim >= 2 and t.shape[-1] == 1:
-            mats[k] = t = t[..., 0]
-        if t is not None and t.ndim > _BASE_NDIM[k] + 1:
-            raise NotImplementedError("simulation_smoother: time-varying matrices are not supported")
-    if y.ndim == 3 and y.shape[-1] == 1 and y.shape[-2] == Z.shape[-2]:
-        y = y[..., 0]  # reference layout [n, p, 1]
+    mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
     n_series = 1 if y.ndim == 2 else y.shape[0]
     m, p, r = T.shape[-1], Z.shape[-2], R.shape[-1]
-    B = max([t.shape[0] for k, t in mats.items() if t is not None and t.ndim == _BASE_NDIM[k] + 1] + [1])
     kalman = BatchedKalman("standard", y.shape[-2], m, p, r, n_draws=B, n_series=n_series, strict_reference=False,
                            device=T.device)
     states, info = _simulation_smoother(kalman, y, mats, int(n_simulations), z_init, z_state, z_obs, generator)
-    bad = torch.nonzero(info != 0)
-    if bad.numel():
-        u = int(bad[0, 0])
-        raise RuntimeError(f"simulation_smoother: unit {u} failed with info {int(info[u])} (codes in include/kfb200.h)")
+    _raise_on_failure("simulation_smoother", (info,))
     return states
 
 
@@ -177,19 +199,10 @@ def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_
     if n_simulations <= 0:
         return res, out["info"], None
     S = U * n_simulations
-    z_init = torch.randn((S, m), generator=generator, **f64) if z_init is None else z_init
-    z_state = torch.randn((H - 1, S, r), generator=generator, **f64) if z_state is None else z_state
-    z_obs = torch.randn((H, S, p), generator=generator, **f64) if z_obs is None else z_obs
-    for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (H - 1, S, r)), ("z_obs", z_obs, (H, S, p))):
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
-            raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
-    z_init, z_state, z_obs = z_init.contiguous(), z_state.contiguous(), z_obs.contiguous()
+    z_init, z_state, z_obs = _normals(S, H, m, p, r, z_init, z_state, z_obs, generator, dev)
     start_mean, start_cov = a[:, 0].contiguous(), P[:, 0].contiguous()
     desc = kalman._desc
-    nbytes = ctypes.c_size_t(0)
-    check(lib.kfb_forecast_paths_workspace_bytes(ctypes.byref(desc), n_simulations, ctypes.byref(nbytes)),
-          "kfb_forecast_paths_workspace_bytes")
-    ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
+    ws = _workspace(lib, "kfb_forecast_paths", desc, dev, n_simulations)
     states = torch.empty((H, S, m), **f64)
     obs = torch.empty((H, S, p), **f64)
     info = torch.empty(U, dtype=torch.int32, device=dev)
@@ -200,19 +213,6 @@ def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_
               "kfb_forecast_paths")
     res["state_paths"], res["obs_paths"] = states.permute(1, 0, 2), obs.permute(1, 0, 2)
     return res, out["info"], info
-
-
-def _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y):
-    mats = {"a0": a0, "P0": P0, "T": T, "Z": Z, "R": R, "H": H, "Q": Q, "c": c, "d": d}
-    for k, t in mats.items():
-        if t is not None and k in ("a0", "c", "d") and t.ndim >= 2 and t.shape[-1] == 1:
-            mats[k] = t = t[..., 0]
-        if t is not None and t.ndim > _BASE_NDIM[k] + 1:
-            raise NotImplementedError("time-varying matrices are not supported")
-    if y is not None and y.ndim == 3 and y.shape[-1] == 1 and y.shape[-2] == Z.shape[-2]:
-        y = y[..., 0]  # reference layout [n, p, 1]
-    B = max([t.shape[0] for k, t in mats.items() if t is not None and t.ndim == _BASE_NDIM[k] + 1] + [1])
-    return mats, y, B
 
 
 def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simulations: int = 0, z_init=None,
@@ -241,11 +241,7 @@ def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simul
     kalman = BatchedKalman("standard", y.shape[-2] + int(horizon), m, p, r, n_draws=B, n_series=n_series,
                            strict_reference=False, device=T.device)
     res, finfo, pinfo = _forecast(kalman, y, mats, int(horizon), int(n_simulations), z_init, z_state, z_obs, generator)
-    for info in (finfo, pinfo):
-        bad = torch.nonzero(info != 0) if info is not None else None
-        if bad is not None and bad.numel():
-            u = int(bad[0, 0])
-            raise RuntimeError(f"forecast: unit {u} failed with info {int(info[u])} (codes in include/kfb200.h)")
+    _raise_on_failure("forecast", (finfo, pinfo))
     return res
 
 
@@ -269,19 +265,9 @@ def _conditional_forecast(kalman: BatchedKalman, y, mats, conditions, n_simulati
     start_mean, start_cov = out["predicted_states"][:, n].contiguous(), out["predicted_covs"][:, n].contiguous()
     S = U * n_simulations
     if S > 0:
-        z_init = torch.randn((S, m), generator=generator, **f64) if z_init is None else z_init
-        z_state = torch.randn((H - 1, S, r), generator=generator, **f64) if z_state is None else z_state
-        z_obs = torch.randn((H, S, p), generator=generator, **f64) if z_obs is None else z_obs
-        for name, t, shape in (("z_init", z_init, (S, m)), ("z_state", z_state, (H - 1, S, r)),
-                               ("z_obs", z_obs, (H, S, p))):
-            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and tuple(t.shape) == shape):
-                raise ValueError(f"{name}: expected a float64 CUDA tensor of shape {shape} (time-major normals)")
-        z_init, z_state, z_obs = z_init.contiguous(), z_state.contiguous(), z_obs.contiguous()
+        z_init, z_state, z_obs = _normals(S, H, m, p, r, z_init, z_state, z_obs, generator, dev)
     desc = kalman._desc
-    nbytes = ctypes.c_size_t(0)
-    check(lib.kfb_conditional_forecast_workspace_bytes(ctypes.byref(desc), H, n_simulations, ctypes.byref(nbytes)),
-          "kfb_conditional_forecast_workspace_bytes")
-    ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=dev)
+    ws = _workspace(lib, "kfb_conditional_forecast", desc, dev, H, n_simulations)
     res = {"state_mean": torch.empty((U, H, m), **f64), "state_cov": torch.empty((U, H, m, m), **f64),
            "obs_mean": torch.empty((U, H, p), **f64), "obs_cov": torch.empty((U, H, p, p), **f64)}
     states = torch.empty((H, S, m), **f64) if S > 0 else None
@@ -322,12 +308,7 @@ def conditional_forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, conditions=No
                            device=T.device)
     res, finfo, winfo = _conditional_forecast(kalman, y, mats, conditions, int(n_simulations), z_init, z_state, z_obs,
                                               generator)
-    for info in (finfo, winfo):
-        bad = torch.nonzero(info != 0)
-        if bad.numel():
-            u = int(bad[0, 0])
-            raise RuntimeError(f"conditional_forecast: unit {u} failed with info {int(info[u])} "
-                               "(codes in include/kfb200.h)")
+    _raise_on_failure("conditional_forecast", (finfo, winfo))
     return res
 
 
@@ -366,8 +347,5 @@ def impulse_responses(T, Z, R, Q, horizon: int, shock: str = "cholesky"):
     leading draw axis B (B = 1 if all are shared).  Returns (states [B, H, m, r], obs [B, H, p, r]).  Raises
     RuntimeError if Q is not positive semi-definite for some draw under "std" / "cholesky"."""
     states, obs, info = _impulse_responses(T, Z, R, Q, horizon, shock)
-    bad = torch.nonzero(info != 0)
-    if bad.numel():
-        b = int(bad[0, 0])
-        raise RuntimeError(f"impulse_responses: draw {b} failed with info {int(info[b])} (Q not positive semi-definite)")
+    _raise_on_failure("impulse_responses", (info,), "draw", "Q not positive semi-definite")
     return states, obs

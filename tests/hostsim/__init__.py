@@ -3,10 +3,13 @@ oracle without a GPU.  One library is built from the .cpp files here:
 
 * hostsim.cpp - the sequential filters and adjoints (kf_core.cuh, kf_pred.cuh, kf_p1.cuh), the DARE and the RTS smoother;
 * tpar.cpp - the time-parallel filter, adjoint and smoother (kf_tpar.cuh, kf_tpar_smooth.cuh) with emulated CTA scans;
-* simsmooth.cpp - the simulation smoother (kf_simsmooth.cuh).
+* draws.cpp - the simulation smoother, forecast paths, impulse responses and conditional forecasts (kf_simsmooth.cuh,
+  kf_forecast.cuh, kf_condfc.cuh); its Python entry points are in ``tests.hostsim.draws``.
 
 The filter entry points take the C ABI's filter kind and KFB_FLAG_* bits and apply the library's own rules to them
-(kf_run.cuh).  Not part of the product; never imported by ``pymc_statespace_b200``.
+(kf_run.cuh); the entry points of draws.cpp take the C ABI's own arguments and build the kernels' arguments and
+workspace with the library's builders (kf_draws_run.cuh).  Not part of the product; never imported by
+``pymc_statespace_b200``.
 """
 from __future__ import annotations
 
@@ -213,43 +216,7 @@ def dare(T, Z, H, C, gPss, gGss):
 
 def simsmooth_is_static(m, p, r):
     """True if (m, p, r) has a compile-time instantiation of the simulation smoother."""
-    return bool(build().simsmooth_host_is_static(m, p, r))
-
-
-def simsmooth(y, mats, pc, spu, z_init, z_state, z_obs, n_draws=1, n_series=1, force_dyn=False):
-    """The simulation smoother (simsmooth.cpp) with the arguments and layouts of kfb_simulation_smoother for
-    n_draws x n_series units.  y [n, p] or [n_series, n, p]; mats: dict of a0 P0 T Z R H Q c d, each shared (base shape)
-    or [n_draws, ...]; pc [U, n+1, m, m].  Returns (states [S, n, m], info [U])."""
-    lib = build()
-    y = f8(y)
-    T = f8(mats["T"])
-    m = T.shape[-1]
-    p = f8(mats["Z"]).shape[-2]
-    r = f8(mats["R"]).shape[-1]
-    n = y.shape[-2]
-    base = {"a0": (m,), "P0": (m, m), "T": (m, m), "Z": (p, m), "R": (m, r), "H": (p, p), "Q": (r, r), "c": (m,),
-            "d": (p,)}
-    args = []
-    for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d"):
-        v = f8(mats.get(k))
-        size = int(np.prod(base[k]))
-        if v is None:
-            args += [None, 0]
-            continue
-        bs = size if v.size == n_draws * size and n_draws > 1 else 0
-        args += [_p(v), bs]
-        mats[k] = v  # keep alive
-    U = n_draws * n_series
-    states = np.zeros((U * spu, n, m))
-    info = np.zeros(U, dtype=np.int32)
-    pc, z_init, z_state, z_obs = f8(pc), f8(z_init), f8(z_state), f8(z_obs)
-    rc = lib.simsmooth_host_run(
-        ctypes.c_longlong(n_draws), ctypes.c_longlong(n_series), ctypes.c_longlong(spu), n, m, p, r, _p(y),
-        ctypes.c_longlong(n * p if y.ndim == 3 else 0), *[a if i % 2 == 0 else ctypes.c_longlong(a) for i, a in enumerate(args)],
-        _p(pc), _p(z_init), _p(z_state), _p(z_obs), _p(states), _p(info), int(force_dyn))
-    if rc != 0:
-        raise RuntimeError(f"simsmooth_host_run rc={rc}")
-    return states, info
+    return bool(build().draws_host_is_static(m, p, r))
 
 
 def chain_to_inputs(kind, g, T, Z, R, H, Q, C, Pss, Gss):

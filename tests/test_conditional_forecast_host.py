@@ -1,5 +1,5 @@
 """CPU checks of the conditional forecasts: the numpy restatement (oracle/condforecast.py) and the host build of the
-kernels' KFB_HD code (tests/hostsim/condfc.cpp) pin themselves against dense joint-Gaussian algebra through the affine
+kernels' KFB_HD code (tests/hostsim/draws.cpp) pin themselves against dense joint-Gaussian algebra through the affine
 map from normals to paths, the host build equals the restatement on every instantiation, and the C ABI validates its
 arguments without a device."""
 import ctypes
@@ -66,7 +66,7 @@ def joint(states, obs):
 
 
 def _host(case, spu, zi, zs, zo, force_dyn=False):
-    from tests.hostsim import condfc as hcf
+    from tests.hostsim import draws as hcf
 
     _, y, a0, P0, T, Z, R, H, Q, c, d, cond = case
     a, P = _start(y, a0, P0, T, Z, R, H, Q, c, d)
@@ -137,7 +137,7 @@ def test_moments_match_dense_law(case):
 @pytest.mark.parametrize("force_dyn", [False, True], ids=["instantiation", "runtime_dims"])
 def test_all_nan_conditions_reproduce_forecast(force_dyn):
     """No condition: the moments are forecast's (to rounding) and the paths are the forecast paths bit for bit."""
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     name, y, a0, P0, T, Z, R, H, Q, c, d, _ = CASES[3]
     m, p, r, hor, spu = T.shape[0], Z.shape[0], R.shape[1], 6, 37
@@ -186,7 +186,7 @@ def _random_cond(rng, U, hor, p, per_unit):
 @pytest.mark.parametrize("geom", GEOMS, ids=[f"m{m}_p{p}_r{r}" for (m, p, r) in GEOMS])
 def test_host_build_equals_oracle(geom, force_dyn):
     from tests import hostsim
-    from tests.hostsim import condfc as hcf
+    from tests.hostsim import draws as hcf
 
     m, p, r = geom
     rng = np.random.default_rng(300 + 100 * m + 10 * p + r)
@@ -222,7 +222,7 @@ def test_host_build_equals_oracle(geom, force_dyn):
 @pytest.mark.parametrize("force_dyn", [False, True], ids=["instantiation", "runtime_dims"])
 def test_host_build_info_codes(force_dyn):
     from pymc_statespace_b200._lib import KFB_INFO_NOT_PSD
-    from tests.hostsim import condfc as hcf
+    from tests.hostsim import draws as hcf
 
     rng = np.random.default_rng(8)
     nD, NS, spu, hor, m, p, r, n = 4, 2, 3, 5, 2, 2, 2, 50

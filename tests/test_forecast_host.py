@@ -1,6 +1,6 @@
 """CPU checks of the forecasts from the end of the sample and the impulse responses: the numpy restatement
 (oracle/forecast.py) pins itself against dense joint-Gaussian algebra through the affine map from normals to paths, the
-host build of the kernels' KFB_HD code (tests/hostsim/forecast.cpp) equals the restatement, and the C ABI validates its
+host build of the kernels' KFB_HD code (tests/hostsim/draws.cpp) equals the restatement, and the C ABI validates its
 arguments without a device."""
 import ctypes
 
@@ -154,7 +154,7 @@ def _starts(rng, U, m):
 @pytest.mark.parametrize("geom", GEOMS, ids=[f"m{m}_p{p}_r{r}" for (m, p, r) in GEOMS])
 def test_host_build_equals_oracle(geom, force_dyn):
     from tests import hostsim
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     m, p, r = geom
     rng = np.random.default_rng(100 * m + 10 * p + r)
@@ -177,7 +177,7 @@ def test_host_build_equals_oracle(geom, force_dyn):
 
 
 def test_host_build_horizon1_shared_matrices():
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     rng = np.random.default_rng(6)
     _, _, _, T, Z, R, H, Q = random_system(rng, 2, 1, 2, 2)
@@ -194,7 +194,7 @@ def test_host_build_horizon1_shared_matrices():
 @pytest.mark.parametrize("force_dyn", [False, True], ids=["instantiation", "runtime_dims"])
 def test_host_build_info_codes(force_dyn):
     from pymc_statespace_b200._lib import KFB_INFO_NOT_PSD
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     rng = np.random.default_rng(8)
     nD, NS, spu, hor, m, p, r = 3, 2, 4, 5, 2, 2, 2
@@ -218,7 +218,7 @@ def test_host_build_info_codes(force_dyn):
 def test_host_build_impulse_responses_equal_oracle(geom, force_dyn):
     from pymc_statespace_b200._lib import SHOCK_KIND
     from tests import hostsim
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     m, p, r = geom
     rng = np.random.default_rng(7 + m + p + r)
@@ -235,7 +235,7 @@ def test_host_build_impulse_responses_equal_oracle(geom, force_dyn):
 
 def test_host_build_impulse_responses_closed_forms_and_info():
     from pymc_statespace_b200._lib import KFB_INFO_NOT_PSD, SHOCK_KIND
-    from tests.hostsim import forecast as hfc
+    from tests.hostsim import draws as hfc
 
     phi, theta, hor = -0.6, 0.25, 15
     _, _, _, T, Z, R, _, Q = arma11(phi, theta)

@@ -159,7 +159,7 @@ def test_oracle_factor_rule():
 @pytest.mark.parametrize("force_dyn", [False, True], ids=["instantiation", "runtime_dims"])
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 def test_host_build_equals_oracle(case, force_dyn):
-    from tests import hostsim
+    from tests.hostsim.draws import simsmooth
 
     name, y, a0, P0, T, Z, R, H, Q, c, d, _ = case
     n, p, m, r = y.shape[0], Z.shape[0], T.shape[0], R.shape[1]
@@ -169,13 +169,13 @@ def test_host_build_equals_oracle(case, force_dyn):
     pc = oss.predicted_covs(y, P0, T, Z, R, H, Q)
     want, info = oss.simulation_smoother(y, a0, P0, T, Z, R, H, Q, c, d, zi, zs, zo, P=pc)
     assert info == 0
-    got, hinfo = hostsim.simsmooth(y[..., 0], mats_of(case), pc[None], S, zi, zs.reshape(-1), zo, force_dyn=force_dyn)
+    got, hinfo = simsmooth(y[..., 0], mats_of(case), pc[None], S, zi, zs.reshape(-1), zo, force_dyn=force_dyn)
     assert (hinfo == 0).all()
     assert np.abs(got - want).max() <= 1e-13 * (np.abs(want).max() + 1.0), name
 
 
 def test_host_build_nile():
-    from tests import hostsim
+    from tests.hostsim.draws import simsmooth
 
     y, a0, P0, T, Z, R, H, Q = nile_inputs(n_missing=5)
     rng = np.random.default_rng(2)
@@ -183,14 +183,14 @@ def test_host_build_nile():
     zi, zs, zo = random_normals(rng, S, n, 2, 1, 2)
     pc = oss.predicted_covs(y, P0, T, Z, R, H, Q)
     want, _ = oss.simulation_smoother(y, a0, P0, T, Z, R, H, Q, None, None, zi, zs, zo, P=pc)
-    got, info = hostsim.simsmooth(y[..., 0], dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q), pc[None], S, zi, zs, zo)
+    got, info = simsmooth(y[..., 0], dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q), pc[None], S, zi, zs, zo)
     assert (info == 0).all()
     # P0 = 1e6 I: xhat_0 = P0 r_{-1} scales the rounding of r_{-1} (different F^-1 and summation orders) by 1e6
     assert np.abs(got - want).max() <= 1e-8 * np.abs(want).max()
 
 
 def test_host_build_info_codes():
-    from tests import hostsim
+    from tests.hostsim.draws import simsmooth
     from pymc_statespace_b200._lib import KFB_INFO_NOT_PSD
 
     rng = np.random.default_rng(5)
@@ -200,13 +200,13 @@ def test_host_build_info_codes():
     mats = dict(a0=a0, P0=P0, T=T, Z=Z, R=R, H=H, Q=Q)
     yp = y.copy()
     yp[3, 1] = np.nan  # partly missing row 3
-    got, info = hostsim.simsmooth(yp[..., 0], dict(mats), pc[None], 2, zi, zs, zo)
+    got, info = simsmooth(yp[..., 0], dict(mats), pc[None], 2, zi, zs, zo)
     assert info[0] == -4 and np.isnan(got).all()
-    got, info = hostsim.simsmooth(y[..., 0], dict(mats, Q=-Q), pc[None], 2, zi, zs, zo)
+    got, info = simsmooth(y[..., 0], dict(mats, Q=-Q), pc[None], 2, zi, zs, zo)
     assert info[0] == KFB_INFO_NOT_PSD and np.isnan(got).all()
     pc_bad = pc.copy()
     pc_bad[2] = -10 * np.eye(2)  # F_2 = Z P_2 Z^T + H not PD
-    got, info = hostsim.simsmooth(y[..., 0], dict(mats), pc_bad[None], 2, zi, zs, zo)
+    got, info = simsmooth(y[..., 0], dict(mats), pc_bad[None], 2, zi, zs, zo)
     assert info[0] == 3 and np.isnan(got).all()
 
 
