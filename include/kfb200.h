@@ -98,6 +98,11 @@ enum {
  * with the sequential recursion; no info code marks it.  The forward pass always uses the tape part of the workspace. */
 #define KFB_FLAG_TIME_PARALLEL 128u
 
+/* Read by kfb_simulation_smoother only: a partly observed row y_t (some entries NaN, not all) is filtered on its
+ * observed entries instead of failing the unit with -(t+1); predicted_covs must then come from kfb_masked_filter.
+ * Without a partly observed row the result is the same, bit for bit, as without the flag. */
+#define KFB_FLAG_PARTIAL_ROWS 256u
+
 typedef struct kfb_desc {
   int32_t filter_kind;
   uint32_t flags;
@@ -244,15 +249,17 @@ kfb_status kfb_mvn_draws(int64_t n_units, int64_t sims_per_unit, int32_t n, int3
  *   2. y* = y - y+; a*_0 = 0, v_t = y*_t - Z a*_t, a*_{t+1} = T a*_t + K_t v_t, K_t = T P_t Z^T F_t^-1;
  *   3. r_{n-1} = 0, r_{t-1} = Z^T F_t^-1 v_t + L_t^T r_t, L_t = T - K_t Z;
  *   4. xhat_0 = P0 r_{-1}, xhat_{t+1} = T xhat_t + R Q R^T r_t;   5. states[s, t] = x+_t + xhat_t.
- * A missing row (all of y_t NaN) has F_t^-1 = 0, K_t = 0.
+ * A missing row (all of y_t NaN) has F_t^-1 = 0, K_t = 0.  With KFB_FLAG_PARTIAL_ROWS in desc->flags a partly observed
+ * row (observed set o) has kfb_masked_filter's F_t^-1 and K_t (zero rows / columns for the missing entries) and
+ * v_t = 0 on its missing entries; predicted_covs then come from kfb_masked_filter.
  * Inputs: desc gives sizes and batch strides; every time stride must be 0 (else KFB_ERR_UNSUPPORTED); filter_kind and
- * flags are ignored.  k_states, k_endog, k_posdef <= 32 (else KFB_ERR_UNSUPPORTED).  predicted_covs[U, n+1, m, m] is
+ * every other flag are ignored.  k_states, k_endog, k_posdef <= 32 (else KFB_ERR_UNSUPPORTED).  predicted_covs[U, n+1, m, m] is
  * the output of a preceding kfb_forward (standard filter, KFB_FLAG_CORRECTED) on the same desc and inputs
  * (its row 0 is not read: P_0 is the input P0).  Simulation
  * s = unit * sims_per_unit + k (S = U * sims_per_unit).  Normals, time-major: z_init[S, m], z_state[n-1, S, r] (may be
  * NULL if n = 1), z_obs[n, S, p].  c, d may be NULL.  Output states[S, n, m]; info[U] (written, no zeroing needed):
- * 0 ok, t+1 F_t not positive definite, -(t+1) y_t partly missing, KFB_INFO_NOT_PSD; a failing unit's paths are NaN.
- * Workspace (kfb_simulation_smoother_workspace_bytes), each term rounded up to 256 bytes, with U = n_draws * n_series
+ * 0 ok, t+1 F_t not positive definite, -(t+1) y_t partly missing (never with KFB_FLAG_PARTIAL_ROWS), KFB_INFO_NOT_PSD;
+ * a failing unit's paths are NaN.  Workspace (kfb_simulation_smoother_workspace_bytes), each term rounded up to 256 bytes, with U = n_draws * n_series
  * and S32 = S rounded up to a multiple of 32:  8 U n (m p + p p)  +  8 U (2 m m + m r + p p + r r)  +  8 n S32 p
  *   +  8 (n - 1) S32 m  +  4 U. */
 kfb_status kfb_simulation_smoother_workspace_bytes(const kfb_desc *desc, int64_t sims_per_unit, size_t *bytes);
@@ -260,6 +267,25 @@ kfb_status kfb_simulation_smoother(const kfb_desc *desc, const kfb_inputs *in, c
                                    int64_t sims_per_unit, const double *z_init, const double *z_state,
                                    const double *z_obs, double *states, int32_t *info, void *workspace,
                                    size_t workspace_bytes, void *stream);
+
+/* The exact filter over data with partly observed rows (not on the logp/grad path): the predicted moments that
+ * kfb_forward (standard filter, KFB_FLAG_CORRECTED) gives, for a sample in which some rows y_t have NaN in some entries
+ * and not others (series released on different dates: the ragged edge of a multivariate sample, gaps inside it).
+ * kfb_forward refuses such a row (-(t+1)); this filter conditions on its observed entries.  At step t with observed
+ * set o, every product in the masked p x p form:
+ *   F = Z_o P Z_o^T + H_oo,  K = T P Z^T F^-1 (zero columns for the missing entries),  v = y - Z a - d on o, 0 elsewhere,
+ *   a <- T a + c + K v,  P <- T P L^T + R Q R^T (L = T - K Z), symmetrised.
+ * An all-missing row has K = 0; a complete row is the ordinary update; a non-diagonal H enters through H_oo.  Outputs
+ * predicted_states[U, n+1, m] and predicted_covs[U, n+1, m, m] (row 0: a0, P0) have kfb_forward's layout and meaning,
+ * so kfb_simulation_smoother (with KFB_FLAG_PARTIAL_ROWS), kfb_forecast_paths and kfb_conditional_forecast read them
+ * unchanged; either may be NULL, not both.  info[U] (written): 0, or t+1 if F_o is not positive definite at step t (that
+ * unit's outputs are NaN); never -(t+1).  desc as in kfb_simulation_smoother (n >= 1; filter_kind and flags ignored;
+ * every time stride 0, sizes <= 32, else KFB_ERR_UNSUPPORTED); y, a0, P0, T, Z, R, H, Q required, c, d may be NULL.
+ * Workspace (kfb_masked_filter_workspace_bytes), rounded up to 256 bytes:  8 U (5 m m + 2 m p + 3 p p). */
+kfb_status kfb_masked_filter_workspace_bytes(const kfb_desc *desc, size_t *bytes);
+kfb_status kfb_masked_filter(const kfb_desc *desc, const kfb_inputs *in, double *predicted_states,
+                             double *predicted_covs, int32_t *info, void *workspace, size_t workspace_bytes,
+                             void *stream);
 
 /* Forecast paths from the end of the sample (not on the logp/grad path): joint draws of x_n..x_{n+H-1} and
  * y_n..y_{n+H-1} given y_0..y_{n-1}, sims_per_unit of them per unit.  Same model as kfb_simulation_smoother.  The start

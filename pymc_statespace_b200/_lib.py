@@ -26,6 +26,7 @@ KFB_FLAG_H_ZERO = 16
 KFB_FLAG_T_COMPANION = 32
 KFB_FLAG_NO_MISSING = 64
 KFB_FLAG_TIME_PARALLEL = 128
+KFB_FLAG_PARTIAL_ROWS = 256
 KFB_INFO_DARE_FAILED = 0x40000001
 KFB_INFO_NOT_STATIONARY = 0x40000002
 KFB_INFO_BAD_STRUCTURE = 0x40000003
@@ -106,6 +107,9 @@ EXPORTS = {
     "kfb_conditional_forecast": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _vp, _c_i32, _vp, _c_i64,
                                           _c_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_size_t,
                                           _vp]),
+    "kfb_masked_filter_workspace_bytes": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(ctypes.c_size_t)]),
+    "kfb_masked_filter": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _vp, _vp, _vp, _vp, ctypes.c_size_t,
+                                   _vp]),
     "kfb_impulse_response": (_c_i32, [ctypes.POINTER(KfbDesc), ctypes.POINTER(KfbInputs), _c_i32, _c_i32, _vp, _vp, _vp,
                                       _vp]),
     "kfb_fp64_peak": (_c_i32, [_c_i32, _c_i32, _c_i32, _vp, ctypes.POINTER(ctypes.c_double), _vp]),

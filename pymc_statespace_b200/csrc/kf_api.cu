@@ -24,6 +24,7 @@ cudaError_t launch_simulation_smoother(const ss::Args& A, cudaStream_t s);
 cudaError_t launch_forecast_paths(const fc::Args& A, cudaStream_t s);
 cudaError_t launch_impulse_response(const fc::IrfArgs& A, cudaStream_t s);
 cudaError_t launch_conditional_forecast(const cf::Args& A, cudaStream_t s);
+cudaError_t launch_masked_filter(const cf::FilterArgs& A, cudaStream_t s);
 
 // k_states with launchers of their own, one object per size (kf_thread.cu: thread-per-unit filters and smoother;
 // kf_coopT.cu: compile-time-dims kernels; the tensor-core DARE in kf_coopT.cu from k_states 10).  The Makefile repeats
@@ -532,6 +533,29 @@ kfb_status kfb_conditional_forecast(const kfb_desc* desc, const kfb_inputs* in, 
                                     z_state, z_obs, state_mean, state_cov, obs_mean, obs_cov, states, obs, info,
                                     workspace, pl);
   return launch_status(launch_conditional_forecast(A, (cudaStream_t)stream));
+}
+
+kfb_status kfb_masked_filter_workspace_bytes(const kfb_desc* desc, size_t* bytes) {
+  if (!bytes) return KFB_ERR_INVALID_ARG;
+  draws::MfPlan pl;
+  kfb_status st = draws::plan_mf(desc, &pl);
+  if (st != KFB_OK) return st;
+  *bytes = pl.total;
+  return KFB_OK;
+}
+
+kfb_status kfb_masked_filter(const kfb_desc* desc, const kfb_inputs* in, double* predicted_states,
+                             double* predicted_covs, int32_t* info, void* workspace, size_t workspace_bytes,
+                             void* stream) {
+  draws::MfPlan pl;
+  kfb_status st = draws::plan_mf(desc, &pl);
+  if (st != KFB_OK) return st;
+  if (!in || !in->y || !in->a0 || !in->P0 || !in->T || !in->Z || !in->R || !in->H || !in->Q ||
+      (!predicted_states && !predicted_covs) || !info)
+    return KFB_ERR_INVALID_ARG;
+  if (!workspace || workspace_bytes < pl.total) return KFB_ERR_WORKSPACE;
+  const cf::FilterArgs A = draws::mf_args(desc, in, predicted_states, predicted_covs, info, workspace, pl);
+  return launch_status(launch_masked_filter(A, (cudaStream_t)stream));
 }
 
 kfb_status kfb_impulse_response(const kfb_desc* desc, const kfb_inputs* in, int32_t horizon, int32_t shock,

@@ -22,7 +22,7 @@
 //    K, Fi, G and u of every (unit, h) go to the tape.
 // 2. Paths, one thread per simulation (path_unit): the mean correction of kf_simsmooth.cuh's simulate_one over the
 //    window.  x+ starts at a + S_P z_init and follows the model (xplus_first / xplus_next), eps+_h = S_H z_obs_h; the
-//    masked forward step (forward_obs_masked) filters cond - y+ with a* = 0, backward_step gives r, and x~ = x+ + x^ with
+//    masked forward step (ss::forward_obs_masked) filters cond - y+ with a* = 0, backward_step gives r, and x~ = x+ + x^ with
 //    x^_0 = P r_{-1}, x^_{h+1} = T x^_h + C r_h.  Observations: y_o = cond_o exactly and
 //      y_u = Z_u x~ + d_u + eps+_u + G (cond_o - Z_o x~ - d_o - eps+_o):
 //    given x_{n+h} and the conditioned entries of row h the free entries are independent of everything else, and
@@ -72,34 +72,6 @@ KFB_HD double* buf(double (&reg)[N], double* scr) {
   }
 }
 
-// Step 2 at a partly conditioned row: forward_obs (kf_simsmooth.cuh) with v = 0 on the free (NaN) entries of y.
-template <class D>
-KFB_HD void forward_obs_masked(const D& d, double* a, double* uo, const double* x, const double* y, const double* zo,
-                               const double* T, const double* Z, const double* dd, const double* SH, const double* K,
-                               const double* Fi) {
-  double v[D::PM], an[D::MM];
-  for (int i = 0; i < d.p; ++i) {
-    double yp = dd[i];
-    for (int k = 0; k < d.m; ++k) yp = kf_fma(Z[i * d.m + k], x[k], yp);
-    for (int k = 0; k <= i; ++k) yp = kf_fma(SH[i * d.p + k], zo[k], yp);
-    double za = 0.0;
-    for (int k = 0; k < d.m; ++k) za = kf_fma(Z[i * d.m + k], a[k], za);
-    v[i] = kf_isnan(y[i]) ? 0.0 : (y[i] - yp) - za;
-  }
-  for (int i = 0; i < d.p; ++i) {
-    double s = 0.0;
-    for (int k = 0; k < d.p; ++k) s = kf_fma(Fi[i * d.p + k], v[k], s);
-    uo[i] = s;
-  }
-  for (int i = 0; i < d.m; ++i) {
-    double s = 0.0;
-    for (int k = 0; k < d.m; ++k) s = kf_fma(T[i * d.m + k], a[k], s);
-    for (int k = 0; k < d.p; ++k) s = kf_fma(K[i * d.p + k], v[k], s);
-    an[i] = s;
-  }
-  for (int i = 0; i < d.m; ++i) a[i] = an[i];
-}
-
 // Lm = T - K Z
 template <class D>
 KFB_HD void l_of(const D& d, double* Lm, const double* T, const double* K, const double* Z) {
@@ -109,6 +81,55 @@ KFB_HD void l_of(const D& d, double* Lm, const double* T, const double* K, const
       for (int k = 0; k < d.p; ++k) s = kf_fma(-K[i * d.p + k], Z[k * d.m + j], s);
       Lm[i * d.m + j] = s;
     }
+}
+
+// One step of the exact filter over a row with observed set o (bit i of om: y_i observed): ss::masked_gain's K and
+// Fi, v = y - Z a - d on o (0 elsewhere), then between(), then with Pn
+//   a <- T a + c + K v,  Pn = T P L^T + C  (L = T - K Z, C = R Q R^T), symmetrised.
+// A complete row is the ordinary update.  False if F_o is not positive definite (then nothing else is written).
+// PZt [m p], Lc, Li [p p], Lm, M1 [m m] are working matrices; between() may use Lc and Li.
+template <class D, class Between>
+KFB_HD bool masked_step(const D& d, unsigned om, const double* y, const double* T, const double* Z, const double* Hm,
+                        const double* C, const double* cz, const double* dz, const double* P, double* a, double* v,
+                        double* K, double* Fi, double* Pn, double* PZt, double* Lc, double* Li, double* Lm, double* M1,
+                        Between&& between) {
+  const int m = d.m, p = d.p;
+  if (!ss::masked_gain(d, om, P, T, Z, Hm, K, Fi, PZt, Lc, Li)) return false;
+  // v = y - Z a - d on the observed entries
+  for (int i = 0; i < p; ++i) {
+    double za = dz[i];
+    for (int k = 0; k < m; ++k) za = kf_fma(Z[i * m + k], a[k], za);
+    v[i] = ((om >> i) & 1u) ? y[i] - za : 0.0;
+  }
+  between();
+  if (!Pn) return true;
+  // a <- T a + c + K v;  Pn = T P L^T + C, symmetrised
+  {
+    double an[D::MM];
+    for (int i = 0; i < m; ++i) {
+      double s = cz[i];
+      for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], a[k], s);
+      for (int k = 0; k < p; ++k) s = kf_fma(K[i * p + k], v[k], s);
+      an[i] = s;
+    }
+    for (int i = 0; i < m; ++i) a[i] = an[i];
+  }
+  l_of(d, Lm, T, K, Z);
+  for (int i = 0; i < m; ++i)
+    for (int j = 0; j < m; ++j) {
+      double s = 0.0;
+      for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Lm[j * m + k], s);
+      M1[i * m + j] = s;
+    }
+  for (int i = 0; i < m; ++i)
+    for (int j = 0; j < m; ++j) {
+      double s = C[i * m + j];
+      for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], M1[k * m + j], s);
+      Lm[i * m + j] = s;  // Lm is free again: the new P before symmetrising
+    }
+  for (int i = 0; i < m; ++i)
+    for (int j = 0; j < m; ++j) Pn[i * m + j] = 0.5 * (Lm[i * m + j] + Lm[j * m + i]);
+  return true;
 }
 
 // Factors of one unit into fac[u] (the layout of ss::fac_stride, the factors computed as fc::unit_prep computes them);
@@ -181,123 +202,44 @@ KFB_HD int window_forward(const D& d, const Args& A, long long u) {
     for (int i = 0; i < p; ++i) om |= kf_isnan(y[i]) ? 0u : 1u << i;
     for (int i = 0; i < m; ++i) ta[i] = a[i];
     const double* P = ss::stage<D>(bP, tP, m * m);
-    for (int i = 0; i < m; ++i)
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Z[j * m + k], s);
-        PZt[i * p + j] = s;
-      }
-    // F = Z P Z^T + H on the conditioned entries, 1 on the diagonal of the free ones: its lower factor in Lc
-    bool ok = true;
-    for (int j = 0; j < p; ++j)
-      for (int i = j; i < p; ++i) {
-        double s = i == j ? 1.0 : 0.0;
-        if (((om >> i) & 1u) && ((om >> j) & 1u)) {
-          s = Hm[i * p + j];
-          for (int k = 0; k < m; ++k) s = kf_fma(Z[i * m + k], PZt[k * p + j], s);
-        }
-        for (int k = 0; k < j; ++k) s -= Lc[i * p + k] * Lc[j * p + k];
-        if (i == j) {
-          ok = ok && (s > 0.0);
-          Lc[j * p + j] = sqrt(s);
-        } else {
-          Lc[i * p + j] = s / Lc[j * p + j];
-        }
-      }
-    if (!ok) return A.n + h + 1;
-    // Li = Lc^-1 (lower); Fi = Li^T Li on the conditioned entries, 0 elsewhere
-    for (int j = 0; j < p; ++j)
+    // u_h = Fi v and G between the gain and the update
+    const auto u_and_g = [&]() {
+      // u = Fi v
       for (int i = 0; i < p; ++i) {
-        if (i < j) { Li[i * p + j] = 0.0; continue; }
-        double s = (i == j) ? 1.0 : 0.0;
-        for (int k = j; k < i; ++k) s -= Lc[i * p + k] * Li[k * p + j];
-        Li[i * p + j] = s / Lc[i * p + i];
-      }
-    for (int i = 0; i < p; ++i)
-      for (int j = 0; j < p; ++j) {
         double s = 0.0;
-        for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
-        Fi[i * p + j] = (((om >> i) & 1u) && ((om >> j) & 1u)) ? s : 0.0;
+        for (int k = 0; k < p; ++k) s = kf_fma(Fi[i * p + k], v[k], s);
+        uo[i] = s;
       }
-    // K = T (P Z^T) Fi
-    for (int i = 0; i < m; ++i) {
-      double tpz[D::PM];
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], PZt[k * p + j], s);
-        tpz[j] = s;
-      }
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < p; ++k) s = kf_fma(tpz[k], Fi[k * p + j], s);
-        K[i * p + j] = s;
-      }
-    }
-    // v = cond - Z a - d on the conditioned entries, u = Fi v
-    for (int i = 0; i < p; ++i) {
-      double za = dz[i];
-      for (int k = 0; k < m; ++k) za = kf_fma(Z[i * m + k], a[k], za);
-      v[i] = ((om >> i) & 1u) ? y[i] - za : 0.0;
-    }
-    for (int i = 0; i < p; ++i) {
-      double s = 0.0;
-      for (int k = 0; k < p; ++k) s = kf_fma(Fi[i * p + k], v[k], s);
-      uo[i] = s;
-    }
-    // G = H_uo H_oo^-: W = the inverse of psd_factor(H_oo) on its non-zero pivots (0 elsewhere), H_oo^- = W^T W
-    for (int i = 0; i < p; ++i)
-      for (int j = 0; j < p; ++j) Hg[i * p + j] = (((om >> i) & 1u) && ((om >> j) & 1u)) ? Hm[i * p + j] : 0.0;
-    ss::psd_factor(Hg, HL, p);  // a principal block of H, which unit_factors found PSD
-    for (int j = 0; j < p; ++j)
-      for (int i = 0; i < p; ++i) {
-        if (i < j || HL[i * p + i] == 0.0 || HL[j * p + j] == 0.0) { Li[i * p + j] = 0.0; continue; }
-        double s = (i == j) ? 1.0 : 0.0;
-        for (int k = j; k < i; ++k) s -= HL[i * p + k] * Li[k * p + j];
-        Li[i * p + j] = s / HL[i * p + i];
-      }
-    for (int i = 0; i < p; ++i)
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
-        Hg[i * p + j] = s;
-      }
-    for (int i = 0; i < p; ++i)
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        if (!((om >> i) & 1u) && ((om >> j) & 1u))
-          for (int k = 0; k < p; ++k)
-            if (((om >> k) & 1u)) s = kf_fma(Hm[i * p + k], Hg[k * p + j], s);
-        G[i * p + j] = s;
-      }
-    for (int i = 0; i < p; ++i) tu[i] = uo[i];
-    if (h + 1 == H) break;
-    // a <- T a + c + K v;  P <- T P L^T + C, symmetrised, into the next record
-    {
-      double an[D::MM];
-      for (int i = 0; i < m; ++i) {
-        double s = cz[i];
-        for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], a[k], s);
-        for (int k = 0; k < p; ++k) s = kf_fma(K[i * p + k], v[k], s);
-        an[i] = s;
-      }
-      for (int i = 0; i < m; ++i) a[i] = an[i];
-    }
-    l_of(d, Lm, T, K, Z);
-    for (int i = 0; i < m; ++i)
-      for (int j = 0; j < m; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Lm[j * m + k], s);
-        M1[i * m + j] = s;
-      }
-    for (int i = 0; i < m; ++i)
-      for (int j = 0; j < m; ++j) {
-        double s = C[i * m + j];
-        for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], M1[k * m + j], s);
-        Lm[i * m + j] = s;  // Lm is free again: the new P before symmetrising
-      }
-    double* Pn = tP + ts;
-    for (int i = 0; i < m; ++i)
-      for (int j = 0; j < m; ++j) Pn[i * m + j] = 0.5 * (Lm[i * m + j] + Lm[j * m + i]);
+      // G = H_uo H_oo^-: W = the inverse of psd_factor(H_oo) on its non-zero pivots (0 elsewhere), H_oo^- = W^T W
+      for (int i = 0; i < p; ++i)
+        for (int j = 0; j < p; ++j) Hg[i * p + j] = (((om >> i) & 1u) && ((om >> j) & 1u)) ? Hm[i * p + j] : 0.0;
+      ss::psd_factor(Hg, HL, p);  // a principal block of H, which unit_factors found PSD
+      for (int j = 0; j < p; ++j)
+        for (int i = 0; i < p; ++i) {
+          if (i < j || HL[i * p + i] == 0.0 || HL[j * p + j] == 0.0) { Li[i * p + j] = 0.0; continue; }
+          double s = (i == j) ? 1.0 : 0.0;
+          for (int k = j; k < i; ++k) s -= HL[i * p + k] * Li[k * p + j];
+          Li[i * p + j] = s / HL[i * p + i];
+        }
+      for (int i = 0; i < p; ++i)
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
+          Hg[i * p + j] = s;
+        }
+      for (int i = 0; i < p; ++i)
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          if (!((om >> i) & 1u) && ((om >> j) & 1u))
+            for (int k = 0; k < p; ++k)
+              if (((om >> k) & 1u)) s = kf_fma(Hm[i * p + k], Hg[k * p + j], s);
+          G[i * p + j] = s;
+        }
+      for (int i = 0; i < p; ++i) tu[i] = uo[i];
+    };
+    if (!masked_step(d, om, y, T, Z, Hm, C, cz, dz, P, a, v, K, Fi, h + 1 < H ? tP + ts : nullptr, PZt, Lc, Li, Lm, M1,
+                     u_and_g))
+      return A.n + h + 1;
   }
   return 0;
 }
@@ -518,7 +460,7 @@ KFB_HD void path_unit(const D& d, const Args& A, long long s) {
     const double* K = ss::stage<D>(bK, tape + h * ts, m * p);
     const double* Fi = ss::stage<D>(bFi, tape + h * ts + m * p, p * p);
     load_zo(zb, h);
-    forward_obs_masked(d, a, uo, x, cond + (long long)h * p, zb, T, Z, dz, SH, K, Fi);
+    ss::forward_obs_masked(d, a, uo, x, cond + (long long)h * p, zb, T, Z, dz, SH, K, Fi);
     double* us = A.uscr + ((long long)h * W + w) * p * 32 + lane;
     for (int k = 0; k < p; ++k) us[k * 32] = uo[k];
     if (h + 1 < H) {
@@ -586,6 +528,92 @@ KFB_HD void path_unit(const D& d, const Args& A, long long s) {
       ss::xhat_next(d, xh, T, C, r, false);
     }
   }
+}
+
+// The exact filter over a sample with partly observed rows (kfb_masked_filter): one thread per unit runs masked_step
+// over y_0..y_{n-1} from (a0, P0) and writes the predicted moments, rows 0..n, in kfb_forward's layout.
+struct FilterArgs {
+  long long U, n_series, S, spu;  // units (draw * n_series + series); S, spu are 0
+  int n, m, p, r;
+  MatArg y, a0, P0, T, Z, R, Hm, Q, c, d;  // batch strides only (static matrices); Hm is the observation covariance H
+  double *ps, *pc;                         // predicted_states [U][n + 1][m], predicted_covs [U][n + 1][m][m]; one may be null
+  int* info;                               // [U] 0, or t + 1 if F_o is not positive definite at step t
+  double* scr;                             // [U][filter_scr_stride]: C, then the working matrices of the run-time dims
+};
+
+// C (m m) | P (m m) | Pn (m m) | Lm (m m) | M1 (m m) | PZt (m p) | K (m p) | Lc (p p) | Li (p p) | Fi (p p)
+KFB_HD long long filter_scr_stride(int m, int p) { return 5LL * m * m + 2LL * m * p + 3LL * p * p; }
+
+template <class D>
+KFB_HD void filter_unit(const D& d, const FilterArgs& A, long long u) {
+  const int m = d.m, p = d.p, n = A.n;
+  const long long dr = u / A.n_series, se = u % A.n_series;
+  constexpr bool ST = D::STATIC;
+  constexpr int MM = ST ? D::MM : 1, PM = ST ? D::PM : 1;
+  double* scr = A.scr + u * filter_scr_stride(m, p);
+  double* C = scr;  // R Q R^T, summed as unit_factors sums it; read in place, as H is
+  {
+    const double* R = A.R.p + dr * A.R.bs;
+    const double* Q = A.Q.p + dr * A.Q.bs;
+    const int r = A.r;
+    for (int i = 0; i < m; ++i)
+      for (int j = 0; j < m; ++j) {
+        double s = 0.0;
+        for (int k = 0; k < r; ++k) {
+          double rq = 0.0;
+          for (int l = 0; l < r; ++l) rq = kf_fma(R[i * r + l], Q[l * r + k], rq);
+          s = kf_fma(rq, R[j * r + k], s);
+        }
+        C[i * m + j] = s;
+      }
+  }
+  double bT[MM * MM], bZ[PM * MM];
+  const double* T = ss::stage<D>(bT, A.T.p + dr * A.T.bs, m * m);
+  const double* Z = ss::stage<D>(bZ, A.Z.p + dr * A.Z.bs, p * m);
+  const double* Hm = A.Hm.p + dr * A.Hm.bs;
+  double rP[MM * MM], rPn[MM * MM], rLm[MM * MM], rM1[MM * MM], rPZ[MM * PM], rK[MM * PM], rLc[PM * PM], rLi[PM * PM],
+      rFi[PM * PM];
+  const long long mm = (long long)m * m, mp = (long long)m * p;
+  double* P = buf<D>(rP, scr + mm);
+  double* Pn = buf<D>(rPn, scr + 2 * mm);
+  double* Lm = buf<D>(rLm, scr + 3 * mm);
+  double* M1 = buf<D>(rM1, scr + 4 * mm);
+  double* PZt = buf<D>(rPZ, scr + 5 * mm);
+  double* K = buf<D>(rK, scr + 5 * mm + mp);
+  double* Lc = buf<D>(rLc, scr + 5 * mm + 2 * mp);
+  double* Li = buf<D>(rLi, scr + 5 * mm + 2 * mp + p * p);
+  double* Fi = buf<D>(rFi, scr + 5 * mm + 2 * mp + 2 * p * p);
+  double a[D::MM], cz[D::MM], dz[D::PM], v[D::PM];
+  for (int i = 0; i < m; ++i) a[i] = A.a0.p[dr * A.a0.bs + i];
+  for (int i = 0; i < m * m; ++i) P[i] = A.P0.p[dr * A.P0.bs + i];
+  for (int i = 0; i < m; ++i) cz[i] = A.c.p ? A.c.p[dr * A.c.bs + i] : 0.0;
+  for (int i = 0; i < p; ++i) dz[i] = A.d.p ? A.d.p[dr * A.d.bs + i] : 0.0;
+  double* ps = A.ps ? A.ps + u * (n + 1) * m : nullptr;
+  double* pc = A.pc ? A.pc + u * (n + 1) * mm : nullptr;
+  const double* y = A.y.p + se * A.y.bs;
+  int st = 0;
+  for (int t = 0; t <= n; ++t) {
+    if (ps)
+      for (int i = 0; i < m; ++i) ps[(long long)t * m + i] = a[i];
+    if (pc)
+      for (int i = 0; i < m * m; ++i) pc[t * mm + i] = P[i];
+    if (t == n) break;
+    const double* yt = y + (long long)t * p;
+    unsigned om = 0;  // bit i: y_t,i observed
+    for (int i = 0; i < p; ++i) om |= kf_isnan(yt[i]) ? 0u : 1u << i;
+    if (!masked_step(d, om, yt, T, Z, Hm, C, cz, dz, P, a, v, K, Fi, Pn, PZt, Lc, Li, Lm, M1, [] {})) {
+      st = t + 1;
+      break;
+    }
+    for (int i = 0; i < m * m; ++i) P[i] = Pn[i];
+  }
+  if (st != 0) {
+    for (long long i = 0; i < (n + 1LL) * m; ++i)
+      if (ps) ps[i] = NAN;
+    for (long long i = 0; i < (n + 1LL) * mm; ++i)
+      if (pc) pc[i] = NAN;
+  }
+  A.info[u] = st;
 }
 
 }  // namespace cf

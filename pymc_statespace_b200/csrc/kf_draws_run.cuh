@@ -1,5 +1,6 @@
 // kf_draws_run.cuh - the requests of the per-draw sampling calls (kfb_simulation_smoother, kfb_forecast_paths,
-// kfb_conditional_forecast, kfb_impulse_response): validation of the descriptor, the workspace plans and the kernel
+// kfb_conditional_forecast, kfb_impulse_response) and of the masked filter they start from on data with partly observed
+// rows (kfb_masked_filter): validation of the descriptor, the workspace plans and the kernel
 // arguments built from the C ABI's arguments.  Shared by the C ABI (kf_api.cu) and the host build of the kernels
 // (tests/hostsim/draws.cpp), so that the CPU tests run the library's own argument fill and workspace layout.
 #pragma once
@@ -14,6 +15,7 @@
 namespace kfb {
 namespace draws {
 
+static_assert(KFB_FLAG_PARTIAL_ROWS == 256u, "include/kfb200.h");
 static_assert(fc::SHOCK_UNIT == KFB_SHOCK_UNIT && fc::SHOCK_STD == KFB_SHOCK_STD &&
                   fc::SHOCK_CHOLESKY == KFB_SHOCK_CHOLESKY && ss::INFO_NOT_PSD == KFB_INFO_NOT_PSD,
               "kf_forecast.cuh / kf_simsmooth.cuh constants differ from include/kfb200.h");
@@ -94,7 +96,21 @@ inline kfb_status plan_cf(const kfb_desc* d, int32_t horizon, int64_t sims_per_u
   return KFB_OK;
 }
 
-// The fields ss::Args, fc::Args and cf::Args share: unit and simulation counts, dims and the seven static matrices.
+// kfb_masked_filter: per-unit C and working matrices.
+struct MfPlan : Regions {
+  size_t off_scr;
+};
+
+inline kfb_status plan_mf(const kfb_desc* d, MfPlan* pl) {
+  const kfb_status st = check_desc(d, d && d->n > 0);
+  if (st != KFB_OK) return st;
+  if (d->n >= (1 << 29)) return KFB_ERR_UNSUPPORTED;
+  const long long U = d->n_draws * d->n_series;
+  pl->off_scr = pl->take((size_t)U * cf::filter_scr_stride(d->m, d->p) * 8);
+  return KFB_OK;
+}
+
+// The fields ss::Args, fc::Args, cf::Args and cf::FilterArgs share: unit and simulation counts, dims and the seven static matrices.
 // obs_cov is the member that holds the observation covariance H (ss::Args::H, fc::Args::Hm, cf::Args::Hm).
 template <class Args>
 void fill_model(Args* A, MatArg Args::*obs_cov, const kfb_desc* d, const kfb_inputs* in, int64_t sims_per_unit) {
@@ -123,6 +139,7 @@ inline ss::Args ss_args(const kfb_desc* d, const kfb_inputs* in, const double* p
   A.pc = predicted_covs; A.z_init = z_init; A.z_state = z_state; A.z_obs = z_obs; A.states = states; A.info = info;
   A.gain = (double*)(ws + pl.off_gain); A.fac = (double*)(ws + pl.off_fac);
   A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r); A.ustat = (int*)(ws + pl.off_stat);
+  A.partial_rows = (d->flags & KFB_FLAG_PARTIAL_ROWS) != 0;
   return A;
 }
 
@@ -165,6 +182,17 @@ inline cf::Args cf_args(const kfb_desc* d, const kfb_inputs* in, const double* s
   }
   A.tape = (double*)(ws + pl.off_tape); A.fac = (double*)(ws + pl.off_fac); A.wscr = (double*)(ws + pl.off_wscr);
   A.ustat = (int*)(ws + pl.off_stat); A.uscr = (double*)(ws + pl.off_u); A.rscr = (double*)(ws + pl.off_r);
+  return A;
+}
+
+inline cf::FilterArgs mf_args(const kfb_desc* d, const kfb_inputs* in, double* predicted_states,
+                              double* predicted_covs, int32_t* info, void* workspace, const MfPlan& pl) {
+  cf::FilterArgs A;
+  fill_model(&A, &cf::FilterArgs::Hm, d, in, 0);
+  A.n = d->n;
+  A.y = {in->y, d->y_bs, 0}; A.a0 = {in->a0, d->a0_bs, 0}; A.P0 = {in->P0, d->P0_bs, 0};
+  A.ps = predicted_states; A.pc = predicted_covs; A.info = info;
+  A.scr = (double*)((char*)workspace + pl.off_scr);
   return A;
 }
 

@@ -12,7 +12,8 @@
 //   5. x~_t = x+_t + xhat_t.
 // S_A S_A^T = A is the PSD lower factor of psd_factor below.  K_t = T P_t Z^T F_t^-1 and F_t^-1 do not depend on y: the
 // gain pass computes them once per (unit, t) from the filter's predicted covariances.  A missing row has K_t = 0 and
-// u_t = 0 (L_t = T), as in the filter.  x+ is not stored: step 4 recomputes it from the normals with the same arithmetic.
+// u_t = 0 (L_t = T), as in the filter.  With Args::partial_rows a partly observed row has v_t = 0 on its missing entries
+// and K_t, F_t^-1 zero on their columns (predicted covariances of kfb_masked_filter); steps 3-4 need no change.  x+ is not stored: step 4 recomputes it from the normals with the same arithmetic.
 #pragma once
 #include "kf_core.cuh"
 
@@ -22,7 +23,8 @@ namespace ss {
 constexpr int SS_MAX = 32;            // k_states / k_endog / k_posdef limit of the run-time-dims path
 constexpr double PSD_RTOL = 1e-10;    // psd_factor: pivots within this fraction of the largest diagonal entry are zero
 constexpr int KEY_NONE = 0x7f7f7f7f;  // unit status before any failure (a byte-wise memset value)
-constexpr int KEY_FACTOR = -1;        // P0, Q or H not PSD; otherwise 2 t (F_t not PD) or 2 t + 1 (row t partly missing)
+constexpr int KEY_FACTOR = -1;        // P0, Q or H not PSD; otherwise 2 t (F_t not PD) or 2 t + 1 (row t partly missing
+                                      // without Args::partial_rows)
 constexpr int INFO_NOT_PSD = 0x40000004;  // = KFB_INFO_NOT_PSD (include/kfb200.h)
 
 // Compile-time k_states / k_endog (registers); k_posdef r <= M is a run-time value, and R S_Q is stored M x M with
@@ -54,6 +56,7 @@ struct Args {
   double* fac;                             // [U][S_P0 (m m) | R S_Q (m r) | S_H (p p) | C (m m) | S_Q (r r)]
   int* ustat;                              // [U] smallest failure key, KEY_NONE if none
   double *uscr, *rscr;                     // u_t [n][warp][p][32], r_t [n - 1][warp][m][32]
+  bool partial_rows;                       // KFB_FLAG_PARTIAL_ROWS: partly observed rows are filtered, not refused
 };
 
 KFB_HD long long gain_stride(int m, int p) { return (long long)m * p + (long long)p * p; }
@@ -138,10 +141,75 @@ KFB_HD void unit_prep(const Args& A, long long u) {
   if (!ok) key_min(A.ustat + u, KEY_FACTOR);
 }
 
-// Gain pass, one (unit, t): K_t = T P_t Z^T F_t^-1 and F_t^-1 with F_t = Z P_t Z^T + H, into gain[u][t]; zeros for a
-// missing row.  A partly missing row or an F_t that is not positive definite sets its key.
+// The gain of a row with observed set o (bit i of om: y_i observed) in the masked p x p form: F = Z_o P Z_o^T + H_oo
+// with 1 on the diagonal of the missing entries, Fi = F^-1 on o x o (0 elsewhere), K = T P Z^T Fi (zero columns for
+// the missing entries; K = 0 for an all-missing row).  False if F_o is not positive definite (then K and Fi are not
+// written).  PZt [m p], Lc, Li [p p] are working matrices.
 template <class D>
-KFB_HD void gain_entry(const D& d, const Args& A, long long u, int t) {
+KFB_HD bool masked_gain(const D& d, unsigned om, const double* P, const double* T, const double* Z, const double* Hm,
+                        double* K, double* Fi, double* PZt, double* Lc, double* Li) {
+  const int m = d.m, p = d.p;
+  for (int i = 0; i < m; ++i)
+    for (int j = 0; j < p; ++j) {
+      double s = 0.0;
+      for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Z[j * m + k], s);
+      PZt[i * p + j] = s;
+    }
+  // F = Z P Z^T + H on the observed entries, 1 on the diagonal of the missing ones: its lower factor in Lc
+  bool ok = true;
+  for (int j = 0; j < p; ++j)
+    for (int i = j; i < p; ++i) {
+      double s = i == j ? 1.0 : 0.0;
+      if (((om >> i) & 1u) && ((om >> j) & 1u)) {
+        s = Hm[i * p + j];
+        for (int k = 0; k < m; ++k) s = kf_fma(Z[i * m + k], PZt[k * p + j], s);
+      }
+      for (int k = 0; k < j; ++k) s -= Lc[i * p + k] * Lc[j * p + k];
+      if (i == j) {
+        ok = ok && (s > 0.0);
+        Lc[j * p + j] = sqrt(s);
+      } else {
+        Lc[i * p + j] = s / Lc[j * p + j];
+      }
+    }
+  if (!ok) return false;
+  // Li = Lc^-1 (lower); Fi = Li^T Li on the observed entries, 0 elsewhere
+  for (int j = 0; j < p; ++j)
+    for (int i = 0; i < p; ++i) {
+      if (i < j) { Li[i * p + j] = 0.0; continue; }
+      double s = (i == j) ? 1.0 : 0.0;
+      for (int k = j; k < i; ++k) s -= Lc[i * p + k] * Li[k * p + j];
+      Li[i * p + j] = s / Lc[i * p + i];
+    }
+  for (int i = 0; i < p; ++i)
+    for (int j = 0; j < p; ++j) {
+      double s = 0.0;
+      for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
+      Fi[i * p + j] = (((om >> i) & 1u) && ((om >> j) & 1u)) ? s : 0.0;
+    }
+  // K = T (P Z^T) Fi
+  for (int i = 0; i < m; ++i) {
+    double tpz[D::PM];
+    for (int j = 0; j < p; ++j) {
+      double s = 0.0;
+      for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], PZt[k * p + j], s);
+      tpz[j] = s;
+    }
+    for (int j = 0; j < p; ++j) {
+      double s = 0.0;
+      for (int k = 0; k < p; ++k) s = kf_fma(tpz[k], Fi[k * p + j], s);
+      K[i * p + j] = s;
+    }
+  }
+  return true;
+}
+
+// Gain pass, one (unit, t): K_t = T P_t Z^T F_t^-1 and F_t^-1 with F_t = Z P_t Z^T + H, into gain[u][t]; zeros for a
+// missing row.  An F_t that is not positive definite sets its key, and so does a partly observed row unless PARTIAL
+// (Args::partial_rows), which gives every row that is not all missing masked_gain's K_t and F_t^-1 (the same bits as
+// below on a complete row).  The kernels instantiate both; gain_entry below picks one from A.partial_rows.
+template <bool PARTIAL, class D>
+KFB_HD void gain_entry_for(const D& d, const Args& A, long long u, int t) {
   const int m = d.m, p = d.p;
   const long long dr = u / A.n_series, se = u % A.n_series;
   double* K = A.gain + (u * A.n + t) * gain_stride(m, p);
@@ -149,8 +217,8 @@ KFB_HD void gain_entry(const D& d, const Args& A, long long u, int t) {
   const double* y = A.y.p + se * A.y.bs + (long long)t * p;
   int nmiss = 0;
   for (int i = 0; i < p; ++i) nmiss += kf_isnan(y[i]) ? 1 : 0;
-  bool ok = nmiss == 0;
-  if (nmiss > 0 && nmiss < p) key_min(A.ustat + u, 2 * t + 1);
+  bool ok = PARTIAL ? nmiss < p : nmiss == 0;
+  if (!PARTIAL && nmiss > 0 && nmiss < p) key_min(A.ustat + u, 2 * t + 1);
   double PZt[D::MM * D::PM], L[D::PM * D::PM], Li[D::PM * D::PM];
   if (ok) {
     // P_0 is the input P0: kfb_forward writes predicted_covs[u, 0] only together with predicted_states
@@ -158,58 +226,76 @@ KFB_HD void gain_entry(const D& d, const Args& A, long long u, int t) {
     const double* Z = A.Z.p + dr * A.Z.bs;
     const double* H = A.H.p + dr * A.H.bs;
     const double* T = A.T.p + dr * A.T.bs;
-    for (int i = 0; i < m; ++i)
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Z[j * m + k], s);
-        PZt[i * p + j] = s;
+    if constexpr (PARTIAL) {
+      unsigned om = 0;  // bit i: y_t,i observed
+      for (int i = 0; i < p; ++i) om |= kf_isnan(y[i]) ? 0u : 1u << i;
+      if (!masked_gain(d, om, P, T, Z, H, K, Fi, PZt, L, Li)) {
+        key_min(A.ustat + u, 2 * t);
+        for (int i = 0; i < m * p + p * p; ++i) K[i] = 0.0;
       }
-    // F = Z P Z^T + H and its lower Cholesky factor in L
-    for (int j = 0; j < p; ++j) {
-      for (int i = j; i < p; ++i) {
-        double s = H[i * p + j];
-        for (int k = 0; k < m; ++k) s = kf_fma(Z[i * m + k], PZt[k * p + j], s);
-        for (int k = 0; k < j; ++k) s -= L[i * p + k] * L[j * p + k];
-        if (i == j) {
-          ok = ok && (s > 0.0);
-          L[j * p + j] = sqrt(s);
-        } else {
-          L[i * p + j] = s / L[j * p + j];
+    } else {
+      for (int i = 0; i < m; ++i)
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          for (int k = 0; k < m; ++k) s = kf_fma(P[i * m + k], Z[j * m + k], s);
+          PZt[i * p + j] = s;
+        }
+      // F = Z P Z^T + H and its lower Cholesky factor in L
+      for (int j = 0; j < p; ++j) {
+        for (int i = j; i < p; ++i) {
+          double s = H[i * p + j];
+          for (int k = 0; k < m; ++k) s = kf_fma(Z[i * m + k], PZt[k * p + j], s);
+          for (int k = 0; k < j; ++k) s -= L[i * p + k] * L[j * p + k];
+          if (i == j) {
+            ok = ok && (s > 0.0);
+            L[j * p + j] = sqrt(s);
+          } else {
+            L[i * p + j] = s / L[j * p + j];
+          }
         }
       }
-    }
-    if (!ok) key_min(A.ustat + u, 2 * t);
-    // Li = L^-1 (lower), F^-1 = Li^T Li
-    for (int j = 0; j < p; ++j)
-      for (int i = 0; i < p; ++i) {
-        if (i < j) { Li[i * p + j] = 0.0; continue; }
-        double s = (i == j) ? 1.0 : 0.0;
-        for (int k = j; k < i; ++k) s -= L[i * p + k] * Li[k * p + j];
-        Li[i * p + j] = s / L[i * p + i];
-      }
-    for (int i = 0; i < p; ++i)
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
-        Fi[i * p + j] = ok ? s : 0.0;
-      }
-    // K = T (P Z^T) F^-1
-    for (int i = 0; i < m; ++i) {
-      double tpz[D::PM];
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], PZt[k * p + j], s);
-        tpz[j] = s;
-      }
-      for (int j = 0; j < p; ++j) {
-        double s = 0.0;
-        for (int k = 0; k < p; ++k) s = kf_fma(tpz[k], Fi[k * p + j], s);
-        K[i * p + j] = s;
+      if (!ok) key_min(A.ustat + u, 2 * t);
+      // Li = L^-1 (lower), F^-1 = Li^T Li
+      for (int j = 0; j < p; ++j)
+        for (int i = 0; i < p; ++i) {
+          if (i < j) { Li[i * p + j] = 0.0; continue; }
+          double s = (i == j) ? 1.0 : 0.0;
+          for (int k = j; k < i; ++k) s -= L[i * p + k] * Li[k * p + j];
+          Li[i * p + j] = s / L[i * p + i];
+        }
+      for (int i = 0; i < p; ++i)
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          for (int k = (i > j ? i : j); k < p; ++k) s = kf_fma(Li[k * p + i], Li[k * p + j], s);
+          Fi[i * p + j] = ok ? s : 0.0;
+        }
+      // K = T (P Z^T) F^-1
+      for (int i = 0; i < m; ++i) {
+        double tpz[D::PM];
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          for (int k = 0; k < m; ++k) s = kf_fma(T[i * m + k], PZt[k * p + j], s);
+          tpz[j] = s;
+        }
+        for (int j = 0; j < p; ++j) {
+          double s = 0.0;
+          for (int k = 0; k < p; ++k) s = kf_fma(tpz[k], Fi[k * p + j], s);
+          K[i * p + j] = s;
+        }
       }
     }
   } else {
     for (int i = 0; i < m * p + p * p; ++i) K[i] = 0.0;
   }
+}
+
+// gain_entry_for with PARTIAL = A.partial_rows (the host build of the kernels runs the passes through this).
+template <class D>
+KFB_HD void gain_entry(const D& d, const Args& A, long long u, int t) {
+  if (A.partial_rows)
+    gain_entry_for<true>(d, A, u, t);
+  else
+    gain_entry_for<false>(d, A, u, t);
 }
 
 // x <- T x + c + G z  (G = R S_Q; the state innovation of step t)
@@ -248,6 +334,34 @@ KFB_HD void forward_obs(const D& d, double* a, double* uo, const double* x, cons
     double za = 0.0;
     for (int k = 0; k < d.m; ++k) za = kf_fma(Z[i * d.m + k], a[k], za);
     v[i] = (y[i] - yp) - za;
+  }
+  for (int i = 0; i < d.p; ++i) {
+    double s = 0.0;
+    for (int k = 0; k < d.p; ++k) s = kf_fma(Fi[i * d.p + k], v[k], s);
+    uo[i] = s;
+  }
+  for (int i = 0; i < d.m; ++i) {
+    double s = 0.0;
+    for (int k = 0; k < d.m; ++k) s = kf_fma(T[i * d.m + k], a[k], s);
+    for (int k = 0; k < d.p; ++k) s = kf_fma(K[i * d.p + k], v[k], s);
+    an[i] = s;
+  }
+  for (int i = 0; i < d.m; ++i) a[i] = an[i];
+}
+
+// Step 2 at a partly observed row: forward_obs with v = 0 on the missing (NaN) entries of y
+template <class D>
+KFB_HD void forward_obs_masked(const D& d, double* a, double* uo, const double* x, const double* y, const double* zo,
+                               const double* T, const double* Z, const double* dd, const double* SH, const double* K,
+                               const double* Fi) {
+  double v[D::PM], an[D::MM];
+  for (int i = 0; i < d.p; ++i) {
+    double yp = dd[i];
+    for (int k = 0; k < d.m; ++k) yp = kf_fma(Z[i * d.m + k], x[k], yp);
+    for (int k = 0; k <= i; ++k) yp = kf_fma(SH[i * d.p + k], zo[k], yp);
+    double za = 0.0;
+    for (int k = 0; k < d.m; ++k) za = kf_fma(Z[i * d.m + k], a[k], za);
+    v[i] = kf_isnan(y[i]) ? 0.0 : (y[i] - yp) - za;
   }
   for (int i = 0; i < d.p; ++i) {
     double s = 0.0;
@@ -320,9 +434,10 @@ KFB_HD const double* stage(double (&dst)[N], const double* src, int cnt) {
   }
 }
 
-// One simulation s (steps 1-5); writes states[s] and, for the first simulation of a unit, info[u].
-template <class D>
-KFB_HD void simulate_one(const D& d, const Args& A, long long s) {
+// One simulation s (steps 1-5); writes states[s] and, for the first simulation of a unit, info[u].  PARTIAL
+// (Args::partial_rows): a partly observed row takes forward_obs_masked (without it the row's key failed the unit).
+template <bool PARTIAL, class D>
+KFB_HD void simulate_one_for(const D& d, const Args& A, long long s) {
   const int m = d.m, p = d.p, n = A.n;
   const long long u = s / A.spu, dr = u / A.n_series, se = u % A.n_series;
   const long long S = A.S, W = warps_of(S), w = s >> 5;
@@ -372,7 +487,12 @@ KFB_HD void simulate_one(const D& d, const Args& A, long long s) {
   for (int t = 0; t < n; ++t) {
     const double* yt = y + (long long)t * p;
     bool miss = false;
-    for (int i = 0; i < p; ++i) miss = miss || kf_isnan(yt[i]);
+    if constexpr (PARTIAL) {
+      miss = true;
+      for (int i = 0; i < p; ++i) miss = miss && kf_isnan(yt[i]);
+    } else {
+      for (int i = 0; i < p; ++i) miss = miss || kf_isnan(yt[i]);
+    }
     if (miss) {
       forward_missing(d, a, uo, T);
     } else {
@@ -381,7 +501,10 @@ KFB_HD void simulate_one(const D& d, const Args& A, long long s) {
       const double* zo = A.z_obs + ((long long)t * S + s) * p;
       double zb[D::PM];
       for (int k = 0; k < p; ++k) zb[k] = zo[k];
-      forward_obs(d, a, uo, x, yt, zb, T, Z, dz, SH, K, Fi);
+      if constexpr (PARTIAL)
+        forward_obs_masked(d, a, uo, x, yt, zb, T, Z, dz, SH, K, Fi);
+      else
+        forward_obs(d, a, uo, x, yt, zb, T, Z, dz, SH, K, Fi);
     }
     double* us = A.uscr + ((long long)t * W + w) * p * 32 + lane;
     for (int k = 0; k < p; ++k) us[k * 32] = uo[k];
@@ -425,6 +548,15 @@ KFB_HD void simulate_one(const D& d, const Args& A, long long s) {
       xhat_next(d, xh, T, C, r, false);
     }
   }
+}
+
+// simulate_one_for with PARTIAL = A.partial_rows (the host build of the kernels runs the passes through this).
+template <class D>
+KFB_HD void simulate_one(const D& d, const Args& A, long long s) {
+  if (A.partial_rows)
+    simulate_one_for<true>(d, A, s);
+  else
+    simulate_one_for<false>(d, A, s);
 }
 
 // The one list of instantiations, used by the launcher (kf_simsmooth.cu) and the host build: run(Static<M, P>{r}) for

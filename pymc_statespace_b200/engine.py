@@ -137,15 +137,8 @@ class BatchedKalman:
                 setattr(d, k + "_ts", ts)
         return d
 
-    # ------------------------------------------------------------------ forward
-    def forward(self, y, a0, P0, T, Z, R, H, Q, c=None, d=None, outputs=("loglik",), save_for_backward=False,
-                check_info=False, out: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
-        """``out``: optional caller-owned result buffers (name -> contiguous tensor of the documented shape, "info"
-        included); anything not given is allocated.  Lets a captured CUDA graph write straight into a staging buffer."""
-        self._via_inner = self._inner is not None and set(outputs) <= {"loglik"} and y.ndim <= 3 and y.shape[0] == self.n
-        if self._via_inner:
-            return self._inner.forward(y, *self._pad_inputs(a0, P0, T, Z, R, H, Q, c), d=d, outputs=outputs,
-                                       save_for_backward=save_for_backward, check_info=check_info, out=out)
+    def _request(self, y, a0, P0, T, Z, R, H, Q, c, d):
+        """(held tensors, KfbDesc) of one call on y and the matrices: shapes checked, batch and time strides set."""
         if y.ndim >= 2 and y.shape[-1] == 1 and y.shape[-2] == self.p and y.ndim in (3, 4) and y.shape[-3] == self.n:
             y = y[..., 0]  # reference layout data[n,p,1]
         if not (y.is_cuda and y.dtype == torch.float64):
@@ -164,7 +157,18 @@ class BatchedKalman:
         for name, t in zip(MATRIX_NAMES, (a0, P0, T, Z, R, H, Q, c, d)):
             tt, bs, ts = self._canon(name, t)
             held[name], strides[name] = tt, (bs, ts)
-        desc = self._make_desc(strides)
+        return held, self._make_desc(strides)
+
+    # ------------------------------------------------------------------ forward
+    def forward(self, y, a0, P0, T, Z, R, H, Q, c=None, d=None, outputs=("loglik",), save_for_backward=False,
+                check_info=False, out: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
+        """``out``: optional caller-owned result buffers (name -> contiguous tensor of the documented shape, "info"
+        included); anything not given is allocated.  Lets a captured CUDA graph write straight into a staging buffer."""
+        self._via_inner = self._inner is not None and set(outputs) <= {"loglik"} and y.ndim <= 3 and y.shape[0] == self.n
+        if self._via_inner:
+            return self._inner.forward(y, *self._pad_inputs(a0, P0, T, Z, R, H, Q, c), d=d, outputs=outputs,
+                                       save_for_backward=save_for_backward, check_info=check_info, out=out)
+        held, desc = self._request(y, a0, P0, T, Z, R, H, Q, c, d)
         nbytes = ctypes.c_size_t(0)
         check(self.lib.kfb_workspace_bytes(ctypes.byref(desc), int(save_for_backward), ctypes.byref(nbytes)),
               "kfb_workspace_bytes")
@@ -190,6 +194,30 @@ class BatchedKalman:
         self._desc, self._inputs, self._held, self._saved = desc, ins, held, bool(save_for_backward)
         if check_info:
             self.raise_on_info(out["info"])
+        return out
+
+    def masked_filter(self, y, a0, P0, T, Z, R, H, Q, c=None, d=None,
+                      outputs=("predicted_states", "predicted_covs")) -> Dict[str, torch.Tensor]:
+        """The exact filter over y with partly observed rows (kfb_masked_filter): the predicted moments ``forward``
+        gives with the corrected standard filter, where a row with some entries NaN is filtered on its observed entries
+        instead of failing with -(t+1).  Static matrices only.  ``outputs``: any of predicted_states [U, n+1, m] and
+        predicted_covs [U, n+1, m, m]; "info" [U] is 0 or t+1 (F_o not positive definite at step t, NaN outputs).
+        Afterwards ``_desc`` / ``_inputs`` describe this call, as after ``forward``."""
+        held, desc = self._request(y, a0, P0, T, Z, R, H, Q, c, d)
+        U, n, m = self.units, self.n, self.m
+        shapes = {"predicted_states": (U, n + 1, m), "predicted_covs": (U, n + 1, m, m)}
+        out = {k: torch.empty(shapes[k], dtype=torch.float64, device=self.device) for k in outputs}
+        out["info"] = torch.empty((U,), dtype=torch.int32, device=self.device)
+        ins = KfbInputs(*[_ptr(held[k]) for k in ("y",) + MATRIX_NAMES])
+        nbytes = ctypes.c_size_t(0)
+        check(self.lib.kfb_masked_filter_workspace_bytes(ctypes.byref(desc), ctypes.byref(nbytes)),
+              "kfb_masked_filter_workspace_bytes")
+        ws = torch.empty(max(nbytes.value, 256), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.kfb_masked_filter(ctypes.byref(desc), ctypes.byref(ins), _ptr(out.get("predicted_states")),
+                                             _ptr(out.get("predicted_covs")), _ptr(out["info"]), _ptr(ws), ws.numel(),
+                                             _stream_ptr(self.device)), "kfb_masked_filter")
+        self._desc, self._inputs, self._held, self._saved = desc, ins, held, False
         return out
 
     def _pad_inputs(self, a0, P0, T, Z, R, H, Q, c):

@@ -193,6 +193,10 @@ class KalmanLogp:
             raise ValueError('Cannot use filter_type = "single" with multiple observed time series')
         self.B = int(n_draws)
         self.y = torch.as_tensor(y, dtype=torch.float64, device=self.device).contiguous()
+        from .simulation import _has_partial_rows
+
+        # sample_states / forecast / conditional_forecast start from the masked filter if a row is partly observed
+        self._partial_rows = _has_partial_rows(self.y)
         # structure the model guarantees for every draw: constant (unmapped) design row [1, 0, ..] / zero observation variance
         z_unit0 = (p == 1 and not spec.maps.get("Z") and np.array_equal(
             np.asarray(spec.base["Z"], dtype=np.float64).ravel(), np.eye(spec.k_states)[0]))
@@ -362,13 +366,14 @@ class KalmanLogp:
         NaN and ``sample_states_info`` holds the per-draw status.
 
         Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
-        built with: the posterior of the states does not depend on the reference's as-coded likelihood quirks.  Normals
-        may be given as in ``simulation_smoother``, sized for the model's own k_states."""
+        built with: the posterior of the states does not depend on the reference's as-coded likelihood quirks.  If the
+        data have a partly observed row, that row is conditioned on its observed entries (the masked filter,
+        kfb_masked_filter).  Normals may be given as in ``simulation_smoother``, sized for the model's own k_states."""
         from .simulation import _simulation_smoother
 
         def run(kal, mats, z_init):
             states, info = _simulation_smoother(kal, self.y, mats, int(n_simulations), z_init, z_state, z_obs,
-                                                generator)
+                                                generator, self._partial_rows)
             return {"state_paths": states}, (info,)
 
         # the kernel writes NaN paths for its own failures
@@ -381,12 +386,13 @@ class KalmanLogp:
         stationary P0), as ``sample_states`` does.  Returns its dict (state_mean [B, H, k_states], state_cov, obs_mean,
         obs_cov and, with n_simulations > 0, state_paths [B * n_simulations, H, k_states] and obs_paths, draw-major)
         plus "info" [B] (int32): KFB_INFO_NOT_STATIONARY for a draw whose stationary P0 does not exist (it replaces the
-        forward's follow-on code, as in ``sample_states``), else the forward's code (t+1: F_t not positive definite;
-        -(t+1): y_t partly missing), else the paths' code (KFB_INFO_NOT_PSD: P_n, Q or H not positive semi-definite).
+        forward's follow-on code, as in ``sample_states``), else the forward's code (t+1: F_t not positive definite on
+        the observed entries), else the paths' code (KFB_INFO_NOT_PSD: P_n, Q or H not positive semi-definite).
         Every output of a failing draw is NaN.
 
         Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
-        built with.  Normals may be given as in ``simulation.forecast``, sized for the model's own k_states."""
+        built with; partly observed rows of the data are conditioned on their observed entries, as in
+        ``sample_states``.  Normals may be given as in ``simulation.forecast``, sized for the model's own k_states."""
         from .simulation import _forecast
 
         H = int(horizon)
@@ -394,7 +400,8 @@ class KalmanLogp:
             raise ValueError("horizon must be >= 1")
 
         def run(kal, mats, z_init):
-            res, info, pinfo = _forecast(kal, self.y, mats, H, int(n_simulations), z_init, z_state, z_obs, generator)
+            res, info, pinfo = _forecast(kal, self.y, mats, H, int(n_simulations), z_init, z_state, z_obs, generator,
+                                         self._partial_rows)
             return res, (info, pinfo)
 
         res, res_info = self._per_draw(theta, self.n + H, n_simulations, generator, z_init, run)
@@ -411,13 +418,14 @@ class KalmanLogp:
         at window step h; KFB_INFO_NOT_PSD).  Every output of a failing draw is NaN.
 
         Always the exact Kalman recursion (the corrected standard filter), whatever ``filter_type`` this evaluator was
-        built with.  Normals may be given as in ``simulation.conditional_forecast``, sized for the model's own
+        built with; partly observed rows of the data are conditioned on their observed entries, as in
+        ``sample_states``.  Normals may be given as in ``simulation.conditional_forecast``, sized for the model's own
         k_states."""
         from .simulation import _conditional_forecast
 
         def run(kal, mats, z_init):
             res, info, winfo = _conditional_forecast(kal, self.y, mats, conditions, int(n_simulations), z_init,
-                                                     z_state, z_obs, generator)
+                                                     z_state, z_obs, generator, self._partial_rows)
             return res, (info, winfo)
 
         res, res_info = self._per_draw(theta, self.n, n_simulations, generator, z_init, run)
@@ -441,8 +449,8 @@ class KalmanLogp:
 
     @property
     def sample_states_info(self) -> torch.Tensor:
-        """Per-draw status of the last ``sample_states`` (int32, 0 = ok; t+1: F_t not positive definite; -(t+1): y_t
-        partly missing; KFB_INFO_NOT_PSD: P0, Q or H not positive semi-definite; KFB_INFO_NOT_STATIONARY as in
+        """Per-draw status of the last ``sample_states`` (int32, 0 = ok; t+1: F_t not positive definite on the observed
+        entries; KFB_INFO_NOT_PSD: P0, Q or H not positive semi-definite; KFB_INFO_NOT_STATIONARY as in
         ``info``).  A failing draw's paths are NaN."""
         return self._ss_info
 

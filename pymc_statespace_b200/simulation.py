@@ -18,7 +18,7 @@ import ctypes
 
 import torch
 
-from ._lib import SHOCK_KIND, KfbInputs, check, load
+from ._lib import KFB_FLAG_PARTIAL_ROWS, SHOCK_KIND, KfbDesc, KfbInputs, check, load
 from .engine import BatchedKalman, _ptr, _stream_ptr
 
 
@@ -128,17 +128,34 @@ def _raise_on_failure(what, infos, unit="unit", codes="codes in include/kfb200.h
             raise RuntimeError(f"{what}: {unit} {u} failed with info {int(info[u])} ({codes})")
 
 
-def _simulation_smoother(kalman: BatchedKalman, y, mats, n_simulations, z_init, z_state, z_obs, generator):
-    """kfb_forward (predicted covariances) then kfb_simulation_smoother on ``kalman``'s geometry.  Returns
-    (states [U*S, n, m], info [U]) without raising on a non-zero info."""
+def _has_partial_rows(y) -> bool:
+    """True if some row of y [..., n, p] has NaN in some entries and not in all (a partly observed row)."""
+    nan = torch.isnan(y).sum(-1)
+    return bool(((nan > 0) & (nan < y.shape[-1])).any())
+
+
+def _predicted(kalman: BatchedKalman, y, mats, outputs, partial_rows):
+    """The predicted moments ``outputs`` of the exact filter over y: kfb_masked_filter if ``partial_rows`` (y has a
+    partly observed row), else the corrected standard filter.  Returns its outputs dict, "info" included."""
+    run = kalman.masked_filter if partial_rows else kalman.forward
+    return run(y, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")], outputs=outputs)
+
+
+def _simulation_smoother(kalman: BatchedKalman, y, mats, n_simulations, z_init, z_state, z_obs, generator,
+                         partial_rows=False):
+    """kfb_forward (predicted covariances; kfb_masked_filter with ``partial_rows``) then kfb_simulation_smoother on
+    ``kalman``'s geometry (with KFB_FLAG_PARTIAL_ROWS if ``partial_rows``).  Returns (states [U*S, n, m], info [U])
+    without raising on a non-zero info."""
     lib = load()
     dev = kalman.device
     n, m, p, r, U = kalman.n, kalman.m, kalman.p, kalman.r, kalman.units
     S = U * n_simulations
-    pc = kalman.forward(y, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
-                        outputs=("predicted_covs",))["predicted_covs"]
+    pc = _predicted(kalman, y, mats, ("predicted_covs",), partial_rows)["predicted_covs"]
     z_init, z_state, z_obs = _normals(S, n, m, p, r, z_init, z_state, z_obs, generator, dev)
     desc = kalman._desc
+    if partial_rows:
+        desc = KfbDesc.from_buffer_copy(desc)
+        desc.flags |= KFB_FLAG_PARTIAL_ROWS
     ws = _workspace(lib, "kfb_simulation_smoother", desc, dev, n_simulations)
     states = torch.empty((S, n, m), dtype=torch.float64, device=dev)
     info = torch.empty(U, dtype=torch.int32, device=dev)
@@ -156,24 +173,26 @@ def simulation_smoother(y, a0, P0, T, Z, R, H, Q, c=None, d=None, n_simulations:
 
     Float64 CUDA tensors; each matrix is shared (a0 [m], P0 [m, m], T [m, m], Z [p, m], R [m, r], H [p, p], Q [r, r],
     c [m], d [p]) or one per draw with a leading [B] axis, as in ``BatchedKalman``.  y is [n, p] or [n_series, n, p]
-    (NaN = missing; a row must be all observed or all missing).  Units are draw-major (u = draw * n_series + series) and
+    (NaN = missing; a partly observed row is conditioned on its observed entries).  Units are draw-major (u = draw * n_series + series) and
     so are the simulations (s = u * n_simulations + k).  Normals may be given, time-major: z_init [S, m], z_state
     [n-1, S, r], z_obs [n, S, p] for S = U * n_simulations; otherwise they are drawn with ``torch.randn``.
-    Returns states [S, n, m].  Raises RuntimeError if some unit fails (F_t not positive definite, a partly missing row,
+    Returns states [S, n, m].  Raises RuntimeError if some unit fails (F_t not positive definite on the observed entries,
     P0 / Q / H not positive semi-definite) and NotImplementedError for time-varying matrices."""
     mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
     n_series = 1 if y.ndim == 2 else y.shape[0]
     m, p, r = T.shape[-1], Z.shape[-2], R.shape[-1]
     kalman = BatchedKalman("standard", y.shape[-2], m, p, r, n_draws=B, n_series=n_series, strict_reference=False,
                            device=T.device)
-    states, info = _simulation_smoother(kalman, y, mats, int(n_simulations), z_init, z_state, z_obs, generator)
+    states, info = _simulation_smoother(kalman, y, mats, int(n_simulations), z_init, z_state, z_obs, generator,
+                                        _has_partial_rows(y))
     _raise_on_failure("simulation_smoother", (info,))
     return states
 
 
-def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_state, z_obs, generator):
+def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_state, z_obs, generator,
+              partial_rows=False):
     """Forecast moments (and paths if n_simulations > 0) on ``kalman``'s geometry: the standard corrected filter of
-    length n + horizon, run on y extended by ``horizon`` all-NaN rows.  Returns (result dict, forward info [U], paths
+    length n + horizon (kfb_masked_filter with ``partial_rows``), run on y extended by ``horizon`` all-NaN rows.  Returns (result dict, forward info [U], paths
     info [U] or None) without raising on a non-zero info."""
     lib = load()
     dev = kalman.device
@@ -181,8 +200,7 @@ def _forecast(kalman: BatchedKalman, y, mats, horizon, n_simulations, z_init, z_
     n = kalman.n - H
     f64 = dict(dtype=torch.float64, device=dev)
     yx = torch.cat([y, torch.full(y.shape[:-2] + (H, p), float("nan"), **f64)], dim=-2)
-    out = kalman.forward(yx, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
-                         outputs=("predicted_states", "predicted_covs"))
+    out = _predicted(kalman, yx, mats, ("predicted_states", "predicted_covs"), partial_rows)
     a, P = out["predicted_states"][:, n:n + H], out["predicted_covs"][:, n:n + H]
     ns = kalman.n_series
 
@@ -223,7 +241,8 @@ def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simul
     Arguments and conventions as in ``simulation_smoother``: float64 CUDA tensors, each matrix shared or one per draw,
     y [n, p] or [n_series, n, p], draw-major units (u = draw * n_series + series) and simulations
     (s = u * n_simulations + k).  The moments are the predicted moments of the exact (corrected standard) filter run
-    on y extended by H all-NaN rows.  Each path starts from x_n ~ N(a_n, P_n) and follows the model with its own state
+    on y extended by H all-NaN rows; a partly observed row of y is conditioned on its observed entries
+    (kfb_masked_filter).  Each path starts from x_n ~ N(a_n, P_n) and follows the model with its own state
     and observation noise (include/kfb200.h, kfb_forecast_paths), so the paths have the joint law of the future,
     cross-horizon covariances included.  Normals may be given, time-major: z_init [S, m], z_state [H-1, S, r],
     z_obs [H, S, p] for S = U * n_simulations; otherwise they are drawn with ``torch.randn``.
@@ -231,7 +250,7 @@ def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simul
     Returns a dict: state_mean [U, H, m], state_cov [U, H, m, m], obs_mean [U, H, p], obs_cov [U, H, p, p], and with
     n_simulations > 0 state_paths [S, H, m] and obs_paths [S, H, p].  The paths are ``permute(1, 0, 2)`` views of the
     kernel's time-major [H, S, .] buffers (no copy): call ``.contiguous()`` for path-major storage.  Raises
-    RuntimeError if some unit fails (F_t not positive definite, a partly missing row, P_n / Q / H not positive
+    RuntimeError if some unit fails (F_t not positive definite on the observed entries, P_n / Q / H not positive
     semi-definite) and NotImplementedError for time-varying matrices."""
     mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
     n_series = 1 if y.ndim == 2 else y.shape[0]
@@ -240,15 +259,16 @@ def forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, horizon: int = 1, n_simul
         raise ValueError("horizon must be >= 1")
     kalman = BatchedKalman("standard", y.shape[-2] + int(horizon), m, p, r, n_draws=B, n_series=n_series,
                            strict_reference=False, device=T.device)
-    res, finfo, pinfo = _forecast(kalman, y, mats, int(horizon), int(n_simulations), z_init, z_state, z_obs, generator)
+    res, finfo, pinfo = _forecast(kalman, y, mats, int(horizon), int(n_simulations), z_init, z_state, z_obs, generator,
+                                  _has_partial_rows(y))
     _raise_on_failure("forecast", (finfo, pinfo))
     return res
 
 
 def _conditional_forecast(kalman: BatchedKalman, y, mats, conditions, n_simulations, z_init, z_state, z_obs,
-                          generator):
-    """Conditional forecast on ``kalman``'s geometry (the standard corrected filter over the n observations): its
-    predicted moments at index n start kfb_conditional_forecast.  conditions [H, p] shared or [U, H, p].  Returns
+                          generator, partial_rows=False):
+    """Conditional forecast on ``kalman``'s geometry (the standard corrected filter over the n observations;
+    kfb_masked_filter with ``partial_rows``): its predicted moments at index n start kfb_conditional_forecast.  conditions [H, p] shared or [U, H, p].  Returns
     (result dict, forward info [U], window / paths info [U]) without raising on a non-zero info."""
     lib = load()
     dev = kalman.device
@@ -260,8 +280,7 @@ def _conditional_forecast(kalman: BatchedKalman, y, mats, conditions, n_simulati
         raise ValueError(f"conditions: expected a float64 CUDA tensor of shape [H, {p}] or [{U}, H, {p}]")
     H = conditions.shape[-2]
     cond = conditions.contiguous()
-    out = kalman.forward(y, *[mats.get(k) for k in ("a0", "P0", "T", "Z", "R", "H", "Q", "c", "d")],
-                         outputs=("predicted_states", "predicted_covs"))
+    out = _predicted(kalman, y, mats, ("predicted_states", "predicted_covs"), partial_rows)
     start_mean, start_cov = out["predicted_states"][:, n].contiguous(), out["predicted_covs"][:, n].contiguous()
     S = U * n_simulations
     if S > 0:
@@ -298,8 +317,9 @@ def conditional_forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, conditions=No
     state_mean [U, H, m], state_cov, obs_mean [U, H, p], obs_cov and with n_simulations > 0 state_paths [S, H, m],
     obs_paths [S, H, p].  Conditioned entries of obs_mean and obs_paths equal the condition exactly and have zero rows
     and columns in obs_cov.  With every entry NaN this is ``forecast`` (the paths bit for bit on the same normals).
-    Raises RuntimeError if some unit fails (F_t not positive definite in the sample or at a window step (n + h + 1),
-    a partly missing row in the sample, P_n / Q / H not positive semi-definite) and NotImplementedError for
+    A partly observed row of y is conditioned on its observed entries (kfb_masked_filter), as a partly conditioned
+    window row is.  Raises RuntimeError if some unit fails (F_t not positive definite on the observed entries in the
+    sample or at a window step (n + h + 1), P_n / Q / H not positive semi-definite) and NotImplementedError for
     time-varying matrices."""
     mats, y, B = _canon_matrices(T, Z, R, H, Q, a0, P0, c, d, y)
     n_series = 1 if y.ndim == 2 else y.shape[0]
@@ -307,7 +327,7 @@ def conditional_forecast(y, a0, P0, T, Z, R, H, Q, c=None, d=None, conditions=No
     kalman = BatchedKalman("standard", y.shape[-2], m, p, r, n_draws=B, n_series=n_series, strict_reference=False,
                            device=T.device)
     res, finfo, winfo = _conditional_forecast(kalman, y, mats, conditions, int(n_simulations), z_init, z_state, z_obs,
-                                              generator)
+                                              generator, _has_partial_rows(y))
     _raise_on_failure("conditional_forecast", (finfo, winfo))
     return res
 
